@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo: libdprt.so on N B200s (torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...   # the CPU oracle of the reference's logic, host cores
+    python bench.py ... --dump-outputs DIR                    # also writes the frame image of the K timed steps to DIR
 
 One STEP = one pass of the hot path = one `runSample` (renderer.cpp:1457-1574: path_gen, then bounces+1 times
 {[secondary-NN], traverse/partition/exchange until quiescent, shade, shadow}) over one frame of camera paths.
@@ -54,6 +55,7 @@ TRAVERSAL_STAGES = ("traverse", "shade", "shadow_trace", "secondary_trace")
 RECORD_BYTES = {"traverse": 128, "secondary_trace": 128, "shade": 64 + 5 * 64, "shadow_trace": 64 + 16, "trace_closest": 32 + 8}
 NODE_BYTES, TRI_BYTES = 80, 48
 MLP_FLOP_PER_QUERY = 573888     # 2 x 286 944 MACs, NeuralVisNetworkWith4Res256SingleOutput (SURVEY.md 8a16)
+DUMP_BYTES = 60 << 20           # --dump-outputs: at most this much .npy data in all
 
 
 def frame_for(world, base_w=1920, base_h=1080):
@@ -249,6 +251,20 @@ def cpu_baseline(dprt, args, seconds_target=15.0):
     return {"value": rays / dt / 1e6, "unit": "Mrays/s", "cores": O.num_threads(), "kind": "port",
             "sample": f"{n} x runSample over a {w}x{h} frame (1/{args.ref_scale} per side) of the same 1-chunk scene, {dt:.1f} s",
             "samples_per_s": w * h * n / dt}
+
+
+def dump_image(out_dir, img, seed=0):
+    """--dump-outputs: the frame image [h, w, 3] as out_dir/image.npy (float32). A frame over DUMP_BYTES (N >= 4) is
+    replaced by a fixed, seeded sample of its pixels: image_pixels.npy [k, 3] and their row-major indices,
+    image_pixel_index.npy [k] (float64, exact)."""
+    img = np.ascontiguousarray(img, np.float32)
+    if img.nbytes <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "image.npy"), img)
+        return
+    pix = img.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(seed).choice(pix.shape[0], DUMP_BYTES // (3 * 4 + 8), replace=False))
+    np.save(os.path.join(out_dir, "image_pixels.npy"), pix[idx])
+    np.save(os.path.join(out_dir, "image_pixel_index.npy"), idx.astype(np.float64))
 
 
 def pinned_array(shape, dtype):
@@ -522,6 +538,13 @@ def run_dprt(args):
     st = F.stats()
     my_rays_walked = st["rays_walked"]
     ms = allreduce(ms, dist.ReduceOp.MAX if W > 1 else None)
+    # ---- --dump-outputs: what a caller of the timed path receives after its last step -- the frame image (warm-up and
+    # timed samples accumulated over the contexts in flight, averaged, reduced to rank 0), as SamplesInFlight.launch returns
+    # it. Taken here, before the passes below add samples to the primary's frame; written after the clock sampler stops.
+    dump_img = None
+    if args.dump_outputs:
+        F.accumulate()
+        dump_img = R.reduce_image(0)
     # ---- per-stage pass over the same samples: CUDA-event pairs around every stage launch on the stream it is launched
     # on. Stage profiling forces strictly serial single-stream execution (no shadow/traverse overlap), so each kernel's
     # duration is its own; the step time of this pass is reported beside it (share_of_step refers to it).
@@ -532,6 +555,8 @@ def run_dprt(args):
     ms_serial = R.timer_stop()
     barrier()
     clk = clocks.stop() if rank == 0 else None          # sampled through the timed region and the serial pass right after it
+    if dump_img is not None:
+        dump_image(args.dump_outputs, dump_img)
     # the per-frame image average + ncclReduce (renderer.cpp:2031-2052), profiled like a stage: 3 times, device events
     keep_r, himg_r = pinned_array((fh, fw, 3), np.float32)
     R.stage_profile(False)
@@ -747,7 +772,16 @@ def main():
     ap.add_argument("--skip-parity", action="store_true", help="N>1: skip the parity gate (A/B runs only)")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frame image they produced to DIR/image.npy (float32; a seeded pixel "
+                         "sample above 60 MiB) so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "dprt":
+            ap.error("--dump-outputs applies to --impl dprt")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3 and args.impl == "dprt":
         args.warmup = 3        # timing rule: at least 3 warm-up steps
     return run_reference(args) if args.impl == "reference" else run_dprt(args)

@@ -1,7 +1,7 @@
 """Generates the committed golden fixtures from the REFERENCE itself (run in the build container only).
 
   rng_kat.json   tea<4>/rnd known answers from /root/reference/optix/random.hpp compiled into
-                 oracle/_ref/librefrng.so (make -C oracle ref)
+                 oracle/_ref/librefrng.so (make -C oracle ref REF=<reference tree>)
   mlp_golden.npz forward outputs of /root/reference/trainingcode/module.py classes on PyTorch-CPU fp32 under
                  torch.manual_seed(19990201) (the reference's seed, trainingcode/main.py:76), for fp16-rounded
                  inputs x ~ U[0,1)^5 from torch.Generator().manual_seed(0); plus a check that
@@ -31,7 +31,7 @@ dprt = importlib.import_module("pg2024-data-parallel-ray-tracing_b200")
 
 def rng_kat():
     R = O.ref_rng()
-    assert R is not None, "run `make -C oracle ref` first"
+    assert R is not None, "run `make -C oracle ref REF=<reference tree>` first"
     cases = [(0, 0), (1, 0), (1920, 1), (2073599, 15), (123456789, 987654321), (0xFFFFFFFF, 0xFFFFFFFF), (8294399, 63)]
     out = []
     for a, b in cases:

@@ -38,15 +38,6 @@ def test_rng_numpy_generator_matches(oracle):
     assert float(val[0]) == float(oracle.rnd_sequence(0x5DF5F2BF, 1)[0])
 
 
-def test_reference_rng_library_when_built(oracle):
-    R = oracle.ref_rng()
-    if R is None:
-        pytest.skip("oracle/_ref/librefrng.so not built on this box (needs /root/reference)")
-    rng = np.random.default_rng(0)
-    for a, b in rng.integers(0, 2**32, (200, 2), dtype=np.uint64):
-        assert int(R.ref_tea4(int(a), int(b))) == oracle.tea4(int(a), int(b))
-
-
 # ---- deterministic transcendentals: accuracy of the specification against libm ------------------------------------
 def test_det_transcendentals_accuracy(oracle):
     L = oracle.lib()
@@ -145,6 +136,20 @@ def test_partition_semantics(oracle):
 
 
 # ---- proxy MLP: oracle fp32 chain vs the reference's module.py outputs (tests/golden/mlp_golden.npz) -----------------
+def _torch_forward_one_thread(m, x16):
+    """fp32 CPU forward on the golden inputs, single-threaded. The GEMM's rounding depends on how many OpenMP threads
+    split it (3, 5, 6, 7 threads give other last bits), and that count is process state which whatever ran before may
+    have changed (torch and liboracle share the OpenMP runtime). One thread reproduces the golden bits."""
+    import torch
+    prev = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        with torch.no_grad():
+            return m(torch.from_numpy(x16.view(np.float16).astype(np.float32))).numpy().reshape(-1)
+    finally:
+        torch.set_num_threads(prev)
+
+
 @pytest.mark.parametrize("nres", [4, 6])
 def test_mlp_oracle_matches_reference_module(oracle, golden_dir, nres):
     import torch
@@ -153,8 +158,7 @@ def test_mlp_oracle_matches_reference_module(oracle, golden_dir, nres):
     m = dprt.proxy.make_proxy(256, nres).eval()
     blob = dprt.proxy.pack_module(m)
     x16 = g["x_f16"]
-    with torch.no_grad():
-        y_torch = m(torch.from_numpy(x16.view(np.float16).astype(np.float32))).numpy().reshape(-1)
+    y_torch = _torch_forward_one_thread(m, x16)
     # our torch definition reproduces the reference class bit for bit (same seed, same parameter order)
     assert np.array_equal(y_torch, g[f"y_{nres}res256"])
     yf, yh = oracle.mlp_forward(blob, x16)
@@ -176,8 +180,7 @@ def test_mlp_oracle_matches_reference_module_other_variants(oracle, golden_dir, 
     m = dprt.proxy.make_proxy(width, nres, sigmoid=sig).eval()
     x16 = g["x_f16"]
     key = f"y_{nres}res{width}" + ("_sigmoid" if sig else "")
-    with torch.no_grad():
-        y_torch = m(torch.from_numpy(x16.view(np.float16).astype(np.float32))).numpy().reshape(-1)
+    y_torch = _torch_forward_one_thread(m, x16)
     assert np.array_equal(y_torch, g[key])
     blob = dprt.proxy.pack_module(m)
     assert dprt.proxy.unpack_blob(blob)["sigmoid"] == sig and dprt.proxy.unpack_blob(blob)["width"] == width
