@@ -209,6 +209,8 @@ typedef struct dprt_stats {
     int64_t walked_shadow;     /* and cache-answered MainRay queries are in rays_* but not here)                               */
     int64_t walked_secondary;
     int64_t paths_partitioned; /* records written by the path partition (Work_Efficient_Scan): the reorder roofline's unit */
+    int64_t shade_cache_stale; /* single-rank bounce of dprt_render_sample: MainRay queries whose hit-cache entry was of another
+                                  epoch (an invariant says never; shaded with the stale entry, so any non-zero count is a bug) */
 } dprt_stats;
 
 /* Buffer identifiers for dprt_download/dprt_upload (parity harness access to Params buffers). */

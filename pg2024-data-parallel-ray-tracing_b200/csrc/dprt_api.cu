@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <atomic>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <string>
@@ -30,7 +31,7 @@ using namespace dprt;
 
 struct dprt_bvh8 { Bvh8 b; };
 
-constexpr int kDevStats = 2 + DPRT_STAGE_COUNT;     // words of dprt_ctx::d_cacheHits
+constexpr int kDevStats = 3 + DPRT_STAGE_COUNT;     // words of dprt_ctx::d_cacheHits
 
 namespace {
 
@@ -144,7 +145,8 @@ struct dprt_ctx {
     uint8_t* d_nnKey = nullptr;         // one key byte per NN query slot
     HitRec* d_hits = nullptr;           // N closest-hit records (MainRay)
     HitRec* d_hitCache = nullptr;       // N per-pixel closest hits of the current epoch (null when cfg.mainRayRetrace)
-    unsigned long long* d_cacheHits = nullptr;   // kDevStats words: [0] MainRay queries answered from the cache, [1] rays that walked a BVH, [2 + stage] per stage (since reset_stats)
+    unsigned long long* d_cacheHits = nullptr;   // kDevStats words: [0] MainRay queries answered from the cache, [1] rays that walked a BVH, [2 + stage] per stage,
+                                                 // [2 + DPRT_STAGE_COUNT] stale hit-cache entries met by launch_shade_cached (since reset_stats)
     // "reset by count" of the shadow planes of directLightingBuffer: MainRay records which pixels get shadow paths
     // (two lists, ping-pong: one describes the planes that are dirty now, the other is free for the next MainRay)
     int32_t* d_live[2] = {nullptr, nullptr};
@@ -180,6 +182,10 @@ struct dprt_ctx {
     int32_t* d_queue_aux = nullptr;     // trace scratch of launches on the aux stream
     bool auxPending = false;            // aux work not yet joined into `stream`
     int auxGuardBase = 0;               // first path slot the pending aux work reads (its shadow paths start there)
+    // single-rank bounce inside dprt_render_sample (single_rank_shortcut): the exchange leaves the partition output in
+    // `transfer` and MainRay shades it from there with the hits of the hit cache
+    bool shortcut = false;
+    bool recsInTransfer = false;        // set by such an exchange, consumed by the dprt_shade that follows
     float* d_image = nullptr;           // averaged image, 3N
     float* d_image_sum = nullptr;       // reduce target, 3N
     int32_t* d_gather = nullptr;        // W*(W+1) offsets of all ranks
@@ -575,6 +581,7 @@ int dprt_get_stats(const dprt_ctx* ctx, dprt_stats* out) {
         out->rays_shade_cached = (int64_t)v[0]; out->rays_walked = (int64_t)v[1];
         out->walked_traverse = (int64_t)v[2 + DPRT_STAGE_TRAVERSE]; out->walked_shade = (int64_t)v[2 + DPRT_STAGE_SHADE];
         out->walked_shadow = (int64_t)v[2 + DPRT_STAGE_SHADOW_TRACE]; out->walked_secondary = (int64_t)v[2 + DPRT_STAGE_SECONDARY_TRACE];
+        out->shade_cache_stale = (int64_t)v[2 + DPRT_STAGE_COUNT];
     }
     return 0;
 }
@@ -963,7 +970,8 @@ int dprt_exchange(dprt_ctx* ctx, int* done) {
     if (W == 1) {
         int r = read_offsets(ctx); if (r) return r;
         const int cnt = ctx->h_offsets[1];
-        if (cnt > 0) CK(cudaMemcpyAsync(ctx->hp.paths, ctx->hp.transfer, cnt * R, cudaMemcpyDeviceToDevice, ctx->stream));
+        if (ctx->shortcut) ctx->recsInTransfer = true;     // dprt_shade reads the records where the partition left them
+        else if (cnt > 0) CK(cudaMemcpyAsync(ctx->hp.paths, ctx->hp.transfer, cnt * R, cudaMemcpyDeviceToDevice, ctx->stream));
         ctx->pathSize = cnt; ctx->stats.paths_partitioned += cnt;
         if (done) *done = 1;
         ctx->stats.exchange_iters++;
@@ -1052,8 +1060,11 @@ int dprt_shade(dprt_ctx* ctx) {
     ctx->hp.livePixel = ctx->d_live[w]; ctx->liveCount[w] = ctx->pathSize; ctx->shadeIdx = w;
     sync_params(ctx);
     StageScope sc_(ctx, DPRT_STAGE_SHADE, ctx->pathSize > 0);
-    launch_shade(ctx->hp, ctx->pathSize, ctx->stream);
-    ctx->stats.kernel_launches += trace_kernels_per_stage() * (ctx->pathSize > 0);
+    const bool cached = ctx->recsInTransfer;
+    ctx->recsInTransfer = false;
+    if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, ctx->stream);
+    else launch_shade(ctx->hp, ctx->pathSize, ctx->stream);
+    ctx->stats.kernel_launches += (cached ? 1 : trace_kernels_per_stage()) * (ctx->pathSize > 0);
     ctx->stats.rays_shade += ctx->pathSize;
     ctx->epoch++;                       // the records now hold the next bounce's rays: cached hits are stale
     ctx->histFresh = false;
@@ -1101,7 +1112,7 @@ int dprt_shadow_trace(dprt_ctx* ctx) {
     CK(cudaMemsetAsync(ctx->hp.queryHist, 0, 64 * sizeof(int32_t), ctx->stream));
     StageScope sc_(ctx, DPRT_STAGE_SHADOW_TRACE, ctx->shadowPathSize > 0);
     launch_shadow_trace(ctx->hp, ctx->shadowPathSize, ctx->stream);
-    ctx->stats.kernel_launches += trace_kernels_per_stage() * (ctx->shadowPathSize > 0);
+    ctx->stats.kernel_launches += shadow_trace_kernels(ctx->hp) * (ctx->shadowPathSize > 0);
     ctx->stats.rays_shadow += ctx->shadowPathSize;
     // planes now hold this bounce's terms: covered by the MainRay list if nothing else was dirty, else unknown
     if (ctx->shadowPathSize > 0)
@@ -1703,8 +1714,21 @@ int bounce_post(dprt_ctx* ctx) {
 }
 }  // namespace
 
-int dprt_render_sample(dprt_ctx* ctx, int sample) {
-    if (!ctx) return DPRT_ERR_INVALID;
+namespace {
+// Single-rank bounce: at W = 1 with proxies off every path the partition keeps was hit on this rank, and traverse_post_kernel
+// filed that hit in the hit cache in the current epoch -- the MainRay trace would only copy it from there. So the exchange
+// skips the copy of the partition output back to `paths`, and dprt_shade shades straight from `transfer` with the cached
+// hits (launch_shade_cached), one launch instead of two plus a D2D copy. The buffers after the bounce are the same: the
+// shading program writes every path slot the copy wrote. The parity aid needs hitPrim from the MainRay trace, and an
+// uploaded proxy can retarget a path that was not hit. DPRT_SINGLE_RANK_SHORTCUT=0 turns it off (A/B, tests).
+bool single_rank_shortcut(const dprt_ctx* ctx) {
+    if (ctx->world != 1 || ctx->cfg.proxyMode || !ctx->d_hitCache || ctx->hp.hitPrim) return false;
+    for (const ObjectHost& o : ctx->objects) if (o.present && o.desc.isProxy) return false;
+    const char* v = getenv("DPRT_SINGLE_RANK_SHORTCUT");
+    return !(v && std::strcmp(v, "0") == 0);
+}
+
+int render_sample(dprt_ctx* ctx, int sample) {
     int r;
     if ((r = dprt_begin_sample(ctx, sample))) return r;
     if ((r = dprt_path_gen(ctx))) return r;
@@ -1731,6 +1755,15 @@ int dprt_render_sample(dprt_ctx* ctx, int sample) {
         ctx->auxPending = true; ctx->auxGuardBase = ctx->pathSize;
     }
     return join_aux(ctx);
+}
+}  // namespace
+
+int dprt_render_sample(dprt_ctx* ctx, int sample) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    ctx->shortcut = single_rank_shortcut(ctx);
+    const int r = render_sample(ctx, sample);
+    ctx->shortcut = false; ctx->recsInTransfer = false;
+    return r;
 }
 
 int dprt_render_sample_group(dprt_ctx** ctxs, int W, int sample) {

@@ -73,7 +73,7 @@ struct DevParams {
     int32_t* traceQueue;           // head of the persistent trace kernel's ray queue
     HitRec*  hitCache;             // per pixel: closest local hit of the pixel's path in the current epoch (null = off)
     uint32_t hitEpoch;             // one epoch per bounce of a sample: entries of older epochs are stale
-    unsigned long long* cacheHits; // device counter: MainRay queries answered from the cache
+    unsigned long long* cacheHits; // device statistics (dprt_api.cu kDevStats): [0] MainRay queries answered from the cache
     int32_t  splitL;               // settled-deque mode of the migrate loop: records at index >= splitL that stay on this
                                    // rank are counted in bucket worldSize instead of bucket worldID (INT_MAX: reference)
     int32_t* secLive;              // per path slot of the last Target_Node_Update: pixel whose tMax scratch it used, or -1
@@ -89,7 +89,11 @@ struct DevParams {
 void launch_path_gen(const DevParams& p, int n, cudaStream_t stream);
 void launch_traverse(const DevParams& p, int n, cudaStream_t stream);
 void launch_shade(const DevParams& p, int n, cudaStream_t stream);
+// MainRay without its trace: shades the partition output p.transfer[0..n) with the hits of the hit cache (single rank only)
+void launch_shade_cached(const DevParams& p, int n, cudaStream_t stream);
+// proxies off: the any-hit trace also adds the unoccluded terms to directLightingBuffer and no post kernel follows
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t stream);
+int shadow_trace_kernels(const DevParams& p);   // kernels launch_shadow_trace launches
 void launch_secondary_trace(const DevParams& p, int n, cudaStream_t stream);
 int trace_kernels_per_stage();  // kernels one traversal stage launches (trace, the parked tail's finish kernel, post)
 size_t trace_scratch_bytes();   // per-context scratch of the persistent trace kernel (queue head + cooperative-mode pools)

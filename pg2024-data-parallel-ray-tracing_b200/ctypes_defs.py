@@ -84,7 +84,8 @@ class Stats(C.Structure):
                 ("rays_secondary", C.c_int64), ("nn_queries", C.c_int64), ("paths_sent_offrank", C.c_int64),
                 ("exchange_iters", C.c_int64), ("kernel_launches", C.c_int64), ("bytes_alltoall", C.c_int64),
                 ("rays_shade_cached", C.c_int64), ("rays_walked", C.c_int64), ("walked_traverse", C.c_int64),
-                ("walked_shade", C.c_int64), ("walked_shadow", C.c_int64), ("walked_secondary", C.c_int64), ("paths_partitioned", C.c_int64)]
+                ("walked_shade", C.c_int64), ("walked_shadow", C.c_int64), ("walked_secondary", C.c_int64), ("paths_partitioned", C.c_int64),
+                ("shade_cache_stale", C.c_int64)]
 
     def as_dict(self):
         return {k: int(getattr(self, k)) for k, _ in self._fields_ if k != "reserved_"}
@@ -107,7 +108,7 @@ TRI_DTYPE = np.dtype([("v0", "<f4", 3), ("primID", "<i4"), ("v1", "<f4", 3), ("m
 
 assert PATH_DTYPE.itemsize == 64 and QUERY_DTYPE.itemsize == 48 and RAY_DTYPE.itemsize == 32 and HIT_DTYPE.itemsize == 8
 assert NODE_DTYPE.itemsize == 80 and TRI_DTYPE.itemsize == 48 and MATERIAL_DTYPE.itemsize == 16 and LIGHT_DTYPE.itemsize == 48
-assert C.sizeof(Config) == 64 and C.sizeof(ObjectDesc) == 84 and C.sizeof(Camera) == 56 and C.sizeof(Stats) == 128
+assert C.sizeof(Config) == 64 and C.sizeof(ObjectDesc) == 84 and C.sizeof(Camera) == 56 and C.sizeof(Stats) == 136
 assert C.sizeof(MeshDesc) == 88 and C.sizeof(InstanceDesc) == 56
 
 P2P_HANDLE_BYTES = 208     # DPRT_P2P_HANDLE_BYTES
