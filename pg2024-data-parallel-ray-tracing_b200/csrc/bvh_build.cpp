@@ -12,7 +12,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstring>
-#include <cstdlib>
 #include <limits>
 
 namespace dprt {
@@ -177,14 +176,13 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
     // (cost cPrim x triangles x area):
     //   C(n, 1) = min(leaf(n), cNode A_n + min_k C(left, k) + C(right, 8 - k))
     //   C(n, i) = min(C(n, i - 1), min_k C(left, k) + C(right, i - k))
-    // A top-down greedy collapse ("open the largest child until there are eight") leaves ragged bottoms -- wide nodes with two or
-    // three leaf children, 42 % slot occupancy on the benchmark chunk -- and every such node costs a ray a full node step.
+    // Why the optimum: a wide node costs a ray a full node step however few of its eight slots it uses, and a collapse decided
+    // one node at a time leaves many nodes with two or three leaf children at the bottom of the tree. Minimising the cost over
+    // the whole subtree avoids them.
     // cNode : cPrim = 4 : 1 is the trace kernel's issue-slot ratio of a node step to a triangle test (profiles/bvh_quality.py).
     const int nn = b2.nnodes.load();
-    const float cNode = getenv("DPRT_BVH_CNODE") ? (float)atof(getenv("DPRT_BVH_CNODE")) : 4.0f;
+    const float cNode = 4.0f;
     const float cPrim = 1.0f;
-    // DPRT_BVH_COLLAPSE=greedy selects the previous top-down collapse (A/B in profiles/ab_r2_bvh_collapse.txt)
-    const bool greedy = getenv("DPRT_BVH_COLLAPSE") && std::strcmp(getenv("DPRT_BVH_COLLAPSE"), "greedy") == 0;
     const float INF = std::numeric_limits<float>::max();
     std::vector<float> C((size_t)nn * 8);          // C[n * 8 + i - 1]
     std::vector<uint8_t> K((size_t)nn * 8);        // i = 1: 1 = leaf, 2 = wide node; i >= 2: roots given to the left child, 0 = as for i - 1
@@ -235,22 +233,7 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         const Node2& nd = n2[it.n2];
         Child ch[8]; int nch = 0;
         if (nd.count > 0 || (it.n2 == root && K[(size_t)root * 8] == 1)) ch[nch++] = Child{it.n2, true};     // a root that is itself a leaf
-        else if (!greedy) { collector.run(nd.left, K8[it.n2], ch, nch); collector.run(nd.right, 8 - K8[it.n2], ch, nch); }
-        else {
-            ch[nch++] = Child{nd.left, n2[nd.left].count > 0}; ch[nch++] = Child{nd.right, n2[nd.right].count > 0};
-            for (;;) {                                // greedy: open the internal child with the largest area
-                if (nch >= 8) break;
-                int best = -1; float ba = -1.f;
-                for (int i = 0; i < nch; i++) {
-                    if (ch[i].leaf) continue;
-                    float a = n2[ch[i].n].box.half_area();
-                    if (a > ba) { ba = a; best = i; }
-                }
-                if (best < 0) break;
-                int l = n2[ch[best].n].left, r = n2[ch[best].n].right;
-                ch[best] = Child{l, n2[l].count > 0}; ch[nch++] = Child{r, n2[r].count > 0};
-            }
-        }
+        else { collector.run(nd.left, K8[it.n2], ch, nch); collector.run(nd.right, 8 - K8[it.n2], ch, nch); }
         // node frame
         Box nb; nb.reset();
         for (int i = 0; i < nch; i++) nb.grow(n2[ch[i].n].box);

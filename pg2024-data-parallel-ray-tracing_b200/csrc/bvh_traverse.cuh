@@ -22,12 +22,6 @@ DPRT_D float qbias(uint32_t w, uint32_t magic) {
 }
 
 #define DPRT_STACK 40
-#ifndef DPRT_PREFETCH_NODE
-#define DPRT_PREFETCH_NODE 0
-#endif
-#ifndef DPRT_PREFETCH_TRI
-#define DPRT_PREFETCH_TRI 0
-#endif
 
 // instrumentation (dprt_enable_counters): BVH8 nodes fetched and triangles tested by one thread
 struct TraceCount { uint32_t nodes, tris; };
@@ -155,19 +149,6 @@ DPRT_D uint32_t trav_node(Trav& s, uint2* stack, TraceCount& cnt, const uint32_t
     if (COUNT) cnt.nodes++;
     uint32_t tmask;
     expand_node(s.nodes, ni, s.o.x, s.o.y, s.o.z, s.idx, s.idy, s.idz, s.octinv, s.tmin, s.tbest, magic, s.ng, s.tg, tmask);
-#if DPRT_PREFETCH_NODE
-    {   // the node this lane expands next (nearest hit child, else the top of its stack) is known now, ~100 instructions of
-        // warp bookkeeping before its five LDG.128 are issued: pull its lines into L1 meanwhile
-        uint2 g = s.ng;
-        if (!(g.y & 0xff000000u) && s.sp > 0) g = stack[s.sp - 1];
-        if (g.y & 0xff000000u) {
-            const uint32_t nb = 31u - __clz(g.y);
-            const char* np = reinterpret_cast<const char*>(s.nodes + 5 * (size_t)group_node(g, nb, s.octinv));
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(np));
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(np + 79));
-        }
-    }
-#endif
     return tmask;
 }
 
@@ -235,9 +216,6 @@ DPRT_D void wq_append(WarpQueue& w, int& qlen, int lane, bool busy, Trav& s, int
         s.tg.y &= s.tg.y - 1u;
         const uint32_t ti = s.tg.x + __popc(tm & ((1u << k) - 1u));
         w.q[pos++] = ((uint32_t)lane << DPRT_TRI_BITS) | ti;
-#if DPRT_PREFETCH_TRI
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char*>(s.tris + 3 * (size_t)ti)));
-#endif
         pend++;
     }
     qlen = min(DPRT_QCAP, qlen + total);

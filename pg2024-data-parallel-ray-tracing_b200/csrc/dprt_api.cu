@@ -192,7 +192,6 @@ struct dprt_ctx {
     int32_t* h_pinned = nullptr;        // pinned staging for counts/offsets
     void* d_flush = nullptr; size_t flush_bytes = 0;
     void* d_io = nullptr; size_t io_bytes = 0;   // staging for the standalone host-buffer operators
-    HitRec* d_rayPark = nullptr; size_t rayParkCount = 0;     // tail-parking scratch of the standalone closest-hit operator
     int pathSize = 0, shadowPathSize = 0;
     int sample = 0;
     int queryTotal = 0;                 // rows of the last bucketing
@@ -324,16 +323,6 @@ int upload_objects(dprt_ctx* ctx) {
     return 0;
 }
 
-// n HitRec for the parked tail of a standalone closest-hit launch (the stage launches use the stage's own hits[] array)
-int ensure_ray_park(dprt_ctx* ctx, size_t n) {
-    if (ctx->rayParkCount >= n) return 0;
-    if (ctx->d_rayPark) cudaFree(ctx->d_rayPark);
-    ctx->d_rayPark = nullptr; ctx->rayParkCount = 0;
-    CK(cudaMalloc(&ctx->d_rayPark, n * sizeof(HitRec)));
-    ctx->rayParkCount = n;
-    return 0;
-}
-
 int ensure_io(dprt_ctx* ctx, size_t bytes) {
     if (ctx->io_bytes >= bytes) return 0;
     if (ctx->d_io) cudaFree(ctx->d_io);
@@ -424,7 +413,7 @@ static int create_impl(const dprt_config* cfg, int rank, int world, int device, 
         CK(cudaMemsetAsync(ctx->d_mlpTable, 0, 2 * 32 * sizeof(MlpGroupEntry), ctx->stream));
         CK(cudaMalloc(&ctx->d_hist, 128 * sizeof(int32_t)));
         CK(cudaMemsetAsync(ctx->d_hist, 0, 128 * sizeof(int32_t), ctx->stream));
-        ctx->scratch.maxTiles = (int)((std::max(Q, N) + 255) / 256) + 1;       // the smallest tile any partition variant uses
+        ctx->scratch.maxTiles = (int)((std::max(Q, N) + 1023) / 1024) + 1;     // the smallest tile any partition kernel uses
         CK(cudaMalloc(&ctx->scratch.tileState, (size_t)ctx->scratch.maxTiles * 32 * sizeof(unsigned long long)));
         CK(cudaMemsetAsync(ctx->scratch.tileState, 0, (size_t)ctx->scratch.maxTiles * 32 * sizeof(unsigned long long), ctx->stream));
         CK(cudaMalloc(&ctx->scratch.tileCounter, sizeof(uint32_t)));
@@ -557,7 +546,6 @@ void dprt_destroy(dprt_ctx* ctx) {
     if (ctx->d_counters) cudaFree(ctx->d_counters);
     if (ctx->d_flush) cudaFree(ctx->d_flush);
     if (ctx->d_io) cudaFree(ctx->d_io);
-    if (ctx->d_rayPark) cudaFree(ctx->d_rayPark);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -912,7 +900,7 @@ int dprt_traverse(dprt_ctx* ctx) {
     CK(cudaMemsetAsync(ctx->hp.pathHist, 0, 32 * sizeof(int32_t), ctx->stream));
     StageScope sc_(ctx, DPRT_STAGE_TRAVERSE, ctx->pathSize > 0);
     launch_traverse(ctx->hp, ctx->pathSize, ctx->stream);
-    ctx->stats.kernel_launches += trace_kernels_per_stage() * (ctx->pathSize > 0);
+    ctx->stats.kernel_launches += 2 * (ctx->pathSize > 0);                  // trace + post
     ctx->stats.rays_traverse += ctx->pathSize;
     ctx->histFresh = true;
     CK(cudaGetLastError());
@@ -1064,7 +1052,7 @@ int dprt_shade(dprt_ctx* ctx) {
     ctx->recsInTransfer = false;
     if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, ctx->stream);
     else launch_shade(ctx->hp, ctx->pathSize, ctx->stream);
-    ctx->stats.kernel_launches += (cached ? 1 : trace_kernels_per_stage()) * (ctx->pathSize > 0);
+    ctx->stats.kernel_launches += (cached ? 1 : 2) * (ctx->pathSize > 0);   // [trace +] post
     ctx->stats.rays_shade += ctx->pathSize;
     ctx->epoch++;                       // the records now hold the next bounce's rays: cached hits are stale
     ctx->histFresh = false;
@@ -1112,7 +1100,7 @@ int dprt_shadow_trace(dprt_ctx* ctx) {
     CK(cudaMemsetAsync(ctx->hp.queryHist, 0, 64 * sizeof(int32_t), ctx->stream));
     StageScope sc_(ctx, DPRT_STAGE_SHADOW_TRACE, ctx->shadowPathSize > 0);
     launch_shadow_trace(ctx->hp, ctx->shadowPathSize, ctx->stream);
-    ctx->stats.kernel_launches += shadow_trace_kernels(ctx->hp) * (ctx->shadowPathSize > 0);
+    ctx->stats.kernel_launches += (ctx->hp.proxyMode ? 2 : 1) * (ctx->shadowPathSize > 0);   // trace [+ post with proxies]
     ctx->stats.rays_shadow += ctx->shadowPathSize;
     // planes now hold this bounce's terms: covered by the MainRay list if nothing else was dirty, else unknown
     if (ctx->shadowPathSize > 0)
@@ -1130,7 +1118,7 @@ int dprt_secondary_trace(dprt_ctx* ctx) {
     CK(cudaMemsetAsync(ctx->hp.queryHist, 0, 64 * sizeof(int32_t), ctx->stream));
     StageScope sc_(ctx, DPRT_STAGE_SECONDARY_TRACE, ctx->pathSize > 0);
     launch_secondary_trace(ctx->hp, ctx->pathSize, ctx->stream);
-    ctx->stats.kernel_launches += trace_kernels_per_stage() * (ctx->pathSize > 0);
+    ctx->stats.kernel_launches += 2 * (ctx->pathSize > 0);                  // trace + post
     ctx->stats.rays_secondary += ctx->pathSize;
     ctx->qhistFresh = true; ctx->queryWhich = 1;
     ctx->histFresh = false;
@@ -1268,7 +1256,7 @@ int deque_traverse(dprt_ctx* ctx) {
         launch_traverse(ctx->hp, ctx->pathSize, ctx->stream);
     }
     ctx->hp.splitL = 0x7fffffff;
-    ctx->stats.kernel_launches += trace_kernels_per_stage() * (ctx->pathSize > 0);
+    ctx->stats.kernel_launches += 2 * (ctx->pathSize > 0);                  // trace + post
     ctx->stats.rays_traverse += ctx->pathSize + (ctx->back - ctx->front);          // the reference launches over the riders too
     CK(cudaGetLastError());
     return 0;
@@ -1901,10 +1889,9 @@ int dprt_trace_closest_device(dprt_ctx* ctx, const void* rays_dev, int64_t n, vo
     if (!ctx || !rays_dev || !hits_dev || n < 0) return DPRT_ERR_INVALID;
     if (n > kMaxTraceRays) return fail(ctx, DPRT_ERR_INVALID, "more rays than one launch can index (split the batch)");
     CK(cudaSetDevice(ctx->device));
-    { int r = ensure_ray_park(ctx, (size_t)n); if (r) return r; }
     StageScope sc_(ctx, DPRT_STAGE_TRACE_CLOSEST, n > 0);
     launch_trace_closest(ctx->d_objects, ctx->cfg.sceneSize, ctx->d_textures, ctx->d_matTex, (const dprt_ray*)rays_dev, (dprt_hit*)hits_dev, n, ctx->d_queue,
-                         ctx->hp.counters, ctx->d_rayPark, ctx->stream);
+                         ctx->hp.counters, ctx->stream);
     ctx->stats.kernel_launches += n > 0;
     ctx->stats.rays_traverse += n;
     CK(cudaGetLastError());
@@ -1939,7 +1926,7 @@ int dprt_gen_train_data(dprt_ctx* ctx, int si, const dprt_ray* rays_host, int64_
     CK(cudaMemcpyAsync(d, rays_host, rb, cudaMemcpyHostToDevice, ctx->stream));
     {
         StageScope sc_(ctx, DPRT_STAGE_TRACE_CLOSEST);
-        launch_trace_closest(ctx->d_objects + si, 1, ctx->d_textures, ctx->d_matTex, (const dprt_ray*)d, (dprt_hit*)(d + rb), n, ctx->d_queue, ctx->hp.counters, nullptr, ctx->stream);   // startObj only
+        launch_trace_closest(ctx->d_objects + si, 1, ctx->d_textures, ctx->d_matTex, (const dprt_ray*)d, (dprt_hit*)(d + rb), n, ctx->d_queue, ctx->hp.counters, ctx->stream);   // startObj only
         launch_train_features(ctx->d_objects + si, (const dprt_ray*)d, (const dprt_hit*)(d + rb), n, (float*)(d + rb + hb), (float*)(d + rb + hb + fb), ctx->stream);
     }
     ctx->stats.kernel_launches += 2;
@@ -1968,7 +1955,7 @@ int dprt_gen_precom_data(dprt_ctx* ctx, int si, const dprt_ray* rays_host, int64
     {
         StageScope sc_(ctx, DPRT_STAGE_TRACE_CLOSEST);
         launch_precom_features(ctx->d_objects + si, d_rays, n, d_feat, d_ta, ctx->stream);                 // proxy AABB (aabbHandle)
-        launch_trace_closest(ctx->d_objects + si, 1, ctx->d_textures, ctx->d_matTex, d_rays, d_hits, n, ctx->d_queue, ctx->hp.counters, nullptr, ctx->stream);   // originHandle, tMax = inf
+        launch_trace_closest(ctx->d_objects + si, 1, ctx->d_textures, ctx->d_matTex, d_rays, d_hits, n, ctx->d_queue, ctx->hp.counters, ctx->stream);   // originHandle, tMax = inf
         launch_precom_labels(ctx->d_objects + si, d_hits, d_ta, n, d_label, d_valid, ctx->stream);
     }
     ctx->stats.kernel_launches += 3;

@@ -93,13 +93,10 @@ void launch_shade(const DevParams& p, int n, cudaStream_t stream);
 void launch_shade_cached(const DevParams& p, int n, cudaStream_t stream);
 // proxies off: the any-hit trace also adds the unoccluded terms to directLightingBuffer and no post kernel follows
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t stream);
-int shadow_trace_kernels(const DevParams& p);   // kernels launch_shadow_trace launches
 void launch_secondary_trace(const DevParams& p, int n, cudaStream_t stream);
-int trace_kernels_per_stage();  // kernels one traversal stage launches (trace, the parked tail's finish kernel, post)
 size_t trace_scratch_bytes();   // per-context scratch of the persistent trace kernel (queue head + cooperative-mode pools)
-// park: n HitRec of scratch for the tail of the launch (kernels.cu "tail parking"), or null
 void launch_trace_closest(const DevObject* objects, int sceneSize, const DevTexture* textures, const int32_t* matTex, const dprt_ray* rays,
-                          dprt_hit* hits, int64_t n, int32_t* queue, unsigned long long* counters, HitRec* park, cudaStream_t stream);
+                          dprt_hit* hits, int64_t n, int32_t* queue, unsigned long long* counters, cudaStream_t stream);
 
 // Vis pipeline epilogue (vis_ray_kernel.cu:145-160): features and label of every traced training ray of object `obj`
 void launch_train_features(const DevObject* obj, const dprt_ray* rays, const dprt_hit* hits, int64_t n, float* features,

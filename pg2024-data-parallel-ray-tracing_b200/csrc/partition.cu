@@ -29,16 +29,25 @@ constexpr uint32_t ST_AGG = 1u << 30, ST_INC = 2u << 30, ST_MASK = 3u << 30, VAL
 // and tile ids are the running ticket counter minus the tickets of all earlier launches -- so neither the state array nor
 // the counter is ever cleared (two cudaMemsetAsync per partition launch gone from the migrate loop).
 
+// Bucket of path record i from its last two words (targetNode, flags): -1 unless it is valid and addressed to one of the W
+// ranks; a record that stays on rank `me` and sits at index >= splitL goes to bucket W, which only exists in settled-deque
+// mode (B == W + 1; me == -1 otherwise). Reading W, me and splitL through `ops` keeps the early exit a branch: as plain
+// arguments, the compiler turns it into selects evaluated for every record.
+template <class Ops>
+__device__ __forceinline__ int path_bucket(const Ops& ops, uint32_t targetNode, uint32_t flags, int i) {
+    const int target = (int)targetNode;
+    const bool valid = (flags >> 16) & 0xffu;
+    if (!(valid && target >= 0 && target < ops.W)) return -1;
+    return (target == ops.me && i >= ops.splitL) ? ops.W : target;
+}
+
 struct PathOps {
     static constexpr bool kDirect = false;
     const dprt_path_record* in; dprt_path_record* out; int B; int W; int me; int splitL;
     __device__ __forceinline__ bool skip() const { return false; }
     __device__ __forceinline__ int key(int i) const {
         const uint4 w = reinterpret_cast<const uint4*>(in + i)[3];   // visitedMask, currentNode, targetNode, flags
-        const int target = (int)w.z;
-        const bool valid = (w.w >> 16) & 0xffu;
-        if (!(valid && target >= 0 && target < W)) return -1;
-        return (target == me && i >= splitL) ? W : target;           // bucket W only exists in settled-deque mode (B == W + 1)
+        return path_bucket(*this, w.z, w.w, i);
     }
     __device__ __forceinline__ void copy(int src, int /*bucket*/, int dst) const {
         const float4* s = reinterpret_cast<const float4*>(in + src);
@@ -47,12 +56,7 @@ struct PathOps {
         d[0] = a; d[1] = b; d[2] = c; d[3] = e;
     }
     // staged variant (partition_staged_kernel): key of record i from the last 8 bytes of its staged copy; where bucket b goes
-    __device__ __forceinline__ int key_staged(uint2 w, int i) const {
-        const int target = (int)w.x;
-        const bool valid = (w.y >> 16) & 0xffu;
-        if (!(valid && target >= 0 && target < W)) return -1;
-        return (target == me && i >= splitL) ? W : target;
-    }
+    __device__ __forceinline__ int key_staged(uint2 w, int i) const { return path_bucket(*this, w.x, w.y, i); }
     __device__ __forceinline__ dprt_path_record* dst_base(int /*bucket*/) const { return out; }
 };
 
@@ -65,10 +69,7 @@ struct PeerPathOps {
     __device__ __forceinline__ bool skip() const { return *(const volatile int32_t*)&plan->error != 0; }
     __device__ __forceinline__ int key(int i) const {
         const uint4 w = reinterpret_cast<const uint4*>(in + i)[3];
-        const int target = (int)w.z;
-        const bool valid = (w.w >> 16) & 0xffu;
-        if (!(valid && target >= 0 && target < W)) return -1;
-        return (target == me && i >= splitL) ? W : target;
+        return path_bucket(*this, w.z, w.w, i);
     }
     __device__ __forceinline__ void copy(int src, int bucket, int dst) const {
         const float4* s = reinterpret_cast<const float4*>(in + src);
@@ -76,12 +77,7 @@ struct PeerPathOps {
         const float4 a = s[0], b = s[1], c = s[2], e = s[3];
         d[0] = a; d[1] = b; d[2] = c; d[3] = e;
     }
-    __device__ __forceinline__ int key_staged(uint2 w, int i) const {
-        const int target = (int)w.x;
-        const bool valid = (w.y >> 16) & 0xffu;
-        if (!(valid && target >= 0 && target < W)) return -1;
-        return (target == me && i >= splitL) ? W : target;
-    }
+    __device__ __forceinline__ int key_staged(uint2 w, int i) const { return path_bucket(*this, w.x, w.y, i); }
     __device__ __forceinline__ dprt_path_record* dst_base(int bucket) const { return plan->dst[bucket]; }
 };
 
@@ -107,6 +103,53 @@ struct QueryOps {
         for (int k = 0; k < 5; k++) fd[k] = fs[k];
     }
 };
+
+// Warp 0 of a tile, lane = bucket, once the per-step counts s_cnt[0..kSteps) are in: turns them into exclusive in-tile
+// offsets and returns where the tile's first record of the bucket goes. That is the bucket base plus the bucket's records in
+// all earlier tiles.
+template <class Ops, int kSteps>
+__device__ __forceinline__ int tile_bucket_base(int (*s_cnt)[32], int lane, int B, int tile, const int32_t* __restrict__ hist,
+                                                int32_t* __restrict__ offsets, unsigned long long* tileState, uint32_t gen) {
+    // exclusive scan over the in-tile steps
+    int run = 0;
+#pragma unroll 8
+    for (int s = 0; s < kSteps; s++) { const int c = s_cnt[s][lane]; s_cnt[s][lane] = run; run += c; }
+    // bucket bases = exclusive prefix of the histogram (direct mode: every bucket has its own destination, base 0)
+    int bucketBase = 0;
+    if (!Ops::kDirect) {
+        const int h = lane < B ? hist[lane] : 0;
+        int incl = h;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
+        bucketBase = incl - h;
+        if (tile == 0) {
+            if (lane < B) offsets[lane] = bucketBase;
+            if (lane == B - 1) offsets[B] = incl;
+        }
+    }
+    // decoupled look-back, one chain per bucket
+    int excl = 0;
+    if (lane < B) {
+        volatile unsigned long long* st = tileState;
+        const unsigned long long g = (unsigned long long)gen << 32;
+        if (tile == 0) {
+            st[lane] = g | ST_INC | (uint32_t)run;
+        } else {
+            st[(size_t)tile * 32 + lane] = g | ST_AGG | (uint32_t)run;
+            int t = tile - 1;
+            for (;;) {
+                unsigned long long w;
+                do { w = st[(size_t)t * 32 + lane]; } while ((w >> 32) != gen);      // older generations: not written yet
+                const uint32_t v = (uint32_t)w;
+                excl += (int)(v & VAL_MASK);
+                if ((v & ST_MASK) == ST_INC) break;
+                t--;
+            }
+            st[(size_t)tile * 32 + lane] = g | ST_INC | (uint32_t)(excl + run);
+        }
+    }
+    return bucketBase + excl;
+}
 
 template <class Ops, int kItems>
 __global__ void __launch_bounds__(kThreads) partition_kernel(Ops ops, int n, const int32_t* __restrict__ hist,
@@ -145,47 +188,7 @@ __global__ void __launch_bounds__(kThreads) partition_kernel(Ops ops, int n, con
     }
     __syncthreads();
 
-    if (warp == 0) {
-        // exclusive scan over the 32 in-tile steps, lane = bucket
-        int run = 0;
-#pragma unroll 8
-        for (int s = 0; s < kSteps; s++) { const int c = s_cnt[s][lane]; s_cnt[s][lane] = run; run += c; }
-        // bucket bases = exclusive prefix of the histogram (direct mode: every bucket has its own destination, base 0)
-        int bucketBase = 0;
-        if (!Ops::kDirect) {
-            const int h = lane < B ? hist[lane] : 0;
-            int incl = h;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-            bucketBase = incl - h;
-            if (tile == 0) {
-                if (lane < B) offsets[lane] = bucketBase;
-                if (lane == B - 1) offsets[B] = incl;
-            }
-        }
-        // decoupled look-back, one chain per bucket
-        int excl = 0;
-        if (lane < B) {
-            volatile unsigned long long* st = tileState;
-            const unsigned long long g = (unsigned long long)gen << 32;
-            if (tile == 0) {
-                st[lane] = g | ST_INC | (uint32_t)run;
-            } else {
-                st[(size_t)tile * 32 + lane] = g | ST_AGG | (uint32_t)run;
-                int t = tile - 1;
-                for (;;) {
-                    unsigned long long w;
-                    do { w = st[(size_t)t * 32 + lane]; } while ((w >> 32) != gen);      // older generations: not written yet
-                    const uint32_t v = (uint32_t)w;
-                    excl += (int)(v & VAL_MASK);
-                    if ((v & ST_MASK) == ST_INC) break;
-                    t--;
-                }
-                st[(size_t)tile * 32 + lane] = g | ST_INC | (uint32_t)(excl + run);
-            }
-        }
-        s_base[lane] = bucketBase + excl;
-    }
+    if (warp == 0) s_base[lane] = tile_bucket_base<Ops, kSteps>(s_cnt, lane, B, tile, hist, offsets, tileState, gen);
     __syncthreads();
 
 #pragma unroll
@@ -207,11 +210,11 @@ __global__ void __launch_bounds__(kThreads) partition_kernel(Ops ops, int n, con
 // run of records that stay together (the usual case in a stable partition) leaves the SM as contiguous 512-byte stores,
 // to local HBM or to a peer's receive buffer behind NVLink. The per-thread LDG/STG.128 version above stays for the NN queries.
 
-constexpr int kStageTileDefault = 1024;
+constexpr int kStageTile = 1024;
 
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-template <class Ops, int kStageTile>
+template <class Ops>
 __global__ void __launch_bounds__(kThreads) partition_staged_kernel(Ops ops, int n, const int32_t* __restrict__ hist, int32_t* __restrict__ offsets,
                                                                      unsigned long long* tileState, uint32_t* tileCounter, uint32_t ticketBase,
                                                                      uint32_t gen) {
@@ -274,44 +277,7 @@ __global__ void __launch_bounds__(kThreads) partition_staged_kernel(Ops ops, int
     }
     __syncthreads();
 
-    if (warp == 0) {
-        int run = 0;
-#pragma unroll 8
-        for (int st = 0; st < kStageSteps; st++) { const int c = s_cnt[st][lane]; s_cnt[st][lane] = run; run += c; }
-        int bucketBase = 0;
-        if (!Ops::kDirect) {
-            const int h = lane < B ? hist[lane] : 0;
-            int incl = h;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-            bucketBase = incl - h;
-            if (tile == 0) {
-                if (lane < B) offsets[lane] = bucketBase;
-                if (lane == B - 1) offsets[B] = incl;
-            }
-        }
-        int excl = 0;
-        if (lane < B) {
-            volatile unsigned long long* st = tileState;
-            const unsigned long long g = (unsigned long long)gen << 32;
-            if (tile == 0) {
-                st[lane] = g | ST_INC | (uint32_t)run;
-            } else {
-                st[(size_t)tile * 32 + lane] = g | ST_AGG | (uint32_t)run;
-                int t = tile - 1;
-                for (;;) {
-                    unsigned long long wv;
-                    do { wv = st[(size_t)t * 32 + lane]; } while ((wv >> 32) != gen);
-                    const uint32_t v = (uint32_t)wv;
-                    excl += (int)(v & VAL_MASK);
-                    if ((v & ST_MASK) == ST_INC) break;
-                    t--;
-                }
-                st[(size_t)tile * 32 + lane] = g | ST_INC | (uint32_t)(excl + run);
-            }
-        }
-        s_base[lane] = bucketBase + excl;
-    }
+    if (warp == 0) s_base[lane] = tile_bucket_base<Ops, kStageSteps>(s_cnt, lane, B, tile, hist, offsets, tileState, gen);
     __syncthreads();
 
 #pragma unroll
@@ -382,29 +348,19 @@ void launch_path_histogram(const dprt_path_record* paths, int n, int W, int32_t*
 // DPRT_PARTITION_STAGED=1 selects the TMA-staged kernel for the path records. Off by default on the numbers
 // (profiles/ab_r2_partition_staged.txt): the kernel itself is 11 % faster (reorder 0.27 -> 0.31 of the HBM roofline), but
 // its 64 KiB of shared memory per CTA displace the trace kernels of the other samples in flight (different shared-memory
-// carve-out: the SMs have to drain), and the step gets 5 % slower.
-bool partition_staged() { static bool v = [] { const char* e = getenv("DPRT_PARTITION_STAGED"); return e && e[0] == '1'; }(); return v; }
-
-int partition_tile() { static int v = [] { const char* e = getenv("DPRT_PARTITION_TILE"); const int t = e ? atoi(e) : kStageTileDefault; return (t == 256 || t == 512 || t == 1024) ? t : kStageTileDefault; }(); return v; }
-
-template <class Ops, int TILE>
-void launch_partition_staged(Ops ops, int n, const int32_t* hist, int32_t* offsets, PartitionScratch& s, cudaStream_t stream) {
-    static bool once = [] { cudaFuncSetAttribute(partition_staged_kernel<Ops, TILE>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE * 64); return true; }();
-    (void)once;
-    const int tiles = (n + TILE - 1) / TILE;
-    s.generation++;
-    partition_staged_kernel<Ops, TILE><<<tiles, kThreads, TILE * 64, stream>>>(ops, n, hist, offsets, s.tileState, s.tileCounter, s.tickets, s.generation);
-    s.tickets += (uint32_t)tiles;
-}
+// carve-out: the SMs have to drain), and the step gets 5 % slower. Read on every launch, so that it can be switched within
+// one process.
+bool partition_staged() { const char* e = getenv("DPRT_PARTITION_STAGED"); return e && e[0] == '1'; }
 
 template <class Ops>
 void run_partition_staged(Ops ops, int n, const int32_t* hist, int32_t* offsets, PartitionScratch& s, cudaStream_t stream) {
     if (n <= 0) { if (!Ops::kDirect) empty_offsets_kernel<<<1, 64, 0, stream>>>(offsets, ops.B); return; }
-    switch (partition_tile()) {
-        case 256: launch_partition_staged<Ops, 256>(ops, n, hist, offsets, s, stream); break;
-        case 512: launch_partition_staged<Ops, 512>(ops, n, hist, offsets, s, stream); break;
-        default: launch_partition_staged<Ops, 1024>(ops, n, hist, offsets, s, stream); break;
-    }
+    static bool once = [] { cudaFuncSetAttribute(partition_staged_kernel<Ops>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStageTile * 64); return true; }();
+    (void)once;
+    const int tiles = (n + kStageTile - 1) / kStageTile;
+    s.generation++;
+    partition_staged_kernel<Ops><<<tiles, kThreads, kStageTile * 64, stream>>>(ops, n, hist, offsets, s.tileState, s.tileCounter, s.tickets, s.generation);
+    s.tickets += (uint32_t)tiles;
 }
 
 void launch_partition_paths(const dprt_path_record* paths, int n, int W, int B, int me, int splitL, const int32_t* hist,
@@ -425,12 +381,8 @@ cudaError_t partition_preload_kernels() {
     cudaFuncAttributes fa;
     cudaError_t e = cudaFuncGetAttributes(&fa, partition_kernel<PeerPathOps, 4>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_kernel<PathOps, 4>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PeerPathOps, 256>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PeerPathOps, 512>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PeerPathOps, 1024>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PathOps, 256>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PathOps, 512>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PathOps, 1024>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PeerPathOps>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, partition_staged_kernel<PathOps>);
     return e;
 }
 

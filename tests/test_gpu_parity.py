@@ -136,12 +136,15 @@ def test_multi_rank_group_migration_bit_exact(gpu_required, oracle, W, refmig):
     assert_bits_equal(G.reduce_image(0), world.image(), "reduced image")
 
 
+@pytest.mark.parametrize("staged", [0, 1])
 @pytest.mark.parametrize("W,spp,pgm", [(2, 1, 0), (3, 2, 1), (4, 2, 0)])
-def test_multi_rank_group_peer_memory_exchange_bit_exact(gpu_required, oracle, monkeypatch, W, spp, pgm):
+def test_multi_rank_group_peer_memory_exchange_bit_exact(gpu_required, oracle, monkeypatch, W, spp, pgm, staged):
     """The peer-memory exchange (p2p_exchange.cuh: counts kernel -> partition scattering straight into the owners' receive
     buffers -> flag barrier, no host round trip) driven for W contexts on one device: same kernels and protocol as one
-    process per GPU, with plain device pointers where those use CUDA IPC mappings. Every buffer bit-exact against the oracle."""
+    process per GPU, with plain device pointers where those use CUDA IPC mappings. Every buffer bit-exact against the oracle,
+    with the per-thread and with the TMA-staged partition (DPRT_PARTITION_STAGED)."""
     monkeypatch.setenv("DPRT_P2P_GROUP", "1")
+    monkeypatch.setenv("DPRT_PARTITION_STAGED", str(staged))
     rs, world, _ = build_pair(oracle, W, 6000, 128, 72, spp=spp, bounces=3, proxy_mode=0, path_gen_mode=pgm, serial_stages=1)
     G = dprt.RankGroup(rs)
     img_g, img_o = G.launch(), world.launch()
@@ -168,25 +171,30 @@ def test_striped_path_generation_same_image(gpu_required, oracle):
     assert_bits_equal(img_g, img_o, "striped path generation image")
 
 
-def test_partition_random_keys_against_oracle(gpu_required, oracle):
-    """Work_Efficient_Scan drop-in on arbitrary uploaded paths (histogram fallback path), W = 8, ragged sizes."""
+def test_partition_random_keys_against_oracle(gpu_required, oracle, monkeypatch):
+    """Work_Efficient_Scan drop-in on arbitrary uploaded paths (histogram fallback path), W = 8, ragged sizes: empty, partial
+    and multi-tile launches, with the per-thread and then the TMA-staged partition (DPRT_PARTITION_STAGED, read on every
+    launch) on the same context, so the staged kernel also picks up the tile state the per-thread one left."""
     W, w, h = 8, 256, 128
     cfg = dprt.make_config(w, h, scene_size=1)
     world = oracle.World(cfg, W)
     R = dprt.Renderer(cfg, rank=3, world=W)
     rng = np.random.default_rng(11)
-    for n in (0, 1, 31, 1024, 1025, 5000, w * h):
-        p = np.zeros(n, D.PATH_DTYPE)
-        p["pixelIndex"] = np.arange(n)
-        p["origin"] = rng.random((n, 3), dtype=np.float32)
-        p["isValid"] = rng.random(n) < 0.8
-        p["targetNode"] = rng.integers(-1, W + 1, n)
-        R.upload(D.BUF_PATHS, p); world.upload(3, D.BUF_PATHS, p)
-        R.set_path_size(n); world.set_path_size(3, n)
-        R.partition(); world.partition(3)
-        off_g, off_o = R.download(D.BUF_TRANSFER_OFFSET, W + 1), world.download(3, D.BUF_TRANSFER_OFFSET, W + 1)
-        assert_bits_equal(off_g, off_o, f"offsets n={n}")
-        assert_records_equal(R.download(D.BUF_TRANSFER, int(off_g[W])), world.download(3, D.BUF_TRANSFER, int(off_o[W])), f"transfer n={n}")
+    for staged in (0, 1):
+        monkeypatch.setenv("DPRT_PARTITION_STAGED", str(staged))
+        for n in (0, 1, 31, 1024, 1025, 5000, w * h):
+            p = np.zeros(n, D.PATH_DTYPE)
+            p["pixelIndex"] = np.arange(n)
+            p["origin"] = rng.random((n, 3), dtype=np.float32)
+            p["isValid"] = rng.random(n) < 0.8
+            p["targetNode"] = rng.integers(-1, W + 1, n)
+            R.upload(D.BUF_PATHS, p); world.upload(3, D.BUF_PATHS, p)
+            R.set_path_size(n); world.set_path_size(3, n)
+            R.partition(); world.partition(3)
+            off_g, off_o = R.download(D.BUF_TRANSFER_OFFSET, W + 1), world.download(3, D.BUF_TRANSFER_OFFSET, W + 1)
+            assert_bits_equal(off_g, off_o, f"offsets n={n} staged={staged}")
+            assert_records_equal(R.download(D.BUF_TRANSFER, int(off_g[W])), world.download(3, D.BUF_TRANSFER, int(off_o[W])),
+                                 f"transfer n={n} staged={staged}")
 
 
 @pytest.mark.parametrize("tris,nrays", [(1, 4096), (5000, 200000), (200000, 400000)])
