@@ -145,6 +145,22 @@ int  dprt_render_sample(dprt_ctx* ctx, int sample);   /* runSample              
  * elsewhere): renderer.cpp:2031-2052. */
 int  dprt_reduce_image(dprt_ctx* ctx, int root, float* out_host);
 
+/* ---- first-hit guide buffers (AOVs) for a denoiser ------------------------------------------------------------------
+ * The reference's launch() takes normalImage and albedoImage beside the colour image (renderer.cpp:1576-1589); the
+ * semantics here are this project's own (DESIGN.md 4). Off by default. dprt_enable_aov(ctx, 1) allocates, on the first
+ * enable, one zeroed buffer of 6N floats (DPRT_BUF_AOV: albedo sums 3N, then normal sums 3N), which dprt_reset_frame clears.
+ * Rule: dprt_begin_sample arms the context, and the first dprt_shade after it -- the camera paths' first surface hits on
+ * this rank -- adds, per hit record, the albedo the shading program uses (material baseColor or albedo-map texel) and the
+ * interpolated, normalised, face-forwarded shading normal to the record's pixel. Later dprt_shade calls of the sample add
+ * nothing; a camera ray that hits nothing adds nothing. The per-stage entry points and dprt_render_sample[_group] follow
+ * the same rule. dprt_accumulate_from adds the AOV sums too when both contexts have them on (DPRT_ERR_STATE when only one
+ * does). dprt_reduce_aov: albedo/spp and normal/spp on device (not renormalised), ncclReduce(sum) to root when W > 1,
+ * 3N floats each to albedo_host / normal_host on root (may be NULL elsewhere); collective like dprt_reduce_image.
+ * dprt_reduce_aov_group sums the ranks in rank order on the host. Both return DPRT_ERR_STATE when AOVs were never enabled. */
+int  dprt_enable_aov(dprt_ctx* ctx, int enable);
+int  dprt_reduce_aov(dprt_ctx* ctx, int root, float* albedo_host, float* normal_host);
+int  dprt_reduce_aov_group(dprt_ctx** ctxs, int world, int root, float* albedo_host, float* normal_host);
+
 /* ---- samples in flight ----------------------------------------------------------------------------
  * Samples of a frame are independent (renderer.cpp:1993-2022 runs them one after the other). The late bounces and the later
  * migrate iterations of a sample carry 10^4..10^5 rays -- launches that last as long as their longest ray and leave most of

@@ -229,7 +229,8 @@ enum dprt_buffer_id {
     DPRT_BUF_OCCLUSION = 11,   /* shadowOcclusionFloatTypeBuffer */
     DPRT_BUF_CONTRIBUTION = 12,
     DPRT_BUF_HIT_PRIM = 13,    /* parity aid: per path slot hit primitive id of the last trace */
-    DPRT_BUF_COUNT = 14
+    DPRT_BUF_AOV = 14,         /* first-hit guide buffers (dprt_enable_aov): albedo sums 3N floats, then normal sums 3N floats */
+    DPRT_BUF_COUNT = 15
 };
 
 /* Stage identifiers for dprt_get_stage_times / dprt_get_counters: one per reference call site of runSample. */

@@ -186,6 +186,9 @@ struct dprt_ctx {
     // `transfer` and MainRay shades it from there with the hits of the hit cache
     bool shortcut = false;
     bool recsInTransfer = false;        // set by such an exchange, consumed by the dprt_shade that follows
+    // first-hit guide buffers (dprt_enable_aov): buf_ptr[DPRT_BUF_AOV] while enabled, else null
+    float* d_aov = nullptr;
+    bool aovPending = false;            // armed by dprt_begin_sample, consumed by the dprt_shade that follows
     float* d_image = nullptr;           // averaged image, 3N
     float* d_image_sum = nullptr;       // reduce target, 3N
     int32_t* d_gather = nullptr;        // W*(W+1) offsets of all ranks
@@ -819,10 +822,15 @@ int dprt_adopt_scene(dprt_ctx* ctx, dprt_ctx* from) {
 int dprt_accumulate_from(dprt_ctx* ctx, dprt_ctx* other) {
     if (!ctx || !other || ctx == other) return DPRT_ERR_INVALID;
     if (ctx->device != other->device || ctx->N != other->N) return fail(ctx, DPRT_ERR_INVALID, "dprt_accumulate_from: same device and frame size required");
+    if (!ctx->d_aov != !other->d_aov) return fail(ctx, DPRT_ERR_STATE, "dprt_accumulate_from: AOVs are enabled on only one of the two contexts");
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(other->stream));              // other's samples are complete
     launch_accumulate(ctx->hp.direct, ctx->hp.env, other->hp.direct, other->hp.env, ctx->N * 3, ctx->stream);
     ctx->stats.kernel_launches += 1;
+    if (ctx->d_aov) {                                      // the albedo and normal planes, as one pair of planes
+        launch_accumulate(ctx->d_aov, ctx->d_aov + 3 * (size_t)ctx->N, other->d_aov, other->d_aov + 3 * (size_t)ctx->N, ctx->N * 3, ctx->stream);
+        ctx->stats.kernel_launches += 1;
+    }
     CK(cudaGetLastError());
     return 0;
 }
@@ -853,6 +861,7 @@ int dprt_reset_frame(dprt_ctx* ctx) {
     CK(cudaSetDevice(ctx->device));
     CK(cudaMemsetAsync(ctx->hp.direct, 0, ctx->buf_bytes[DPRT_BUF_DIRECT], ctx->stream));
     CK(cudaMemsetAsync(ctx->hp.env, 0, ctx->buf_bytes[DPRT_BUF_ENV], ctx->stream));
+    if (ctx->buf_ptr[DPRT_BUF_AOV]) CK(cudaMemsetAsync(ctx->buf_ptr[DPRT_BUF_AOV], 0, ctx->buf_bytes[DPRT_BUF_AOV], ctx->stream));
     // contribution / occlusion are only ever written by the proxy epilogues (and by dprt_upload, which raises nnScratchDirty):
     // with proxies off they are still the zeros of the allocation -- 1.6 GB of memset per frame at 5424x3056 not issued
     if (ctx->cfg.proxyMode || ctx->nnScratchDirty) {
@@ -868,6 +877,7 @@ int dprt_begin_sample(dprt_ctx* ctx, int sample) {
     CK(cudaSetDevice(ctx->device));
     ctx->sample = sample;
     ctx->epoch++;
+    ctx->aovPending = true;
     // resetSampleBuffers: offsets to zero. Path buffers are reset by count (slots >= pathSize are never read).
     CK(cudaMemsetAsync(ctx->hp.transferOffset, 0, 64 * sizeof(int32_t), ctx->stream));
     CK(cudaMemsetAsync(ctx->hp.sceneOffset, 0, 64 * sizeof(int32_t), ctx->stream));
@@ -1050,8 +1060,10 @@ int dprt_shade(dprt_ctx* ctx) {
     StageScope sc_(ctx, DPRT_STAGE_SHADE, ctx->pathSize > 0);
     const bool cached = ctx->recsInTransfer;
     ctx->recsInTransfer = false;
-    if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, ctx->stream);
-    else launch_shade(ctx->hp, ctx->pathSize, ctx->stream);
+    float* aov = ctx->aovPending ? ctx->d_aov : nullptr;     // the sample's first shade: the camera paths' first hits
+    ctx->aovPending = false;
+    if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, aov, ctx->stream);
+    else launch_shade(ctx->hp, ctx->pathSize, aov, ctx->stream);
     ctx->stats.kernel_launches += (cached ? 1 : 2) * (ctx->pathSize > 0);   // [trace +] post
     ctx->stats.rays_shade += ctx->pathSize;
     ctx->epoch++;                       // the records now hold the next bounce's rays: cached hits are stale
@@ -1832,6 +1844,54 @@ int dprt_reduce_image_group(dprt_ctx** ctxs, int W, int root, float* out_host) {
     return 0;
 }
 
+// The guide buffers go through the image's scratch (d_image, d_image_sum) one plane at a time: albedo, then normal.
+int dprt_reduce_aov(dprt_ctx* ctx, int root, float* albedo_host, float* normal_host) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!ctx->buf_ptr[DPRT_BUF_AOV]) return fail(ctx, DPRT_ERR_STATE, "dprt_reduce_aov: AOVs were never enabled (dprt_enable_aov)");
+    if (ctx->world > 1 && !ctx->comm) return fail(ctx, DPRT_ERR_STATE, "dprt_reduce_aov on a multi-rank context without an NCCL communicator");
+    CK(cudaSetDevice(ctx->device));
+    const int n3 = ctx->N * 3;
+    float* out[2] = {albedo_host, normal_host};
+    for (int plane = 0; plane < 2; plane++) {
+        const float* src = ctx->d_image;
+        {
+            StageScope sc_(ctx, DPRT_STAGE_IMAGE);
+            launch_aov_average((const float*)ctx->buf_ptr[DPRT_BUF_AOV] + (size_t)plane * n3, ctx->d_image, n3, (float)ctx->cfg.spp, ctx->stream);
+            ctx->stats.kernel_launches += 1;
+            if (ctx->world > 1) {
+                NK(g_nccl.Reduce(ctx->d_image, ctx->d_image_sum, n3, ncclFloat32, ncclSum, root, ctx->comm, ctx->stream));
+                src = ctx->d_image_sum;
+            }
+        }
+        if (ctx->rank == root && out[plane])
+            CK(cudaMemcpyAsync(out[plane], src, sizeof(float) * n3, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));       // the next plane reuses the scratch
+    }
+    return 0;
+}
+
+int dprt_reduce_aov_group(dprt_ctx** ctxs, int W, int root, float* albedo_host, float* normal_host) {
+    if (!ctxs || W < 1 || root < 0 || root >= W || !albedo_host || !normal_host) return DPRT_ERR_INVALID;
+    for (int k = 0; k < W; k++)
+        if (!ctxs[k]->buf_ptr[DPRT_BUF_AOV]) return fail(ctxs[k], DPRT_ERR_STATE, "dprt_reduce_aov_group: AOVs were never enabled (dprt_enable_aov)");
+    // rank-ordered fp32 sum on the host, like dprt_reduce_image_group
+    const int n3 = ctxs[0]->N * 3;
+    std::vector<float> tmp(n3);
+    float* out[2] = {albedo_host, normal_host};
+    for (int plane = 0; plane < 2; plane++) {
+        std::fill(out[plane], out[plane] + n3, 0.f);
+        for (int k = 0; k < W; k++) {
+            dprt_ctx* ctx = ctxs[k];
+            CK(cudaSetDevice(ctx->device));
+            launch_aov_average((const float*)ctx->buf_ptr[DPRT_BUF_AOV] + (size_t)plane * n3, ctx->d_image, n3, (float)ctx->cfg.spp, ctx->stream);
+            CK(cudaMemcpyAsync(tmp.data(), ctx->d_image, sizeof(float) * n3, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            for (int i = 0; i < n3; i++) out[plane][i] += tmp[i];
+        }
+    }
+    return 0;
+}
+
 // ---- state access ----------------------------------------------------------------------------------
 int dprt_get_path_size(const dprt_ctx* ctx, int* ps, int* sps) {
     if (!ctx) return DPRT_ERR_INVALID;
@@ -1878,6 +1938,16 @@ int dprt_enable_hit_prim(dprt_ctx* ctx, int enable) {
         if (r) return r;
     }
     ctx->hp.hitPrim = enable ? (int32_t*)ctx->buf_ptr[DPRT_BUF_HIT_PRIM] : nullptr;
+    return 0;
+}
+int dprt_enable_aov(dprt_ctx* ctx, int enable) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    CK(cudaSetDevice(ctx->device));
+    if (enable && !ctx->buf_ptr[DPRT_BUF_AOV]) {
+        int r = alloc_buf(ctx, DPRT_BUF_AOV, 6 * (size_t)ctx->N * sizeof(float));
+        if (r) return r;
+    }
+    ctx->d_aov = enable ? (float*)ctx->buf_ptr[DPRT_BUF_AOV] : nullptr;
     return 0;
 }
 

@@ -88,9 +88,10 @@ struct DevParams {
 // stage launches (all asynchronous on `stream`)
 void launch_path_gen(const DevParams& p, int n, cudaStream_t stream);
 void launch_traverse(const DevParams& p, int n, cudaStream_t stream);
-void launch_shade(const DevParams& p, int n, cudaStream_t stream);
+// aov: first-hit guide buffers (6N floats) to add to, or null (AOVs off, or not the sample's first shade)
+void launch_shade(const DevParams& p, int n, float* aov, cudaStream_t stream);
 // MainRay without its trace: shades the partition output p.transfer[0..n) with the hits of the hit cache (single rank only)
-void launch_shade_cached(const DevParams& p, int n, cudaStream_t stream);
+void launch_shade_cached(const DevParams& p, int n, float* aov, cudaStream_t stream);
 // proxies off: the any-hit trace also adds the unoccluded terms to directLightingBuffer and no post kernel follows
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t stream);
 void launch_secondary_trace(const DevParams& p, int n, cudaStream_t stream);
@@ -151,5 +152,7 @@ void launch_tmax(const DevParams& p, int size, cudaStream_t stream);
 void launch_target_node(const DevParams& p, int n, cudaStream_t stream);
 void launch_accumulate(float* direct, float* env, const float* direct2, const float* env2, int n3, cudaStream_t stream);
 void launch_image_average(const float* direct, const float* env, float* out, int n3, float invSpp, cudaStream_t stream);
+// out = sum / spp: one plane of the first-hit guide buffers
+void launch_aov_average(const float* sum, float* out, int n3, float spp, cudaStream_t stream);
 
 }  // namespace dprt

@@ -23,6 +23,9 @@
 //                                      -light-move (after a one-off +light-start, LIGHT_MOVE :1941-1966) and the camera origin by
 //                                      +camera-move (CAMERA_MOVE :1968-1983; re-aimed at --camera-target when given, else translated);
 //                                      frame f is written as <f><name> like std::to_string(cframe) + exrFilename (:2055-2058)
+//               [--aov 1]              also the first-hit guide buffers a denoiser takes beside the colour (dprt_enable_aov on every
+//                                      context, samples in flight included): <name>.albedo.<ext> and <name>.normal.<ext>, e.g.
+//                                      --out img.exr writes img.albedo.exr and img.normal.exr (<f>img.albedo.exr per frame f)
 //   dprt_render --convert in.pfm out.exr     no GPU: re-encode an image (the reference's Image::save writes EXR)
 //
 // Output on the root rank: OpenEXR (uncompressed scanlines, float32 B/G/R) when the name ends in .exr, else PFM (RGB float32,
@@ -177,6 +180,13 @@ bool read_pfm(const std::string& path, std::vector<float>& rgb, int& w, int& h) 
 bool ends_with(const std::string& s, const char* suf) { const size_t n = std::strlen(suf); return s.size() >= n && s.compare(s.size() - n, n, suf) == 0; }
 bool write_image(const std::string& path, const float* rgb, int w, int h) { return ends_with(path, ".exr") ? write_exr(path, rgb, w, h) : write_pfm(path, rgb, w, h); }
 
+// "<stem>.<tag><ext>": the guide buffer `tag` of the image `path` (img.exr -> img.albedo.exr; no extension: img -> img.albedo)
+std::string aov_name(const std::string& path, const char* tag) {
+    const size_t slash = path.find_last_of('/'), dot = path.find_last_of('.');
+    if (dot == std::string::npos || (slash != std::string::npos && dot < slash)) return path + "." + tag;
+    return path.substr(0, dot) + "." + tag + path.substr(dot);
+}
+
 // "<dir>/<frame><name>" like std::to_string(cframe) + exrFilename (renderer.cpp:2058)
 std::string frame_name(const std::string& path, int frame, int frames) {
     if (frames <= 1) return path;
@@ -274,7 +284,7 @@ int main(int argc, char** argv) {
     if (scenePath.empty()) {
         fprintf(stderr, "usage: dprt_render --scene S.dprt [--out image.pfm] [--spp n] [--bounces n] [--proxy 0|1] [--path-gen 0|1] "
                         "[--inflight K] [--world W | --nccl-id-file F] [--frames F] [--camera-move x,y,z] [--camera-target x,y,z] "
-                        "[--light-move x,y,z] [--light-start x,y,z]\n       dprt_render --convert in.pfm out.exr\n");
+                        "[--light-move x,y,z] [--light-start x,y,z] [--aov 0|1]\n       dprt_render --convert in.pfm out.exr\n");
         return 2;
     }
     Scene sc; std::string err;
@@ -304,6 +314,8 @@ int main(int argc, char** argv) {
     cfg.envColor[0] = 0.6f; cfg.envColor[1] = 0.7f; cfg.envColor[2] = 0.9f;
     const size_t N = (size_t)cfg.width * cfg.height;
     std::vector<float> image(3 * N);
+    const bool aov = std::atoi(arg(argc, argv, "--aov", "0")) != 0;
+    std::vector<float> albedo(aov ? 3 * N : 0), normal(aov ? 3 * N : 0);
     std::vector<dprt_ctx*> ctxs, extra;
     int inflight = std::atoi(arg(argc, argv, "--inflight", "1"));      // samples in flight per rank
     if (inflight < 1) inflight = 1;
@@ -339,9 +351,18 @@ int main(int argc, char** argv) {
     auto save_frame = [&](int frame) -> bool {
         if (rank != 0 || outPath.empty()) return true;
         const std::string name = frame_name(outPath, frame, frames);
-        if (write_image(name, image.data(), cfg.width, cfg.height)) return true;
-        fprintf(stderr, "dprt_render: cannot write %s\n", name.c_str());
-        return false;
+        bool ok = write_image(name, image.data(), cfg.width, cfg.height);
+        if (ok && aov) {
+            ok = write_image(frame_name(aov_name(outPath, "albedo"), frame, frames), albedo.data(), cfg.width, cfg.height) &&
+                 write_image(frame_name(aov_name(outPath, "normal"), frame, frames), normal.data(), cfg.width, cfg.height);
+        }
+        if (!ok) fprintf(stderr, "dprt_render: cannot write %s or its guide buffers\n", name.c_str());
+        return ok;
+    };
+    auto enable_aov = [&](const std::vector<dprt_ctx*>& all) -> int {
+        int rr = 0;
+        for (dprt_ctx* c : all) if (aov && (rr = dprt_enable_aov(c, 1))) return rr;
+        return 0;
     };
     // K - 1 more contexts of this rank on the same communicator, sharing the uploaded scene (collective across ranks)
     auto make_inflight = [&](dprt_ctx* ctx) -> int {
@@ -383,12 +404,15 @@ int main(int argc, char** argv) {
         if ((r = make_inflight(ctx))) return die("samples in flight", nullptr, r);
         std::vector<dprt_ctx*> all{ctx};
         all.insert(all.end(), extra.begin(), extra.end());
+        if ((r = enable_aov(all))) return die("dprt_enable_aov", ctx, r);
         for (int frame = 0; frame < frames; frame++) {
             if ((r = advance_frame(frame, all))) return die("frame setup", ctx, r);
             const auto t0 = std::chrono::steady_clock::now();
             for (dprt_ctx* c : all) if ((r = dprt_reset_frame(c))) return die("dprt_reset_frame", c, r);
             { const char* what = ""; dprt_ctx* bad = ctx; if ((r = render_samples(ctx, extra, cfg.spp, &what, &bad))) return die(what, bad, r); }
             if ((r = dprt_reduce_image(ctx, 0, rank == 0 ? image.data() : nullptr))) return die("dprt_reduce_image", ctx, r);
+            if (aov && (r = dprt_reduce_aov(ctx, 0, rank == 0 ? albedo.data() : nullptr, rank == 0 ? normal.data() : nullptr)))
+                return die("dprt_reduce_aov", ctx, r);
             const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
             dprt_stats st; dprt_get_stats(ctx, &st);
             printf("{\"frame\": %d, \"rank\": %d, \"world\": %d, \"seconds\": %.6f, \"rays_walked\": %lld, \"paths_sent_offrank\": %lld, \"exchange_iters\": %lld}\n",
@@ -407,6 +431,7 @@ int main(int argc, char** argv) {
         if (world == 1 && (r = make_inflight(ctxs[0]))) return die("samples in flight", nullptr, r);
         std::vector<dprt_ctx*> all(ctxs);
         all.insert(all.end(), extra.begin(), extra.end());
+        if ((r = enable_aov(all))) return die("dprt_enable_aov", ctxs[0], r);
         for (int frame = 0; frame < frames; frame++) {
             if ((r = advance_frame(frame, all))) return die("frame setup", ctxs[0], r);
             const auto t0 = std::chrono::steady_clock::now();
@@ -420,6 +445,11 @@ int main(int argc, char** argv) {
             }
             r = world == 1 ? dprt_reduce_image(ctxs[0], 0, image.data()) : dprt_reduce_image_group(ctxs.data(), world, 0, image.data());
             if (r) return die("dprt_reduce_image", ctxs[0], r);
+            if (aov) {
+                r = world == 1 ? dprt_reduce_aov(ctxs[0], 0, albedo.data(), normal.data())
+                               : dprt_reduce_aov_group(ctxs.data(), world, 0, albedo.data(), normal.data());
+                if (r) return die("dprt_reduce_aov", ctxs[0], r);
+            }
             const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
             long long walked = 0, sent = 0;
             for (int k = 0; k < world; k++) { dprt_stats st; dprt_get_stats(ctxs[k], &st); walked += st.rays_walked; sent += st.paths_sent_offrank; }

@@ -142,6 +142,10 @@ __global__ void image_average_kernel(const float* __restrict__ direct, const flo
         out[i] = (direct[i] + env[i]) / spp;
 }
 
+__global__ void aov_average_kernel(const float* __restrict__ sum, float* __restrict__ out, int n3, float spp) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n3; i += gridDim.x * blockDim.x) out[i] = sum[i] / spp;
+}
+
 }  // namespace
 
 void launch_shadow_occlusion(const DevParams& p, int size, cudaStream_t s) {
@@ -181,6 +185,9 @@ void launch_accumulate(float* direct, float* env, const float* direct2, const fl
 }
 void launch_image_average(const float* direct, const float* env, float* out, int n3, float spp, cudaStream_t s) {
     if (n3 > 0) image_average_kernel<<<grid_for(n3), kBlock, 0, s>>>(direct, env, out, n3, spp);
+}
+void launch_aov_average(const float* sum, float* out, int n3, float spp, cudaStream_t s) {
+    if (n3 > 0) aov_average_kernel<<<grid_for(n3), kBlock, 0, s>>>(sum, out, n3, spp);
 }
 
 }  // namespace dprt

@@ -494,7 +494,11 @@ DPRT_D BsdfSample sample_water(float xi1, V3 normal, V3 woWorld, bool isInside) 
 // generateNextNewPath (:134-162), generateShadowPath x spc (:66-132, :442-465).
 // src: the records to shade (paths, or the partition output when the single-rank bounce skips the copy back). fromCache: the
 // hit comes from the hit cache under the record's pixel instead of hits[i] (the MainRay trace was not launched).
-__global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, const dprt_path_record* src, bool fromCache) {
+// aov: the first-hit guide buffers (albedo sums 3N, normal sums 3N) when this is the sample's first shade with AOVs on, else
+// null. A kernel argument rather than a DevParams field, so that no other kernel's parameters move. At most one record per
+// pixel reaches the first shade of a sample on a rank, and only the rank that owns the hit shades it: plain adds, no race.
+__global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, const dprt_path_record* src, bool fromCache,
+                                                            float* aov) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) p.traceQueue[0] = 0;
     if (i >= n) return;
@@ -556,6 +560,12 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
     }
     bool isInside = false;
     if (v3dot(normal, woWorld) < 0.0f) { normal = v3neg(normal); isInside = true; }
+    if (aov) {
+        float* a = aov + 3 * (size_t)path.pixelIndex;
+        float* nrm = a + 3 * (size_t)p.frameBufferSize;
+        a[0] += albedo.x; a[1] += albedo.y; a[2] += albedo.z;
+        nrm[0] += normal.x; nrm[1] += normal.y; nrm[2] += normal.z;
+    }
     // createSamplingRecord (kernel.cu:50-64): the seed ignores the bounce, as in the reference
     uint32_t seed = tea4((uint32_t)path.pixelIndex, (uint32_t)p.sampleCount);
     const float xi1 = rnd(seed), xi2 = rnd(seed);
@@ -914,13 +924,13 @@ void launch_traverse(const DevParams& p, int n, cudaStream_t s) {
     launch_trace<TM_TRAVERSE>(trace_args(p, p.paths), n, s);
     traverse_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n);
 }
-void launch_shade(const DevParams& p, int n, cudaStream_t s) {
+void launch_shade(const DevParams& p, int n, float* aov, cudaStream_t s) {
     if (n <= 0) return;
     launch_trace<TM_SHADE>(trace_args(p, p.paths), n, s);
-    shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.paths, false);
+    shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.paths, false, aov);
 }
-void launch_shade_cached(const DevParams& p, int n, cudaStream_t s) {
-    if (n > 0) shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.transfer, true);
+void launch_shade_cached(const DevParams& p, int n, float* aov, cudaStream_t s) {
+    if (n > 0) shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.transfer, true, aov);
 }
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t s) {
     if (nShadow <= 0) return;

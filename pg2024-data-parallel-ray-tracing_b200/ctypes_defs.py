@@ -115,7 +115,7 @@ P2P_HANDLE_BYTES = 208     # DPRT_P2P_HANDLE_BYTES
 
 # dprt_buffer_id
 BUF_PATHS, BUF_TRANSFER, BUF_TRANSFER_OFFSET, BUF_DIRECT, BUF_ENV, BUF_NN_INPUT, BUF_NN_QUERY, BUF_NN_PACKED_INPUT, \
-    BUF_NN_PACKED_QUERY, BUF_SCENE_OFFSET, BUF_PRED, BUF_OCCLUSION, BUF_CONTRIBUTION, BUF_HIT_PRIM = range(14)
+    BUF_NN_PACKED_QUERY, BUF_SCENE_OFFSET, BUF_PRED, BUF_OCCLUSION, BUF_CONTRIBUTION, BUF_HIT_PRIM, BUF_AOV = range(15)
 
 # dprt_stage_id
 STAGE_NAMES = ("path_gen", "traverse", "partition", "exchange", "shade", "shadow_trace", "secondary_trace", "bucket",
@@ -126,7 +126,7 @@ BUFFER_DTYPES = {
     BUF_PATHS: PATH_DTYPE, BUF_TRANSFER: PATH_DTYPE, BUF_TRANSFER_OFFSET: np.dtype("<i4"), BUF_DIRECT: np.dtype("<f4"),
     BUF_ENV: np.dtype("<f4"), BUF_NN_INPUT: np.dtype("<u2"), BUF_NN_QUERY: QUERY_DTYPE, BUF_NN_PACKED_INPUT: np.dtype("<u2"),
     BUF_NN_PACKED_QUERY: QUERY_DTYPE, BUF_SCENE_OFFSET: np.dtype("<i4"), BUF_PRED: np.dtype("<u2"),
-    BUF_OCCLUSION: np.dtype("<f4"), BUF_CONTRIBUTION: np.dtype("<f4"), BUF_HIT_PRIM: np.dtype("<i4"),
+    BUF_OCCLUSION: np.dtype("<f4"), BUF_CONTRIBUTION: np.dtype("<f4"), BUF_HIT_PRIM: np.dtype("<i4"), BUF_AOV: np.dtype("<f4"),
 }
 
 

@@ -70,6 +70,9 @@ _PROTOTYPES = {
     "dprt_secondary_ray_module": (C.c_int, [C.c_void_p]),
     "dprt_render_sample": (C.c_int, [C.c_void_p, C.c_int]),
     "dprt_reduce_image": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "dprt_enable_aov": (C.c_int, [C.c_void_p, C.c_int]),
+    "dprt_reduce_aov": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "dprt_reduce_aov_group": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "dprt_adopt_scene": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dprt_accumulate_from": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dprt_p2p_export": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -509,6 +512,19 @@ class Renderer:
         self._ck(self.lib.dprt_reduce_image(self.h, root, _ptr(out)), "dprt_reduce_image")
         return out
 
+    def enable_aov(self, enable=True):
+        """dprt_enable_aov: accumulate the first-hit albedo and shading normal of every sample (the guide buffers a denoiser
+        takes beside the colour; dprt.h has the rule). Off by default; the first enable allocates the buffer."""
+        self._ck(self.lib.dprt_enable_aov(self.h, int(enable)), "dprt_enable_aov")
+
+    def reduce_aov(self, root=0):
+        """dprt_reduce_aov (collective): (albedo, normal), each [H, W, 3] float32 = sum / spp over the ranks, on root; None
+        elsewhere. The averaged normal is not renormalised."""
+        shape = (self.cfg.height, self.cfg.width, 3)
+        a, n = (np.zeros(shape, np.float32), np.zeros(shape, np.float32)) if self.rank == root else (None, None)
+        self._ck(self.lib.dprt_reduce_aov(self.h, root, _ptr(a), _ptr(n)), "dprt_reduce_aov")
+        return (a, n) if self.rank == root else None
+
     def launch(self):
         """Renderer::launch (renderer.cpp:1576): reset, spp x runSample, average + reduce to rank 0."""
         self.reset_frame()
@@ -680,8 +696,17 @@ class SamplesInFlight:
             raise errs[0]
 
     def accumulate(self):
+        """Adds every other context's sums into the primary's: colour, and the AOVs when they are on."""
         for R in self.ctxs[1:]:
             self.primary._ck(self.primary.lib.dprt_accumulate_from(self.primary.h, R.h), "dprt_accumulate_from")
+
+    def enable_aov(self, enable=True):
+        for R in self.ctxs:
+            R.enable_aov(enable)
+
+    def reduce_aov(self, root=0):
+        """The frame's AOVs after launch() (whose accumulate() brought every context's sums to the primary)."""
+        return self.primary.reduce_aov(root)
 
     def launch(self):
         """Renderer.launch with the samples in flight: reset, spp samples, accumulate, average + reduce."""
@@ -724,6 +749,17 @@ class RankGroup:
         out = np.zeros((cfg.height, cfg.width, 3), np.float32)
         self.rs[0]._ck(self.lib.dprt_reduce_image_group(self.arr, len(self.rs), root, _ptr(out)), "dprt_reduce_image_group")
         return out
+
+    def enable_aov(self, enable=True):
+        for r in self.rs:
+            r.enable_aov(enable)
+
+    def reduce_aov(self, root=0):
+        """(albedo, normal), each [H, W, 3]: per rank sum / spp, summed over the ranks in rank order."""
+        cfg = self.rs[0].cfg
+        a, n = np.zeros((cfg.height, cfg.width, 3), np.float32), np.zeros((cfg.height, cfg.width, 3), np.float32)
+        self.rs[0]._ck(self.lib.dprt_reduce_aov_group(self.arr, len(self.rs), root, _ptr(a), _ptr(n)), "dprt_reduce_aov_group")
+        return a, n
 
     def launch(self):
         for r in self.rs:
