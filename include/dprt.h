@@ -161,6 +161,26 @@ int  dprt_enable_aov(dprt_ctx* ctx, int enable);
 int  dprt_reduce_aov(dprt_ctx* ctx, int root, float* albedo_host, float* normal_host);
 int  dprt_reduce_aov_group(dprt_ctx** ctxs, int world, int root, float* albedo_host, float* normal_host);
 
+/* ---- denoiser: edge-avoiding a-trous wavelet filter guided by the first-hit albedo and normal --------------------------
+ * The reference hands its colour, albedo and normal images to OptiX's denoiser (renderer.cpp:1576-1589); this build has no
+ * OptiX, so it filters them itself (Dammertz et al. 2010, on albedo-demodulated colour; DESIGN.md 3.8 is the arithmetic
+ * specification, bit for bit on GPU and host). Inputs are width x height pixels of 3 floats each, pixel (x, y) at
+ * y * width + x: the layouts dprt_reduce_image and dprt_reduce_aov return. p == NULL selects the defaults: iterations 3,
+ * sigma_color 2.0, sigma_normal 1.0, sigma_albedo 0.3 (DPRT_DENOISE_DEFAULT_*). The output may alias any input.
+ * DPRT_ERR_INVALID, with nothing enqueued: a null context or array, width or height < 1, more than DPRT_DENOISE_MAX_PIXELS
+ * pixels, iterations outside 1..10, a sigma that is not finite and > 0, or one whose weight constant 4^(L-1) / sigma_color^2,
+ * 1 / sigma_normal^2 or 1 / sigma_albedo^2 is not finite and > 0 in binary32.
+ * dprt_denoise / dprt_denoise_device run on the context's device and stream (the frame size need not be the context's;
+ * not collective: call it on whichever rank holds the reduced frame) and return after the stream is synchronised. The
+ * context keeps the scratch (56 bytes per pixel), grown to the largest call and freed by dprt_destroy; never allocated
+ * when the denoiser is not used. dprt_spec_denoise runs the same arithmetic on the host, without a device. */
+int  dprt_denoise(dprt_ctx* ctx, const dprt_denoise_params* p, int width, int height, const float* color_host,
+                  const float* albedo_host, const float* normal_host, float* out_host);
+int  dprt_denoise_device(dprt_ctx* ctx, const dprt_denoise_params* p, int width, int height, const void* color_dev,
+                         const void* albedo_dev, const void* normal_dev, void* out_dev);
+int  dprt_spec_denoise(const dprt_denoise_params* p, int width, int height, const float* color, const float* albedo,
+                       const float* normal, float* out);
+
 /* ---- samples in flight ----------------------------------------------------------------------------
  * Samples of a frame are independent (renderer.cpp:1993-2022 runs them one after the other). The late bounces and the later
  * migrate iterations of a sample carry 10^4..10^5 rays -- launches that last as long as their longest ray and leave most of

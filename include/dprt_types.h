@@ -166,6 +166,20 @@ typedef struct dprt_hit {
     int32_t primID;           /* original triangle index, -1 = miss */
 } dprt_hit;
 
+/* Edge-avoiding a-trous denoiser (dprt_denoise, DESIGN.md 3.8). NULL parameters select the defaults below. */
+typedef struct dprt_denoise_params {
+    int32_t iterations;       /* L in 1..DPRT_DENOISE_MAX_ITERATIONS; iteration i reads taps 2^i pixels apart */
+    float sigma_color;        /* colour (albedo-demodulated) edge-stopping sigma of iteration 0; halves every iteration */
+    float sigma_normal;
+    float sigma_albedo;
+} dprt_denoise_params;
+#define DPRT_DENOISE_MAX_ITERATIONS 10
+#define DPRT_DENOISE_MAX_PIXELS (1 << 28)
+#define DPRT_DENOISE_DEFAULT_ITERATIONS 3        /* defaults: the CPU quality study of profiles/denoise_quality.txt */
+#define DPRT_DENOISE_DEFAULT_SIGMA_COLOR 2.0f
+#define DPRT_DENOISE_DEFAULT_SIGMA_NORMAL 1.0f
+#define DPRT_DENOISE_DEFAULT_SIGMA_ALBEDO 0.3f
+
 /* Compressed wide BVH node, 80 bytes (Ylitie, Karras, Laine 2017 layout). */
 typedef struct dprt_bvh8_node {
     float    p[3];

@@ -195,6 +195,7 @@ struct dprt_ctx {
     int32_t* h_pinned = nullptr;        // pinned staging for counts/offsets
     void* d_flush = nullptr; size_t flush_bytes = 0;
     void* d_io = nullptr; size_t io_bytes = 0;   // staging for the standalone host-buffer operators
+    void* d_denoise = nullptr; size_t denoise_bytes = 0;   // denoiser scratch (dprt_denoise_device): grown to the largest frame
     int pathSize = 0, shadowPathSize = 0;
     int sample = 0;
     int queryTotal = 0;                 // rows of the last bucketing
@@ -549,6 +550,7 @@ void dprt_destroy(dprt_ctx* ctx) {
     if (ctx->d_counters) cudaFree(ctx->d_counters);
     if (ctx->d_flush) cudaFree(ctx->d_flush);
     if (ctx->d_io) cudaFree(ctx->d_io);
+    if (ctx->d_denoise) cudaFree(ctx->d_denoise);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -2061,6 +2063,60 @@ int dprt_mlp_infer(dprt_ctx* ctx, int si, int kind, const dprt_half* x_host, int
     CK(cudaMemcpyAsync(y_host, d + xb, yb, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+
+// ---- denoiser (denoise.cu, DESIGN.md 3.8) -------------------------------------------------------------------------------
+int dprt_denoise_device(dprt_ctx* ctx, const dprt_denoise_params* p, int width, int height, const void* color_dev,
+                        const void* albedo_dev, const void* normal_dev, void* out_dev) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!color_dev || !albedo_dev || !normal_dev || !out_dev) return fail(ctx, DPRT_ERR_INVALID, "dprt_denoise_device: null array");
+    dprt_denoise_params q;
+    const char* why = nullptr;
+    if (denoise_check(p, width, height, &q, &why)) return fail(ctx, DPRT_ERR_INVALID, std::string("dprt_denoise_device: ") + why);
+    CK(cudaSetDevice(ctx->device));
+    const size_t bytes = denoise_scratch_bytes((int64_t)width * height);
+    if (ctx->denoise_bytes < bytes) {
+        void* old = ctx->d_denoise;
+        ctx->d_denoise = nullptr; ctx->denoise_bytes = 0;
+        if (old) { CK(cudaStreamSynchronize(ctx->stream)); CK(cudaFree(old)); }
+        CK(cudaMalloc(&ctx->d_denoise, bytes));
+        ctx->denoise_bytes = bytes;
+    }
+    launch_denoise(q, width, height, (const float*)color_dev, (const float*)albedo_dev, (const float*)normal_dev, (float*)out_dev,
+                   ctx->d_denoise, ctx->stream);
+    ctx->stats.kernel_launches += 1 + q.iterations;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int dprt_denoise(dprt_ctx* ctx, const dprt_denoise_params* p, int width, int height, const float* color_host, const float* albedo_host,
+                 const float* normal_host, float* out_host) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!color_host || !albedo_host || !normal_host || !out_host) return fail(ctx, DPRT_ERR_INVALID, "dprt_denoise: null array");
+    dprt_denoise_params q;
+    const char* why = nullptr;
+    if (denoise_check(p, width, height, &q, &why)) return fail(ctx, DPRT_ERR_INVALID, std::string("dprt_denoise: ") + why);
+    CK(cudaSetDevice(ctx->device));
+    const size_t b = (size_t)width * height * 3 * sizeof(float), bs = (b + 255) & ~(size_t)255;
+    int r = ensure_io(ctx, 3 * bs); if (r) return r;
+    char* d = (char*)ctx->d_io;
+    CK(cudaMemcpyAsync(d, color_host, b, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d + bs, albedo_host, b, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d + 2 * bs, normal_host, b, cudaMemcpyHostToDevice, ctx->stream));
+    if ((r = dprt_denoise_device(ctx, &q, width, height, d, d + bs, d + 2 * bs, d))) return r;     // the result over the colour
+    CK(cudaMemcpyAsync(out_host, d, b, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int dprt_spec_denoise(const dprt_denoise_params* p, int width, int height, const float* color, const float* albedo, const float* normal,
+                      float* out) {
+    if (!color || !albedo || !normal || !out) return DPRT_ERR_INVALID;
+    dprt_denoise_params q;
+    const char* why = nullptr;
+    if (denoise_check(p, width, height, &q, &why)) return DPRT_ERR_INVALID;
+    return spec_denoise(q, width, height, color, albedo, normal, out);
 }
 
 int dprt_device_alloc(dprt_ctx* ctx, size_t bytes, void** dev_ptr) {

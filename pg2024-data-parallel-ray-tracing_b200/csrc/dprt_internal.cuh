@@ -113,6 +113,15 @@ void launch_precom_labels(const DevObject* obj, const dprt_hit* hits, const floa
 int spec_texture_sample(const float* rgba, int width, int height, const float* u, const float* v, int64_t n, int clampV, float* out4);
 int spec_env_lookup(const float* rgba, int width, int height, float rotationOffset, const float* dirs3, int64_t n, float* out3);
 
+// denoiser (denoise.cu, DESIGN.md 3.8). denoise_check resolves p (NULL: the defaults) into *out and checks the frame size and
+// parameters: DPRT_ERR_INVALID with the reason in *why. launch_denoise enqueues the pack launch and one launch per iteration on
+// `stream` (scratch: denoise_scratch_bytes(width * height)); out may alias any input. spec_denoise: the same on the host.
+int denoise_check(const dprt_denoise_params* p, int width, int height, dprt_denoise_params* out, const char** why);
+size_t denoise_scratch_bytes(int64_t pixels);
+void launch_denoise(const dprt_denoise_params& p, int width, int height, const float* color, const float* albedo, const float* normal,
+                    float* out, void* scratch, cudaStream_t stream);
+int spec_denoise(const dprt_denoise_params& p, int width, int height, const float* color, const float* albedo, const float* normal, float* out);
+
 // partition / bucketing (partition.cu)
 struct PartitionScratch {
     unsigned long long* tileState; // tiles * 32 words {generation, status | value}; zeroed once at allocation, never cleared

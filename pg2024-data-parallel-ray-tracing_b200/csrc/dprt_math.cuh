@@ -101,6 +101,20 @@ DPRT_HD float det_atan2(float y, float x) {
     if (x < 0.0f) a = PI - a;
     return (y < 0.0f) ? -a : a;
 }
+// e^-x for x >= 0 (the denoiser's edge-stopping weights, DESIGN.md 3.8). x = n ln2 + r with n = floor(x log2(e) + 0.5) and
+// r in about [-ln2/2, ln2/2] (Cody-Waite: ln2 = 0.693359375 - 2.12194440e-4, the first part exact in n * 0.693359375);
+// e^-r from the Cephes expf polynomial, then ldexpf(., -n). Exactly 1 at 0; 0 when !(x < 88) (NaN included).
+// Against exp(): relative error below 1e-7 while the result is normal (x < 87.33), below one subnormal ulp beyond; the
+// result is non-increasing in x (tests/test_denoise_cpu.py checks both on a dense grid).
+DPRT_HD float det_exp_neg(float x) {
+    if (!(x < 88.0f)) return 0.0f;
+    const float n = floorf(fmaf(x, 1.44269504088896341f, 0.5f));
+    const float y = -((n * -0.693359375f + x) - n * -2.12194440e-4f);
+    const float z = y * y;
+    const float p = fmaf(fmaf(fmaf(fmaf(fmaf(1.9875691500e-4f, y, 1.3981999507e-3f), y, 8.3334519073e-3f), y, 4.1665795894e-2f), y,
+                             1.6666665459e-1f), y, 5.0000001201e-1f);
+    return ldexpf(fmaf(p, z, y) + 1.0f, -(int)n);
+}
 // Coordinates::cartesianToSpherical (+ForTrain, same convention: src/cuda/bvh_intersection.cu:18-26):
 // phi = atan2(y,x) wrapped to [0,2pi), theta = acos(clamp(z,-1,1)).
 DPRT_HD void det_cartesian_to_spherical(V3 d, float* phi, float* theta) {

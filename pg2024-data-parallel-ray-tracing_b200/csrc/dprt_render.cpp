@@ -26,6 +26,8 @@
 //               [--aov 1]              also the first-hit guide buffers a denoiser takes beside the colour (dprt_enable_aov on every
 //                                      context, samples in flight included): <name>.albedo.<ext> and <name>.normal.<ext>, e.g.
 //                                      --out img.exr writes img.albedo.exr and img.normal.exr (<f>img.albedo.exr per frame f)
+//               [--denoise 1]          also the frame filtered by dprt_denoise (default parameters) with those guide buffers (turned
+//                                      on for it as --aov 1 does, but written only with --aov 1): <name>.denoised.<ext>
 //   dprt_render --convert in.pfm out.exr     no GPU: re-encode an image (the reference's Image::save writes EXR)
 //
 // Output on the root rank: OpenEXR (uncompressed scanlines, float32 B/G/R) when the name ends in .exr, else PFM (RGB float32,
@@ -284,7 +286,7 @@ int main(int argc, char** argv) {
     if (scenePath.empty()) {
         fprintf(stderr, "usage: dprt_render --scene S.dprt [--out image.pfm] [--spp n] [--bounces n] [--proxy 0|1] [--path-gen 0|1] "
                         "[--inflight K] [--world W | --nccl-id-file F] [--frames F] [--camera-move x,y,z] [--camera-target x,y,z] "
-                        "[--light-move x,y,z] [--light-start x,y,z] [--aov 0|1]\n       dprt_render --convert in.pfm out.exr\n");
+                        "[--light-move x,y,z] [--light-start x,y,z] [--aov 0|1] [--denoise 0|1]\n       dprt_render --convert in.pfm out.exr\n");
         return 2;
     }
     Scene sc; std::string err;
@@ -315,7 +317,9 @@ int main(int argc, char** argv) {
     const size_t N = (size_t)cfg.width * cfg.height;
     std::vector<float> image(3 * N);
     const bool aov = std::atoi(arg(argc, argv, "--aov", "0")) != 0;
-    std::vector<float> albedo(aov ? 3 * N : 0), normal(aov ? 3 * N : 0);
+    const bool denoise = std::atoi(arg(argc, argv, "--denoise", "0")) != 0;
+    const bool guides = aov || denoise;                                 // the denoiser filters with the guide buffers
+    std::vector<float> albedo(guides ? 3 * N : 0), normal(guides ? 3 * N : 0), denoised(denoise ? 3 * N : 0);
     std::vector<dprt_ctx*> ctxs, extra;
     int inflight = std::atoi(arg(argc, argv, "--inflight", "1"));      // samples in flight per rank
     if (inflight < 1) inflight = 1;
@@ -356,12 +360,13 @@ int main(int argc, char** argv) {
             ok = write_image(frame_name(aov_name(outPath, "albedo"), frame, frames), albedo.data(), cfg.width, cfg.height) &&
                  write_image(frame_name(aov_name(outPath, "normal"), frame, frames), normal.data(), cfg.width, cfg.height);
         }
-        if (!ok) fprintf(stderr, "dprt_render: cannot write %s or its guide buffers\n", name.c_str());
+        if (ok && denoise) ok = write_image(frame_name(aov_name(outPath, "denoised"), frame, frames), denoised.data(), cfg.width, cfg.height);
+        if (!ok) fprintf(stderr, "dprt_render: cannot write %s, its guide buffers or its denoised image\n", name.c_str());
         return ok;
     };
     auto enable_aov = [&](const std::vector<dprt_ctx*>& all) -> int {
         int rr = 0;
-        for (dprt_ctx* c : all) if (aov && (rr = dprt_enable_aov(c, 1))) return rr;
+        for (dprt_ctx* c : all) if (guides && (rr = dprt_enable_aov(c, 1))) return rr;
         return 0;
     };
     // K - 1 more contexts of this rank on the same communicator, sharing the uploaded scene (collective across ranks)
@@ -411,8 +416,10 @@ int main(int argc, char** argv) {
             for (dprt_ctx* c : all) if ((r = dprt_reset_frame(c))) return die("dprt_reset_frame", c, r);
             { const char* what = ""; dprt_ctx* bad = ctx; if ((r = render_samples(ctx, extra, cfg.spp, &what, &bad))) return die(what, bad, r); }
             if ((r = dprt_reduce_image(ctx, 0, rank == 0 ? image.data() : nullptr))) return die("dprt_reduce_image", ctx, r);
-            if (aov && (r = dprt_reduce_aov(ctx, 0, rank == 0 ? albedo.data() : nullptr, rank == 0 ? normal.data() : nullptr)))
+            if (guides && (r = dprt_reduce_aov(ctx, 0, rank == 0 ? albedo.data() : nullptr, rank == 0 ? normal.data() : nullptr)))
                 return die("dprt_reduce_aov", ctx, r);
+            if (denoise && rank == 0 && (r = dprt_denoise(ctx, nullptr, cfg.width, cfg.height, image.data(), albedo.data(), normal.data(), denoised.data())))
+                return die("dprt_denoise", ctx, r);
             const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
             dprt_stats st; dprt_get_stats(ctx, &st);
             printf("{\"frame\": %d, \"rank\": %d, \"world\": %d, \"seconds\": %.6f, \"rays_walked\": %lld, \"paths_sent_offrank\": %lld, \"exchange_iters\": %lld}\n",
@@ -445,11 +452,13 @@ int main(int argc, char** argv) {
             }
             r = world == 1 ? dprt_reduce_image(ctxs[0], 0, image.data()) : dprt_reduce_image_group(ctxs.data(), world, 0, image.data());
             if (r) return die("dprt_reduce_image", ctxs[0], r);
-            if (aov) {
+            if (guides) {
                 r = world == 1 ? dprt_reduce_aov(ctxs[0], 0, albedo.data(), normal.data())
                                : dprt_reduce_aov_group(ctxs.data(), world, 0, albedo.data(), normal.data());
                 if (r) return die("dprt_reduce_aov", ctxs[0], r);
             }
+            if (denoise && (r = dprt_denoise(ctxs[0], nullptr, cfg.width, cfg.height, image.data(), albedo.data(), normal.data(), denoised.data())))
+                return die("dprt_denoise", ctxs[0], r);
             const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
             long long walked = 0, sent = 0;
             for (int k = 0; k < world; k++) { dprt_stats st; dprt_get_stats(ctxs[k], &st); walked += st.rays_walked; sent += st.paths_sent_offrank; }

@@ -41,6 +41,15 @@ class InstanceDesc(C.Structure):
     _fields_ = [("mesh", C.c_int32), ("pad_", C.c_int32), ("objectToWorld", C.c_float * 12)]
 
 
+class DenoiseParams(C.Structure):
+    """dprt_denoise_params (DESIGN.md 3.8)."""
+    _fields_ = [("iterations", C.c_int32), ("sigma_color", C.c_float), ("sigma_normal", C.c_float), ("sigma_albedo", C.c_float)]
+
+
+# DPRT_DENOISE_DEFAULT_*: what a NULL dprt_denoise_params selects
+DENOISE_DEFAULTS = {"iterations": 3, "sigma_color": 2.0, "sigma_normal": 1.0, "sigma_albedo": 0.3}
+
+
 MAX_TEXTURES = 64
 MAX_MATERIALS = 256
 

@@ -73,6 +73,10 @@ _PROTOTYPES = {
     "dprt_enable_aov": (C.c_int, [C.c_void_p, C.c_int]),
     "dprt_reduce_aov": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "dprt_reduce_aov_group": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "dprt_denoise": (C.c_int, [C.c_void_p, C.POINTER(D.DenoiseParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dprt_denoise_device": (C.c_int, [C.c_void_p, C.POINTER(D.DenoiseParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p]),
+    "dprt_spec_denoise": (C.c_int, [C.POINTER(D.DenoiseParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dprt_adopt_scene": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dprt_accumulate_from": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dprt_p2p_export": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -202,6 +206,36 @@ def spec_env_lookup(rgba, rotation, dirs):
     rc = load_library().dprt_spec_env_lookup(_ptr(t), t.shape[1], t.shape[0], float(rotation), _ptr(d), d.shape[0], _ptr(out))
     if rc:
         raise DprtError(f"dprt_spec_env_lookup failed ({rc})")
+    return out
+
+
+def denoise_params(iterations=None, sigma_color=None, sigma_normal=None, sigma_albedo=None):
+    """dprt_denoise_params with the DPRT_DENOISE_DEFAULT_* values for the arguments left at None; None when all are."""
+    given = {"iterations": iterations, "sigma_color": sigma_color, "sigma_normal": sigma_normal, "sigma_albedo": sigma_albedo}
+    if all(v is None for v in given.values()):
+        return None
+    return D.DenoiseParams(**{k: D.DENOISE_DEFAULTS[k] if v is None else v for k, v in given.items()})
+
+
+def _denoise_inputs(color, albedo, normal):
+    c = np.ascontiguousarray(color, np.float32)
+    if c.ndim != 3 or c.shape[2] != 3:
+        raise DprtError(f"denoise: colour must be [H, W, 3], got {c.shape}")
+    a, n = np.ascontiguousarray(albedo, np.float32), np.ascontiguousarray(normal, np.float32)
+    if a.shape != c.shape or n.shape != c.shape:
+        raise DprtError(f"denoise: albedo {a.shape} and normal {n.shape} must match the colour {c.shape}")
+    return c, a, n
+
+
+def spec_denoise(color, albedo, normal, iterations=None, sigma_color=None, sigma_normal=None, sigma_albedo=None):
+    """dprt_spec_denoise (host only): the denoiser of dprt_denoise on [H, W, 3] float32 arrays, bit for bit what the GPU
+    computes. Parameters left at None take the DPRT_DENOISE_DEFAULT_* values."""
+    c, a, n = _denoise_inputs(color, albedo, normal)
+    out = np.zeros_like(c)
+    p = denoise_params(iterations, sigma_color, sigma_normal, sigma_albedo)
+    rc = load_library().dprt_spec_denoise(None if p is None else C.byref(p), c.shape[1], c.shape[0], _ptr(c), _ptr(a), _ptr(n), _ptr(out))
+    if rc:
+        raise DprtError(f"dprt_spec_denoise failed ({rc})")
     return out
 
 
@@ -524,6 +558,21 @@ class Renderer:
         a, n = (np.zeros(shape, np.float32), np.zeros(shape, np.float32)) if self.rank == root else (None, None)
         self._ck(self.lib.dprt_reduce_aov(self.h, root, _ptr(a), _ptr(n)), "dprt_reduce_aov")
         return (a, n) if self.rank == root else None
+
+    def denoise(self, color, albedo, normal, iterations=None, sigma_color=None, sigma_normal=None, sigma_albedo=None):
+        """dprt_denoise on this context's GPU: the [H, W, 3] colour filtered with its albedo and normal guides (e.g. reduce_image
+        and reduce_aov of the same frame; any size). Returns [H, W, 3] float32. Parameters left at None take the defaults."""
+        c, a, n = _denoise_inputs(color, albedo, normal)
+        out = np.zeros_like(c)
+        p = denoise_params(iterations, sigma_color, sigma_normal, sigma_albedo)
+        self._ck(self.lib.dprt_denoise(self.h, None if p is None else C.byref(p), c.shape[1], c.shape[0], _ptr(c), _ptr(a), _ptr(n),
+                                       _ptr(out)), "dprt_denoise")
+        return out
+
+    def denoise_device(self, width, height, color_dev, albedo_dev, normal_dev, out_dev, params=None):
+        """dprt_denoise_device on device buffers of 3 * width * height floats (params: D.DenoiseParams or None)."""
+        self._ck(self.lib.dprt_denoise_device(self.h, None if params is None else C.byref(params), width, height, color_dev, albedo_dev,
+                                              normal_dev, out_dev), "dprt_denoise_device")
 
     def launch(self):
         """Renderer::launch (renderer.cpp:1576): reset, spp x runSample, average + reduce to rank 0."""
