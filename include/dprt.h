@@ -50,6 +50,29 @@ void dprt_bvh8_free(dprt_bvh8* b);
  * mat_ids = ntris ints into the material table. */
 int  dprt_upload_chunk(dprt_ctx* ctx, int scene_index, const dprt_object_desc* desc, const float* verts9,
                        const float* normals9, const int32_t* mat_ids, int64_t ntris);
+/* ---- BVH8 refit: moved vertices, same triangles (the counterpart of an OptiX acceleration-structure update) ------------
+ * dprt_refit_chunk rewrites the device geometry of local chunk `scene_index` in place for new corner positions verts9
+ * (ntris*9 floats, indexed by the original triangle index = primID, like the upload's) and, when the chunk was uploaded with
+ * them, new normals9: the BVH8 keeps its topology and every node box is recomputed by the builder's own rule (DESIGN.md 3.9),
+ * so the structure stays exact and conservative and hits are the ones of a fresh upload of the new vertices. Materials and
+ * texture coordinates stay as uploaded. Returns after the context's stream is synchronised.
+ * DPRT_ERR_INVALID with a message, and nothing on the device changed: a null array or context, an index that holds no local
+ * chunk, ntris different from the upload's, a non-finite coordinate, a vertex outside the object's aabbMin / aabbMax (the box
+ * other ranks route by and hold proxies of), normals9 given for a chunk uploaded without normals or missing for one with them.
+ * The device memory is shared with every context that adopted the scene (dprt_adopt_scene): they all see the new geometry,
+ * and none of them may have work in flight (the precondition of a re-upload). Proxies of this chunk trained on other ranks
+ * are NOT retrained: they keep answering for the old geometry. A different triangle count needs dprt_upload_chunk, and so does
+ * a deformation that scatters neighbouring triangles: the old grouping then makes every ray visit far more nodes (DESIGN.md 3.9).
+ * dprt_refit_chunk_device: the same on device arrays; the checks run on the device (one reduction, one read-back).
+ * dprt_spec_bvh8_refit: the refit on caller-owned host arrays (a dprt_bvh8_copy or dprt_chunk_bvh8_copy blob), in place, no
+ * device; rejects, leaving the arrays unchanged, a blob whose childBase / triBase / primID point outside the arrays or whose
+ * children do not follow their parent, and non-finite vertices. dprt_chunk_bvh8_copy reads back a chunk's device blob
+ * (triangle records without the texture-coordinate tail); NULL outputs only query the sizes. */
+int  dprt_refit_chunk(dprt_ctx* ctx, int scene_index, const float* verts9, const float* normals9, int64_t ntris);
+int  dprt_refit_chunk_device(dprt_ctx* ctx, int scene_index, const void* verts9_dev, const void* normals9_dev, int64_t ntris);
+int  dprt_spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9);
+int  dprt_chunk_bvh8_copy(dprt_ctx* ctx, int scene_index, int64_t* nnodes, int64_t* ntris, dprt_bvh8_node* nodes_out,
+                          dprt_bvh8_tri* tris_out);
 /* Scene object `scene_index` is a proxy on this rank: AABB + world->object transform + the two proxy MLPs
  * (torch::jit::load of vis/depth modules, renderer.cpp:1884-1905). Weight blobs use the packed fp32 layout
  * documented in DESIGN.md ("proxy weight blob"); either may be NULL ("padding" entries of the reference). */

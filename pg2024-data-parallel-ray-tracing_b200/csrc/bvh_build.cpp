@@ -7,6 +7,7 @@
 // (Ylitie, Karras, Laine 2017). The result of a closest-hit query does not depend on this structure
 // (tie-break on primitive id, see DESIGN.md), so the oracle is free to use its own.
 #include "bvh_build.h"
+#include "bvh_node.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -124,15 +125,6 @@ struct Builder2 {
     }
 };
 
-inline uint8_t exponent_for(float extent) {
-    // smallest e with 2^e * 255 >= extent; stored biased like an IEEE exponent (e + 127)
-    if (!(extent > 0.f)) return 1;  // 2^-126: degenerate axis
-    int e = (int)std::ceil(std::log2((double)extent / 255.0));
-    while (std::ldexp(255.0, e) < (double)extent) e++;
-    e = std::max(-126, std::min(127, e));
-    return (uint8_t)(e + 127);
-}
-
 }  // namespace
 
 int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, float pad, Bvh8& out) {
@@ -155,7 +147,7 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
     if (pad < 0.f) {
         float m = 0.f;
         for (int a = 0; a < 3; a++) m = std::max(m, std::max(std::fabs(scene.lo[a]), std::fabs(scene.hi[a])));
-        pad = std::ldexp(std::max(m, 1.0f), -16);
+        pad = bvh8_chunk_pad(m);
     }
     for (int a = 0; a < 3; a++) { out.bounds[a] = scene.lo[a]; out.bounds[3 + a] = scene.hi[a]; }
 
@@ -234,16 +226,9 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         Child ch[8]; int nch = 0;
         if (nd.count > 0 || (it.n2 == root && K[(size_t)root * 8] == 1)) ch[nch++] = Child{it.n2, true};     // a root that is itself a leaf
         else { collector.run(nd.left, K8[it.n2], ch, nch); collector.run(nd.right, 8 - K8[it.n2], ch, nch); }
-        // node frame
+        // node frame (the slot assignment below measures the children from its centre)
         Box nb; nb.reset();
         for (int i = 0; i < nch; i++) nb.grow(n2[ch[i].n].box);
-        // The frame is padded by a little more than any child will be (children get pad + 2^-7 of a quantisation step,
-        // the slack the traversal kernel's folded dequantisation needs, bvh_traverse.cuh), so no child bound clamps.
-        Box padded = nb;
-        for (int a = 0; a < 3; a++) {
-            const float fp = pad * 1.01f + (nb.hi[a] - nb.lo[a]) * (1.0f / 8192.0f);
-            padded.lo[a] -= fp; padded.hi[a] += fp;
-        }
 
         // slot assignment (greedy on the octant cost table)
         float cost[8][8]; int slot_of[8]; bool slot_used[8] = {false}; bool child_done[8] = {false};
@@ -275,10 +260,8 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
 
         dprt_bvh8_node node;
         std::memset(&node, 0, sizeof(node));
-        for (int a = 0; a < 3; a++) {
-            node.p[a] = padded.lo[a];
-            node.e[a] = exponent_for(padded.hi[a] - padded.lo[a]);
-        }
+        float slo[8][3], shi[8][3];
+        uint32_t used = 0;
         node.triBase = (uint32_t)out.tris.size();
         int ninternal = 0;
         for (int s = 0; s < 8; s++)
@@ -288,11 +271,7 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         int irank = 0, toff = 0;
         for (int s = 0; s < 8; s++) {
             int c = child_in_slot[s];
-            if (c < 0) {
-                node.qlox[s] = node.qloy[s] = node.qloz[s] = 255;
-                node.qhix[s] = node.qhiy[s] = node.qhiz[s] = 0;
-                continue;
-            }
+            if (c < 0) continue;
             const Node2& cn = n2[c];
             if (!leaf_in_slot[s]) {
                 node.imask |= (uint8_t)(1u << s);
@@ -312,23 +291,11 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
                 }
                 toff += lcount;
             }
-            // conservative quantisation of the padded child box, verified in double
-            uint8_t* qlo[3] = {&node.qlox[s], &node.qloy[s], &node.qloz[s]};
-            uint8_t* qhi[3] = {&node.qhix[s], &node.qhiy[s], &node.qhiz[s]};
-            for (int a = 0; a < 3; a++) {
-                double sc = std::ldexp(1.0, (int)node.e[a] - 127);
-                const double cpad = (double)pad + sc * (1.0 / 128.0);
-                double lo = (double)cn.box.lo[a] - cpad, hi = (double)cn.box.hi[a] + cpad;
-                double p0 = (double)node.p[a];
-                int ql = (int)std::floor((lo - p0) / sc);
-                int qh2 = (int)std::ceil((hi - p0) / sc);
-                ql = std::max(0, std::min(255, ql));
-                qh2 = std::max(0, std::min(255, qh2));
-                while (ql > 0 && p0 + ql * sc > lo) ql--;
-                while (qh2 < 255 && p0 + qh2 * sc < hi) qh2++;
-                *qlo[a] = (uint8_t)ql; *qhi[a] = (uint8_t)qh2;
-            }
+            used |= 1u << s;
+            for (int a = 0; a < 3; a++) { slo[s][a] = cn.box.lo[a]; shi[s][a] = cn.box.hi[a]; }
         }
+        float nlo[3], nhi[3];
+        bvh8_encode_node(node, slo, shi, used, pad, nlo, nhi);
         out.nodes[it.out] = node;
     }
     return 0;

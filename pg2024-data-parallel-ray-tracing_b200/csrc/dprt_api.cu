@@ -23,6 +23,7 @@
 #include "dprt.h"
 #include "dprt_internal.cuh"
 #include "bvh_build.h"
+#include "bvh_node.cuh"
 #include "scene_flatten.h"
 #include "mlp.cuh"
 #include "p2p_exchange.cuh"
@@ -92,6 +93,7 @@ struct ObjMem {
     int device = 0;
     void* d_nodes = nullptr; void* d_tris = nullptr; void* d_normals = nullptr;
     MlpModel* vis = nullptr; MlpModel* depth = nullptr;
+    std::vector<int64_t> levels;     // chunk BVH8: node-index boundaries of the depth levels (dprt_refit_chunk), levels.size() - 1 levels
     ~ObjMem() {
         cudaSetDevice(device);
         if (d_nodes) cudaFree(d_nodes);
@@ -196,6 +198,7 @@ struct dprt_ctx {
     void* d_flush = nullptr; size_t flush_bytes = 0;
     void* d_io = nullptr; size_t io_bytes = 0;   // staging for the standalone host-buffer operators
     void* d_denoise = nullptr; size_t denoise_bytes = 0;   // denoiser scratch (dprt_denoise_device): grown to the largest frame
+    void* d_refit = nullptr; size_t refit_bytes = 0;       // refit scratch (dprt_refit_chunk_device): grown to the largest chunk
     int pathSize = 0, shadowPathSize = 0;
     int sample = 0;
     int queryTotal = 0;                 // rows of the last bucketing
@@ -551,6 +554,7 @@ void dprt_destroy(dprt_ctx* ctx) {
     if (ctx->d_flush) cudaFree(ctx->d_flush);
     if (ctx->d_io) cudaFree(ctx->d_io);
     if (ctx->d_denoise) cudaFree(ctx->d_denoise);
+    if (ctx->d_refit) cudaFree(ctx->d_refit);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -684,6 +688,15 @@ int dprt_upload_chunk_uv(dprt_ctx* ctx, int si, const dprt_object_desc* desc, co
     if (normals9) {
         CK(cudaMalloc(&mem->d_normals, (size_t)ntris * 9 * sizeof(float)));
         CK(cudaMemcpy(mem->d_normals, normals9, (size_t)ntris * 9 * sizeof(float), cudaMemcpyHostToDevice));
+    }
+    // BFS order: level 0 is the root, and the internal children of level d are exactly level d + 1
+    mem->levels.assign(1, 0);
+    for (int64_t first = 0, last = 1; first < last;) {
+        mem->levels.push_back(last);
+        int64_t next = last;
+        for (int64_t i = first; i < last; i++)
+            if (b.nodes[i].imask) next = std::max<int64_t>(next, (int64_t)b.nodes[i].childBase + __builtin_popcount(b.nodes[i].imask));
+        first = last; last = next;
     }
     o.mem = mem; o.d_nodes = mem->d_nodes; o.d_tris = mem->d_tris; o.d_normals = mem->d_normals;
     o.nnodes = (int64_t)b.nodes.size(); o.ntris = (int64_t)nt;
@@ -2117,6 +2130,99 @@ int dprt_spec_denoise(const dprt_denoise_params* p, int width, int height, const
     const char* why = nullptr;
     if (denoise_check(p, width, height, &q, &why)) return DPRT_ERR_INVALID;
     return spec_denoise(q, width, height, color, albedo, normal, out);
+}
+
+// ---- BVH8 refit (refit.cu, DESIGN.md 3.9) -------------------------------------------------------------------------------
+namespace {
+// the checks that need no look at the vertices; *out = the chunk
+int refit_target(dprt_ctx* ctx, int si, bool has_normals, int64_t ntris, const char* fn, ObjectHost** out) {
+    if (si < 0 || si >= ctx->cfg.sceneSize || !ctx->objects[si].present)
+        return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": no scene object uploaded at this index");
+    ObjectHost& o = ctx->objects[si];
+    if (o.desc.isProxy || !o.d_nodes) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": the object is not a local chunk");
+    if (ntris != o.ntris) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": triangle count differs from the upload's");
+    if (has_normals != (o.d_normals != nullptr))
+        return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + (has_normals ? ": normals given for a chunk uploaded without them"
+                                                                          : ": the chunk was uploaded with normals and none are given"));
+    *out = &o;
+    return 0;
+}
+}  // namespace
+
+int dprt_refit_chunk_device(dprt_ctx* ctx, int si, const void* verts9_dev, const void* normals9_dev, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!verts9_dev) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: null vertex array");
+    ObjectHost* o = nullptr;
+    int r = refit_target(ctx, si, normals9_dev != nullptr, ntris, "dprt_refit_chunk_device", &o);
+    if (r) return r;
+    CK(cudaSetDevice(ctx->device));
+    const size_t bytes = refit_scratch_bytes(o->nnodes);
+    if (ctx->refit_bytes < bytes) {
+        void* old = ctx->d_refit;
+        ctx->d_refit = nullptr; ctx->refit_bytes = 0;
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (old) CK(cudaFree(old));
+        CK(cudaMalloc(&ctx->d_refit, bytes));
+        ctx->refit_bytes = bytes;
+    }
+    // validate on the device: one reduction, one read-back; nothing is written before it has passed
+    const float* v = (const float*)verts9_dev;
+    launch_refit_stats(v, ntris, ctx->d_refit, ctx->stream);
+    CK(cudaGetLastError());
+    RefitStats st;
+    CK(cudaMemcpyAsync(&st, ctx->d_refit, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: " + std::to_string(st.nonfinite) + " non-finite coordinates");
+    float m = 0.f;
+    for (int a = 0; a < 3; a++) {
+        if (st.lo[a] < o->desc.aabbMin[a] || st.hi[a] > o->desc.aabbMax[a])
+            return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: a vertex lies outside the object's aabbMin / aabbMax");
+        m = std::max(m, std::max(std::fabs(st.lo[a]), std::fabs(st.hi[a])));
+    }
+    if (ctx->aux) CK(cudaStreamSynchronize(ctx->aux));     // the ShadowRay module dprt_render_sample may have left running
+    const std::vector<int64_t>& lv = o->mem->levels;
+    launch_refit((dprt_bvh8_node*)o->d_nodes, (dprt_bvh8_tri*)o->d_tris, ntris, v, lv.data(), (int)lv.size() - 1, bvh8_chunk_pad(m),
+                 ctx->d_refit, ctx->stream);
+    CK(cudaGetLastError());
+    if (normals9_dev)
+        CK(cudaMemcpyAsync(o->d_normals, normals9_dev, (size_t)ntris * 9 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int dprt_refit_chunk(dprt_ctx* ctx, int si, const float* verts9, const float* normals9, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!verts9) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk: null vertex array");
+    ObjectHost* o = nullptr;
+    int r = refit_target(ctx, si, normals9 != nullptr, ntris, "dprt_refit_chunk", &o);
+    if (r) return r;
+    CK(cudaSetDevice(ctx->device));
+    const size_t b = (size_t)ntris * 9 * sizeof(float);
+    if ((r = ensure_io(ctx, normals9 ? 2 * b : b))) return r;
+    char* d = (char*)ctx->d_io;
+    CK(cudaMemcpyAsync(d, verts9, b, cudaMemcpyHostToDevice, ctx->stream));
+    if (normals9) CK(cudaMemcpyAsync(d + b, normals9, b, cudaMemcpyHostToDevice, ctx->stream));
+    return dprt_refit_chunk_device(ctx, si, d, normals9 ? d + b : nullptr, ntris);
+}
+
+int dprt_spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9) {
+    const char* why = nullptr;
+    return spec_bvh8_refit(nodes, nnodes, tris, ntris, verts9, &why);
+}
+
+int dprt_chunk_bvh8_copy(dprt_ctx* ctx, int si, int64_t* nnodes, int64_t* ntris, dprt_bvh8_node* nodes_out, dprt_bvh8_tri* tris_out) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (si < 0 || si >= ctx->cfg.sceneSize || !ctx->objects[si].present || ctx->objects[si].desc.isProxy || !ctx->objects[si].d_nodes)
+        return fail(ctx, DPRT_ERR_INVALID, "dprt_chunk_bvh8_copy: no local chunk at this index");
+    const ObjectHost& o = ctx->objects[si];
+    if (nnodes) *nnodes = o.nnodes;
+    if (ntris) *ntris = o.ntris;
+    if (!nodes_out && !tris_out) return 0;
+    CK(cudaSetDevice(ctx->device));
+    if (nodes_out) CK(cudaMemcpyAsync(nodes_out, o.d_nodes, (size_t)o.nnodes * sizeof(dprt_bvh8_node), cudaMemcpyDeviceToHost, ctx->stream));
+    if (tris_out) CK(cudaMemcpyAsync(tris_out, o.d_tris, (size_t)o.ntris * sizeof(dprt_bvh8_tri), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
 }
 
 int dprt_device_alloc(dprt_ctx* ctx, size_t bytes, void** dev_ptr) {

@@ -122,6 +122,17 @@ void launch_denoise(const dprt_denoise_params& p, int width, int height, const f
                     float* out, void* scratch, cudaStream_t stream);
 int spec_denoise(const dprt_denoise_params& p, int width, int height, const float* color, const float* albedo, const float* normal, float* out);
 
+// BVH8 refit (refit.cu, DESIGN.md 3.9). launch_refit_stats reduces ntris * 9 coordinates into the RefitStats at the start of
+// the scratch (refit_scratch_bytes(nnodes)). launch_refit rewrites the triangle records from verts9 (by primID) and then the
+// nodes, one launch per depth level: levels holds nlevels + 1 node-index boundaries, level d = [levels[d], levels[d + 1]).
+// spec_bvh8_refit: the same on host arrays, after checking every index of the blob (DPRT_ERR_INVALID with the reason in *why).
+struct RefitStats { float lo[3], hi[3]; uint32_t nonfinite, pad_; };   // over the finite coordinates; count of the others
+size_t refit_scratch_bytes(int64_t nnodes);
+void launch_refit_stats(const float* verts9, int64_t ntris, void* scratch, cudaStream_t stream);
+void launch_refit(dprt_bvh8_node* nodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9, const int64_t* levels, int nlevels,
+                  float pad, void* scratch, cudaStream_t stream);
+int spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9, const char** why);
+
 // partition / bucketing (partition.cu)
 struct PartitionScratch {
     unsigned long long* tileState; // tiles * 32 words {generation, status | value}; zeroed once at allocation, never cleared

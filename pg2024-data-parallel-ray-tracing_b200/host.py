@@ -32,6 +32,10 @@ _PROTOTYPES = {
     "dprt_bvh8_copy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "dprt_bvh8_free": (None, [C.c_void_p]),
     "dprt_upload_chunk": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
+    "dprt_refit_chunk": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64]),
+    "dprt_refit_chunk_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64]),
+    "dprt_spec_bvh8_refit": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    "dprt_chunk_bvh8_copy": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
     "dprt_upload_proxy": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t]),
     "dprt_flatten_count": (C.c_int64, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
     "dprt_flatten_instances": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -168,6 +172,21 @@ def build_bvh8(verts9, mat_ids=None, pad=-1.0):
     finally:
         lib.dprt_bvh8_free(h)
     return nodes, tris, int(md.value)
+
+
+def spec_bvh8_refit(nodes, tris, verts9):
+    """dprt_spec_bvh8_refit (host only, no GPU): the BVH8 (nodes[NODE_DTYPE], tris[TRI_DTYPE], e.g. from build_bvh8) refitted to
+    new corners verts9 [ntris, 9] indexed by primID, exactly as dprt_refit_chunk does it on the device. Returns refitted
+    copies; the inputs are left alone. Raises on a malformed blob, a size mismatch or a non-finite vertex."""
+    n = np.array(nodes, D.NODE_DTYPE, copy=True)
+    t = np.array(tris, D.TRI_DTYPE, copy=True)
+    v = np.ascontiguousarray(verts9, np.float32).reshape(-1, 9)
+    if v.shape[0] != t.shape[0]:
+        raise DprtError(f"spec_bvh8_refit: {v.shape[0]} vertex triples for {t.shape[0]} triangle records")
+    rc = load_library().dprt_spec_bvh8_refit(_ptr(n), n.shape[0], _ptr(t), t.shape[0], _ptr(v))
+    if rc:
+        raise DprtError(f"dprt_spec_bvh8_refit failed ({rc})")
+    return n, t
 
 
 def flatten_instances(meshes, instances):
@@ -433,6 +452,25 @@ class Renderer:
         m = None if mat_ids is None else np.ascontiguousarray(mat_ids, np.int32)
         self._ck(self.lib.dprt_upload_chunk_uv(self.h, scene_index, C.byref(desc), _ptr(v), _ptr(n), _ptr(u), _ptr(m), v.shape[0]),
                  "dprt_upload_chunk_uv")
+
+    def refit_chunk(self, scene_index, verts9, normals9=None):
+        """dprt_refit_chunk: moved corners (and normals, when the chunk has them) of local chunk scene_index, same triangles.
+        Instanced objects: flatten_instances with the moved instances, then this."""
+        v = np.ascontiguousarray(verts9, np.float32).reshape(-1, 9)
+        n = None if normals9 is None else np.ascontiguousarray(normals9, np.float32).reshape(-1, 9)
+        self._ck(self.lib.dprt_refit_chunk(self.h, scene_index, _ptr(v), _ptr(n), v.shape[0]), "dprt_refit_chunk")
+
+    def refit_chunk_device(self, scene_index, verts9_dev, normals9_dev, ntris):
+        """dprt_refit_chunk_device on device buffers of ntris * 9 floats (normals9_dev may be None)."""
+        self._ck(self.lib.dprt_refit_chunk_device(self.h, scene_index, verts9_dev, normals9_dev, ntris), "dprt_refit_chunk_device")
+
+    def chunk_bvh8(self, scene_index):
+        """dprt_chunk_bvh8_copy: the device BVH8 of local chunk scene_index -> (nodes[NODE_DTYPE], tris[TRI_DTYPE])."""
+        nn, nt = C.c_int64(), C.c_int64()
+        self._ck(self.lib.dprt_chunk_bvh8_copy(self.h, scene_index, C.byref(nn), C.byref(nt), None, None), "dprt_chunk_bvh8_copy")
+        nodes, tris = np.zeros(nn.value, D.NODE_DTYPE), np.zeros(nt.value, D.TRI_DTYPE)
+        self._ck(self.lib.dprt_chunk_bvh8_copy(self.h, scene_index, None, None, _ptr(nodes), _ptr(tris)), "dprt_chunk_bvh8_copy")
+        return nodes, tris
 
     def upload_instanced_chunk(self, scene_index, desc, meshes, instances):
         """dprt_upload_instanced_chunk: indexed meshes (ctypes_defs.pack_meshes dicts) placed by (mesh, 3x4 matrix) instances."""
