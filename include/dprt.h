@@ -212,7 +212,10 @@ int  dprt_spec_denoise(const dprt_denoise_params* p, int width, int height, cons
  * one's uploaded scene (chunk geometry, proxies and their networks: shared device memory, freed with the last context that
  * uses it; materials, lights, camera: copied) -- a later re-upload on either side no longer reaches the other. dprt_accumulate_from adds another context's directLighting (plane 0) and
  * envLighting sums into this one's, after which dprt_reduce_image averages and reduces the whole frame. Each sample's
- * arithmetic is unchanged; only the order of the per-pixel sum over samples differs (image within 1e-6 relative). */
+ * arithmetic is unchanged; only the order of the per-pixel sum over samples differs. The image is exact against the
+ * per-context composition: each context's sums are those of its own samples in order (bit for bit the one-context result
+ * of the same sample list), added into the first context in the order of the dprt_accumulate_from calls, then averaged
+ * (tests/test_gpu_inflight.py). */
 int  dprt_adopt_scene(dprt_ctx* ctx, dprt_ctx* from);
 int  dprt_accumulate_from(dprt_ctx* ctx, dprt_ctx* other);
 

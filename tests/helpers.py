@@ -8,8 +8,9 @@ D = dprt.ctypes_defs
 
 
 def build_pair(O, W, tris_per_chunk, width, height, *, spp=1, bounces=2, proxy_mode=0, path_gen_mode=0, water_frac=0.0,
-               group=True, models=None, mlp_dtype=1, device=0, main_ray_retrace=0, serial_stages=0, reference_migrate=0):
-    """Returns (renderers[list of W Renderer], oracle World, chunks). models: {scene_index: (vis_blob, depth_blob)}."""
+               group=True, models=None, mlp_dtype=1, device=0, main_ray_retrace=0, serial_stages=0, reference_migrate=0, gpu=True):
+    """Returns (renderers[list of W Renderer], oracle World, chunks). models: {scene_index: (vis_blob, depth_blob)}.
+    gpu=False builds the oracle world only (no renderers)."""
     chunks, mats, lights = dprt.scene.make_scene(W, tris_per_chunk, water_frac=water_frac)
     cfg = dprt.make_config(width, height, spp=spp, bounces=bounces, scene_size=W, proxy_mode=proxy_mode,
                            path_gen_mode=path_gen_mode, mlp_dtype=mlp_dtype, main_ray_retrace=main_ray_retrace,
@@ -28,7 +29,7 @@ def build_pair(O, W, tris_per_chunk, width, height, *, spp=1, bounces=2, proxy_m
     world.set_lights(lights)
     world.set_camera(cam)
     rs = []
-    for r in range(W):
+    for r in range(W if gpu else 0):
         R = dprt.Renderer(cfg, rank=r, world=W, device=device)
         for c in chunks:
             if c.node_id == r:
