@@ -73,6 +73,27 @@ int  dprt_refit_chunk_device(dprt_ctx* ctx, int scene_index, const void* verts9_
 int  dprt_spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9);
 int  dprt_chunk_bvh8_copy(dprt_ctx* ctx, int scene_index, int64_t* nnodes, int64_t* ntris, dprt_bvh8_node* nodes_out,
                           dprt_bvh8_tri* tris_out);
+/* ---- BVH8 build on the GPU: new triangles (the counterpart of an OptiX acceleration-structure build) ----------------------
+ * dprt_build_chunk makes local chunk `scene_index` out of verts9 (ntris*9 floats), normals9 (ntris*9 floats or NULL), uv6
+ * (ntris*6 floats or NULL) and mat_ids (ntris ints or NULL), like dprt_upload_chunk_uv, but builds the BVH8 on the device
+ * (Morton order, PLOC, the host builder's SAH-optimal collapse; DESIGN.md 3.10). The host arrays are staged through the
+ * context's I/O buffer. The tree differs from the host builder's, the hits do not: a built chunk renders bit for bit like an
+ * uploaded one. Everything after the build is dprt_upload_chunk_uv's: normals, the texture-coordinate tail, the depth levels
+ * a later dprt_refit_chunk walks; the old geometry at the index is released once the context's streams are idle.
+ * Returns after the context's stream is synchronised. DPRT_ERR_INVALID with a message, and the object at the index unchanged:
+ * a null context, description or vertex array, an index out of range, ntris <= 0, a nodeID outside the world, a material id
+ * outside [0, DPRT_MAX_MATERIALS), a non-finite coordinate. DPRT_ERR_CAPACITY: ntris >= 2^27 (checked before any array is
+ * read) or a BVH8 deeper than 36 levels.
+ * dprt_build_chunk_device: the same on device arrays; no triangle data goes through the host (the checks run on the device:
+ * one reduction, one read-back; the build reads back one count per clustering iteration and per tree level).
+ * dprt_spec_bvh8_build_gpu: the host twin of the device build (no device): the blob dprt_build_chunk_device makes, bit for
+ * bit, as a handle for dprt_bvh8_info / dprt_bvh8_copy / dprt_bvh8_free (triangle records without texture coordinates).
+ * DPRT_ERR_INVALID: null vertices or handle, ntris <= 0 or >= 2^27, a non-finite coordinate. */
+int  dprt_build_chunk(dprt_ctx* ctx, int scene_index, const dprt_object_desc* desc, const float* verts9, const float* normals9,
+                      const float* uv6, const int32_t* mat_ids, int64_t ntris);
+int  dprt_build_chunk_device(dprt_ctx* ctx, int scene_index, const dprt_object_desc* desc, const void* verts9_dev,
+                             const void* normals9_dev, const void* uv6_dev, const void* mat_ids_dev, int64_t ntris);
+int  dprt_spec_bvh8_build_gpu(const float* verts9, const int32_t* mat_ids, int64_t ntris, dprt_bvh8** out);
 /* Scene object `scene_index` is a proxy on this rank: AABB + world->object transform + the two proxy MLPs
  * (torch::jit::load of vis/depth modules, renderer.cpp:1884-1905). Weight blobs use the packed fp32 layout
  * documented in DESIGN.md ("proxy weight blob"); either may be NULL ("padding" entries of the reference). */

@@ -30,11 +30,7 @@ struct Box {
     void grow(const float* p) {
         for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], p[a]); hi[a] = std::max(hi[a], p[a]); }
     }
-    float half_area() const {
-        float dx = hi[0] - lo[0], dy = hi[1] - lo[1], dz = hi[2] - lo[2];
-        if (dx < 0 || dy < 0 || dz < 0) return 0.f;
-        return dx * dy + dy * dz + dz * dx;
-    }
+    float half_area() const { return bvh8_half_area(lo, hi); }
 };
 
 struct Node2 {
@@ -162,20 +158,8 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         b2.build(root, 0, ntris, 0);
     }
 
-    // ---- collapse to 8-wide: the SAH-optimal choice by dynamic programming (Ylitie, Karras, Laine 2017, section 3.1) ----
-    // C(n, i) = least SAH cost of representing the subtree of binary node n by at most i wide-BVH roots, a root being a wide
-    // internal node (cost cNode x area, its <= 8 children are roots of n's two subtrees) or a leaf slot with <= 3 triangles
-    // (cost cPrim x triangles x area):
-    //   C(n, 1) = min(leaf(n), cNode A_n + min_k C(left, k) + C(right, 8 - k))
-    //   C(n, i) = min(C(n, i - 1), min_k C(left, k) + C(right, i - k))
-    // Why the optimum: a wide node costs a ray a full node step however few of its eight slots it uses, and a collapse decided
-    // one node at a time leaves many nodes with two or three leaf children at the bottom of the tree. Minimising the cost over
-    // the whole subtree avoids them.
-    // cNode : cPrim = 4 : 1 is the trace kernel's issue-slot ratio of a node step to a triangle test (profiles/bvh_quality.py).
+    // ---- collapse to 8-wide: the SAH-optimal choice by dynamic programming (bvh_node.cuh) ----
     const int nn = b2.nnodes.load();
-    const float cNode = 4.0f;
-    const float cPrim = 1.0f;
-    const float INF = std::numeric_limits<float>::max();
     std::vector<float> C((size_t)nn * 8);          // C[n * 8 + i - 1]
     std::vector<uint8_t> K((size_t)nn * 8);        // i = 1: 1 = leaf, 2 = wide node; i >= 2: roots given to the left child, 0 = as for i - 1
     std::vector<uint8_t> K8((size_t)nn);           // wide node rooted at n: roots given to its left child
@@ -183,34 +167,16 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         const Node2& nd = n2[n];
         const float A = nd.box.half_area();
         float* c = &C[(size_t)n * 8]; uint8_t* k = &K[(size_t)n * 8];
-        if (nd.count > 0) { for (int i = 0; i < 8; i++) { c[i] = A * (float)nd.count * cPrim; k[i] = 1; } continue; }
-        const float* cl = &C[(size_t)nd.left * 8]; const float* cr = &C[(size_t)nd.right * 8];
-        float dist[9]; uint8_t dk[9];
-        for (int j = 2; j <= 8; j++) {
-            float best = INF; int bk = 1;
-            for (int x = 1; x < j; x++) { const float v = cl[x - 1] + cr[j - x - 1]; if (v < best) { best = v; bk = x; } }
-            dist[j] = best; dk[j] = (uint8_t)bk;
-        }
-        K8[n] = dk[8];
-        const float cLeaf = nd.pcount <= 3 ? A * (float)nd.pcount * cPrim : INF;
-        const float cInt = dist[8] + A * cNode;
-        c[0] = std::min(cLeaf, cInt); k[0] = cLeaf <= cInt ? 1 : 2;
-        for (int i = 2; i <= 8; i++) {
-            if (dist[i] < c[i - 2]) { c[i - 1] = dist[i]; k[i - 1] = dk[i]; } else { c[i - 1] = c[i - 2]; k[i - 1] = 0; }
-        }
+        if (nd.count > 0) { bvh8_dp_leaf(A, nd.count, c, k); continue; }
+        K8[n] = bvh8_dp_node(A, nd.pcount, &C[(size_t)nd.left * 8], &C[(size_t)nd.right * 8], c, k);
     }
-    struct Child { int n; bool leaf; };
-    struct Collector {
+    struct Tree {
         const std::vector<Node2>& n2; const std::vector<uint8_t>& K;
-        void run(int n, int i, Child* out, int& cnt) const {
-            const Node2& nd = n2[n];
-            if (nd.count > 0) { out[cnt++] = Child{n, true}; return; }
-            if (i == 1) { out[cnt++] = Child{n, K[(size_t)n * 8] == 1}; return; }
-            const int k = K[(size_t)n * 8 + i - 1];
-            if (k == 0) { run(n, i - 1, out, cnt); return; }
-            run(nd.left, k, out, cnt); run(nd.right, i - k, out, cnt);
-        }
-    } collector{n2, K};
+        bool is_leaf(int n) const { return n2[n].count > 0; }
+        int left(int n) const { return n2[n].left; }
+        int right(int n) const { return n2[n].right; }
+        const uint8_t* k(int n) const { return &K[(size_t)n * 8]; }
+    } tree{n2, K};
 
     // BFS so that the internal children of a node are contiguous
     struct Item { int n2; int out; int depth; };
@@ -223,37 +189,13 @@ int bvh8_build(const float* verts, const int32_t* mat_ids, int64_t ntris64, floa
         Item it = queue[qh++];
         out.max_depth = std::max(out.max_depth, it.depth);
         const Node2& nd = n2[it.n2];
-        Child ch[8]; int nch = 0;
-        if (nd.count > 0 || (it.n2 == root && K[(size_t)root * 8] == 1)) ch[nch++] = Child{it.n2, true};     // a root that is itself a leaf
-        else { collector.run(nd.left, K8[it.n2], ch, nch); collector.run(nd.right, 8 - K8[it.n2], ch, nch); }
-        // node frame (the slot assignment below measures the children from its centre)
-        Box nb; nb.reset();
-        for (int i = 0; i < nch; i++) nb.grow(n2[ch[i].n].box);
-
-        // slot assignment (greedy on the octant cost table)
-        float cost[8][8]; int slot_of[8]; bool slot_used[8] = {false}; bool child_done[8] = {false};
-        float ncx[3];
-        for (int a = 0; a < 3; a++) ncx[a] = 0.5f * (nb.lo[a] + nb.hi[a]);
-        for (int c = 0; c < nch; c++) {
-            const Box& cb = n2[ch[c].n].box;
-            float d[3];
-            for (int a = 0; a < 3; a++) d[a] = 0.5f * (cb.lo[a] + cb.hi[a]) - ncx[a];
-            for (int s = 0; s < 8; s++) {
-                float sx = (s & 1) ? -1.f : 1.f, sy = (s & 2) ? -1.f : 1.f, sz = (s & 4) ? -1.f : 1.f;
-                cost[c][s] = d[0] * sx + d[1] * sy + d[2] * sz;
-            }
-        }
-        for (int k = 0; k < nch; k++) {
-            int bc = -1, bs = -1; float bv = std::numeric_limits<float>::max();
-            for (int c = 0; c < nch; c++) {
-                if (child_done[c]) continue;
-                for (int s = 0; s < 8; s++) {
-                    if (slot_used[s]) continue;
-                    if (cost[c][s] < bv) { bv = cost[c][s]; bc = c; bs = s; }
-                }
-            }
-            child_done[bc] = true; slot_used[bs] = true; slot_of[bc] = bs;
-        }
+        Bvh8Child ch[8]; int nch = 0;
+        if (nd.count > 0 || (it.n2 == root && K[(size_t)root * 8] == 1)) ch[nch++] = Bvh8Child{it.n2, true};     // a root that is itself a leaf
+        else { bvh8_collect(tree, nd.left, K8[it.n2], ch, nch); bvh8_collect(tree, nd.right, 8 - K8[it.n2], ch, nch); }
+        float clo[8][3], chi[8][3]; int slot_of[8];
+        for (int c = 0; c < nch; c++)
+            for (int a = 0; a < 3; a++) { clo[c][a] = n2[ch[c].n].box.lo[a]; chi[c][a] = n2[ch[c].n].box.hi[a]; }
+        bvh8_assign_slots(clo, chi, nch, slot_of);
         int child_in_slot[8]; bool leaf_in_slot[8];
         for (int s = 0; s < 8; s++) { child_in_slot[s] = -1; leaf_in_slot[s] = false; }
         for (int c = 0; c < nch; c++) { child_in_slot[slot_of[c]] = ch[c].n; leaf_in_slot[slot_of[c]] = ch[c].leaf; }

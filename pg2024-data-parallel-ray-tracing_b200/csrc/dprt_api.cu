@@ -199,6 +199,7 @@ struct dprt_ctx {
     void* d_io = nullptr; size_t io_bytes = 0;   // staging for the standalone host-buffer operators
     void* d_denoise = nullptr; size_t denoise_bytes = 0;   // denoiser scratch (dprt_denoise_device): grown to the largest frame
     void* d_refit = nullptr; size_t refit_bytes = 0;       // refit scratch (dprt_refit_chunk_device): grown to the largest chunk
+    void* d_gbuild = nullptr; size_t gbuild_bytes = 0;     // GPU build scratch (dprt_build_chunk_device): grown to the largest chunk
     int pathSize = 0, shadowPathSize = 0;
     int sample = 0;
     int queryTotal = 0;                 // rows of the last bucketing
@@ -555,6 +556,7 @@ void dprt_destroy(dprt_ctx* ctx) {
     if (ctx->d_io) cudaFree(ctx->d_io);
     if (ctx->d_denoise) cudaFree(ctx->d_denoise);
     if (ctx->d_refit) cudaFree(ctx->d_refit);
+    if (ctx->d_gbuild) cudaFree(ctx->d_gbuild);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -2208,6 +2210,102 @@ int dprt_refit_chunk(dprt_ctx* ctx, int si, const float* verts9, const float* no
 int dprt_spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9) {
     const char* why = nullptr;
     return spec_bvh8_refit(nodes, nnodes, tris, ntris, verts9, &why);
+}
+
+// ---- BVH8 build on the GPU (bvh_gpu_build.cu, DESIGN.md 3.10) ------------------------------------------------------------
+namespace {
+// the checks that read no array: those of dprt_upload_chunk_uv, in its order
+int build_target(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* verts9, int64_t ntris, const char* fn) {
+    if (!desc || !verts9) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": null object description or vertex array");
+    if (si < 0 || si >= ctx->cfg.sceneSize) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": scene index out of range");
+    if (ntris <= 0) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": ntris <= 0");
+    if (desc->nodeID < 0 || desc->nodeID >= ctx->world) return fail(ctx, DPRT_ERR_INVALID, "nodeID out of range");
+    if (ntris >= ((int64_t)1 << 27)) return fail(ctx, DPRT_ERR_CAPACITY, "more than 2^27 triangles in one chunk (bvh_traverse.cuh: DPRT_TRI_BITS)");
+    return 0;
+}
+}  // namespace
+
+int dprt_build_chunk_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* verts9_dev, const void* normals9_dev,
+                            const void* uv6_dev, const void* mat_ids_dev, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    int r = build_target(ctx, si, desc, verts9_dev, ntris, "dprt_build_chunk_device");
+    if (r) return r;
+    CK(cudaSetDevice(ctx->device));
+    const size_t bytes = gpu_build_scratch_bytes(ntris);
+    if (ctx->gbuild_bytes < bytes) {
+        void* old = ctx->d_gbuild;
+        ctx->d_gbuild = nullptr; ctx->gbuild_bytes = 0;
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (old) CK(cudaFree(old));
+        CK(cudaMalloc(&ctx->d_gbuild, bytes));
+        ctx->gbuild_bytes = bytes;
+    }
+    const float* v = (const float*)verts9_dev;
+    const int32_t* mats = (const int32_t*)mat_ids_dev;
+    const float* uv = (const float*)uv6_dev;
+    // validate on the device: one reduction (and the material range), one read-back; nothing is replaced before it has passed
+    RefitStats st; uint32_t badMat = 0;
+    CK(gpu_build_check(v, mats, ntris, ctx->d_gbuild, ctx->stream, &st, &badMat));
+    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, "dprt_build_chunk_device: " + std::to_string(st.nonfinite) + " non-finite coordinates");
+    if (badMat) return fail(ctx, DPRT_ERR_INVALID, "material id out of range");
+    float m = 0.f;
+    for (int a = 0; a < 3; a++) m = std::max(m, std::max(std::fabs(st.lo[a]), std::fabs(st.hi[a])));
+    std::vector<int64_t> levels, triBase;
+    const char* why = nullptr;
+    CK(gpu_build_tree(v, ntris, ctx->d_gbuild, ctx->stream, 36, levels, triBase, &why));
+    if (why) return fail(ctx, DPRT_ERR_STATE, std::string("dprt_build_chunk_device: ") + why);
+    if ((int)levels.size() - 1 > 36) return fail(ctx, DPRT_ERR_CAPACITY, "BVH8 deeper than the traversal stack");
+    auto mem = std::make_shared<ObjMem>();
+    mem->device = ctx->device;
+    const int64_t nnodes = levels.back();
+    // texture coordinates: 32 bytes per triangle in leaf order behind the triangle array (dprt_bvh8_tri.pad_ = triangle count)
+    CK(cudaMalloc(&mem->d_nodes, (size_t)nnodes * sizeof(dprt_bvh8_node)));
+    CK(cudaMalloc(&mem->d_tris, (size_t)ntris * (sizeof(dprt_bvh8_tri) + (uv ? 8 * sizeof(float) : 0))));
+    launch_gpu_build_write(v, mats, uv, ntris, bvh8_chunk_pad(m), ctx->d_gbuild, levels, triBase, (dprt_bvh8_node*)mem->d_nodes,
+                           (dprt_bvh8_tri*)mem->d_tris, ctx->stream);
+    CK(cudaGetLastError());
+    if (normals9_dev) {
+        CK(cudaMalloc(&mem->d_normals, (size_t)ntris * 9 * sizeof(float)));
+        CK(cudaMemcpyAsync(mem->d_normals, normals9_dev, (size_t)ntris * 9 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));             // nothing in flight reads the old geometry
+    if (ctx->aux) CK(cudaStreamSynchronize(ctx->aux));
+    ObjectHost& o = ctx->objects[si];
+    o.release();
+    o.desc = *desc; o.desc.isProxy = 0; o.present = true;
+    mem->levels = levels;
+    o.mem = mem; o.d_nodes = mem->d_nodes; o.d_tris = mem->d_tris; o.d_normals = mem->d_normals;
+    o.nnodes = nnodes; o.ntris = ntris;
+    return upload_objects(ctx);
+}
+
+int dprt_build_chunk(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const float* verts9, const float* normals9, const float* uv6,
+                     const int32_t* mat_ids, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    int r = build_target(ctx, si, desc, verts9, ntris, "dprt_build_chunk");
+    if (r) return r;
+    CK(cudaSetDevice(ctx->device));
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b9 = (size_t)ntris * 9 * sizeof(float), b6 = (size_t)ntris * 6 * sizeof(float), b1 = (size_t)ntris * sizeof(int32_t);
+    const size_t on = up(b9), ou = on + (normals9 ? up(b9) : 0), om = ou + (uv6 ? up(b6) : 0), total = om + (mat_ids ? up(b1) : 0);
+    if ((r = ensure_io(ctx, total))) return r;
+    char* d = (char*)ctx->d_io;
+    CK(cudaMemcpyAsync(d, verts9, b9, cudaMemcpyHostToDevice, ctx->stream));
+    if (normals9) CK(cudaMemcpyAsync(d + on, normals9, b9, cudaMemcpyHostToDevice, ctx->stream));
+    if (uv6) CK(cudaMemcpyAsync(d + ou, uv6, b6, cudaMemcpyHostToDevice, ctx->stream));
+    if (mat_ids) CK(cudaMemcpyAsync(d + om, mat_ids, b1, cudaMemcpyHostToDevice, ctx->stream));
+    return dprt_build_chunk_device(ctx, si, desc, d, normals9 ? d + on : nullptr, uv6 ? d + ou : nullptr, mat_ids ? d + om : nullptr, ntris);
+}
+
+int dprt_spec_bvh8_build_gpu(const float* verts9, const int32_t* mat_ids, int64_t ntris, dprt_bvh8** out) {
+    if (!out) return DPRT_ERR_INVALID;
+    *out = nullptr;
+    dprt_bvh8* b = new dprt_bvh8();
+    const char* why = nullptr;
+    const int r = spec_bvh8_build_gpu(verts9, mat_ids, ntris, b->b, &why);
+    if (r) { delete b; return r; }
+    *out = b;
+    return 0;
 }
 
 int dprt_chunk_bvh8_copy(dprt_ctx* ctx, int si, int64_t* nnodes, int64_t* ntris, dprt_bvh8_node* nodes_out, dprt_bvh8_tri* tris_out) {

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <vector>
 #include "dprt_types.h"
 #include "dprt_math.cuh"
 
@@ -132,6 +133,21 @@ void launch_refit_stats(const float* verts9, int64_t ntris, void* scratch, cudaS
 void launch_refit(dprt_bvh8_node* nodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9, const int64_t* levels, int nlevels,
                   float pad, void* scratch, cudaStream_t stream);
 int spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, int64_t ntris, const float* verts9, const char** why);
+
+// GPU BVH8 build (bvh_gpu_build.cu, DESIGN.md 3.10); scratch: gpu_build_scratch_bytes(ntris), all calls on one stream.
+// gpu_build_check: the vertices' RefitStats and whether a material id lies outside [0, DPRT_MAX_MATERIALS) (mats may be null),
+// read back with one synchronisation. gpu_build_tree: Morton order, PLOC tree and emission pass 1 (one read-back per PLOC
+// iteration and per level); levels gets the node-index boundaries of the BFS levels (depth = levels.size() - 1, which stops at
+// maxDepth + 1) and triBase the first triangle record of each level; *why is set only when the tree could not be built.
+// launch_gpu_build_write: emission pass 2 into nodes[levels.back()] and tris[ntris] (+ the texture-coordinate tail when uv6).
+size_t gpu_build_scratch_bytes(int64_t ntris);
+cudaError_t gpu_build_check(const float* verts9, const int32_t* mats, int64_t ntris, void* scratch, cudaStream_t stream, RefitStats* st,
+                            uint32_t* badMat);
+cudaError_t gpu_build_tree(const float* verts9, int64_t ntris, void* scratch, cudaStream_t stream, int maxDepth, std::vector<int64_t>& levels,
+                           std::vector<int64_t>& triBase, const char** why);
+void launch_gpu_build_write(const float* verts9, const int32_t* mats, const float* uv6, int64_t ntris, float pad, void* scratch,
+                            const std::vector<int64_t>& levels, const std::vector<int64_t>& triBase, dprt_bvh8_node* nodes,
+                            dprt_bvh8_tri* tris, cudaStream_t stream);
 
 // partition / bucketing (partition.cu)
 struct PartitionScratch {

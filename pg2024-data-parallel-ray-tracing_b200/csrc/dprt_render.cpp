@@ -26,6 +26,8 @@
 //               [--aov 1]              also the first-hit guide buffers a denoiser takes beside the colour (dprt_enable_aov on every
 //                                      context, samples in flight included): <name>.albedo.<ext> and <name>.normal.<ext>, e.g.
 //                                      --out img.exr writes img.albedo.exr and img.normal.exr (<f>img.albedo.exr per frame f)
+//               [--gpu-build 1]        build the own chunks' BVH8s on the GPU (dprt_build_chunk) instead of on the host; the
+//                                      image is the same bit for bit
 //               [--denoise 1]          also the frame filtered by dprt_denoise (default parameters) with those guide buffers (turned
 //                                      on for it as --aov 1 does, but written only with --aov 1): <name>.denoised.<ext>
 //   dprt_render --convert in.pfm out.exr     no GPU: re-encode an image (the reference's Image::save writes EXR)
@@ -216,15 +218,18 @@ void move_camera(dprt_camera& c, const float move[3], const float* target) {
     for (int a = 0; a < 3; a++) { c.U[a] = (float)(u[a] * lu); c.V[a] = (float)(v[a] * lv); c.W[a] = (float)w[a]; }
 }
 
-// the AccelerationStructure table of one rank (renderer.cpp:1812-1842): own objects as geometry, the others as proxies
-int upload_scene(dprt_ctx* ctx, const Scene& sc, int rank) {
+// the AccelerationStructure table of one rank (renderer.cpp:1812-1842): own objects as geometry, the others as proxies.
+// gpuBuild: own objects' BVH8s are built on the GPU (dprt_build_chunk) instead of on the host
+int upload_scene(dprt_ctx* ctx, const Scene& sc, int rank, bool gpuBuild) {
     int r;
     for (size_t k = 0; k < sc.objects.size(); k++) {
         const Object& o = sc.objects[k];
         dprt_object_desc d = o.desc;
         if (o.desc.nodeID == rank) {
             d.isProxy = 0;
-            if ((r = dprt_upload_chunk_uv(ctx, (int)k, &d, o.verts.data(), o.normals.data(), o.uvs.empty() ? nullptr : o.uvs.data(), o.mats.data(), o.ntris))) return r;
+            const float* uv = o.uvs.empty() ? nullptr : o.uvs.data();
+            if ((r = gpuBuild ? dprt_build_chunk(ctx, (int)k, &d, o.verts.data(), o.normals.data(), uv, o.mats.data(), o.ntris)
+                              : dprt_upload_chunk_uv(ctx, (int)k, &d, o.verts.data(), o.normals.data(), uv, o.mats.data(), o.ntris))) return r;
         } else {
             d.isProxy = 1;
             if ((r = dprt_upload_proxy(ctx, (int)k, &d, o.vis.empty() ? nullptr : o.vis.data(), o.vis.size(),
@@ -286,7 +291,7 @@ int main(int argc, char** argv) {
     if (scenePath.empty()) {
         fprintf(stderr, "usage: dprt_render --scene S.dprt [--out image.pfm] [--spp n] [--bounces n] [--proxy 0|1] [--path-gen 0|1] "
                         "[--inflight K] [--world W | --nccl-id-file F] [--frames F] [--camera-move x,y,z] [--camera-target x,y,z] "
-                        "[--light-move x,y,z] [--light-start x,y,z] [--aov 0|1] [--denoise 0|1]\n       dprt_render --convert in.pfm out.exr\n");
+                        "[--light-move x,y,z] [--light-start x,y,z] [--aov 0|1] [--denoise 0|1] [--gpu-build 0|1]\n       dprt_render --convert in.pfm out.exr\n");
         return 2;
     }
     Scene sc; std::string err;
@@ -316,6 +321,7 @@ int main(int argc, char** argv) {
     cfg.envColor[0] = 0.6f; cfg.envColor[1] = 0.7f; cfg.envColor[2] = 0.9f;
     const size_t N = (size_t)cfg.width * cfg.height;
     std::vector<float> image(3 * N);
+    const bool gpuBuild = std::atoi(arg(argc, argv, "--gpu-build", "0")) != 0;
     const bool aov = std::atoi(arg(argc, argv, "--aov", "0")) != 0;
     const bool denoise = std::atoi(arg(argc, argv, "--denoise", "0")) != 0;
     const bool guides = aov || denoise;                                 // the denoiser filters with the guide buffers
@@ -405,7 +411,7 @@ int main(int argc, char** argv) {
         dprt_ctx* ctx = nullptr;
         if ((r = dprt_create(&cfg, rank, world, local, id, &ctx))) return die("dprt_create", nullptr, r);
         ctxs.push_back(ctx);
-        if ((r = upload_scene(ctx, sc, rank))) return die("scene upload", ctx, r);
+        if ((r = upload_scene(ctx, sc, rank, gpuBuild))) return die("scene upload", ctx, r);
         if ((r = make_inflight(ctx))) return die("samples in flight", nullptr, r);
         std::vector<dprt_ctx*> all{ctx};
         all.insert(all.end(), extra.begin(), extra.end());
@@ -433,7 +439,7 @@ int main(int argc, char** argv) {
         ctxs.resize(world, nullptr);
         for (int k = 0; k < world; k++) {
             if ((r = dprt_create(&cfg, k, world, k % ndev, nullptr, &ctxs[k]))) return die("dprt_create", nullptr, r);
-            if ((r = upload_scene(ctxs[k], sc, k))) return die("scene upload", ctxs[k], r);
+            if ((r = upload_scene(ctxs[k], sc, k, gpuBuild))) return die("scene upload", ctxs[k], r);
         }
         if (world == 1 && (r = make_inflight(ctxs[0]))) return die("samples in flight", nullptr, r);
         std::vector<dprt_ctx*> all(ctxs);

@@ -36,6 +36,10 @@ _PROTOTYPES = {
     "dprt_refit_chunk_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64]),
     "dprt_spec_bvh8_refit": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     "dprt_chunk_bvh8_copy": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
+    "dprt_build_chunk": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
+    "dprt_build_chunk_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_int64]),
+    "dprt_spec_bvh8_build_gpu": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
     "dprt_upload_proxy": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t]),
     "dprt_flatten_count": (C.c_int64, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
     "dprt_flatten_instances": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -163,6 +167,26 @@ def build_bvh8(verts9, mat_ids=None, pad=-1.0):
     rc = lib.dprt_bvh8_build(_ptr(v), _ptr(m), v.shape[0], float(pad), C.byref(h))
     if rc:
         raise DprtError(f"dprt_bvh8_build failed: {rc}")
+    return _take_bvh8(lib, h)
+
+
+def spec_bvh8_build_gpu(verts9, mat_ids=None):
+    """dprt_spec_bvh8_build_gpu (host only, no GPU): the BVH8 that Renderer.build_chunk_device makes of these triangles, bit for
+    bit -> (nodes[NODE_DTYPE], tris[TRI_DTYPE], max_depth). Raises on ntris <= 0 or a non-finite coordinate."""
+    lib = load_library()
+    v = np.ascontiguousarray(verts9, np.float32).reshape(-1, 9)
+    m = None if mat_ids is None else np.ascontiguousarray(mat_ids, np.int32)
+    if m is not None and m.shape[0] != v.shape[0]:
+        raise DprtError(f"spec_bvh8_build_gpu: {m.shape[0]} material ids for {v.shape[0]} triangles")
+    h = C.c_void_p()
+    rc = lib.dprt_spec_bvh8_build_gpu(_ptr(v), _ptr(m), v.shape[0], C.byref(h))
+    if rc:
+        raise DprtError(f"dprt_spec_bvh8_build_gpu failed ({rc})")
+    return _take_bvh8(lib, h)
+
+
+def _take_bvh8(lib, h):
+    """copies a dprt_bvh8 handle's blob out and frees the handle"""
     try:
         nn, nt, md = C.c_int64(), C.c_int64(), C.c_int32()
         lib.dprt_bvh8_info(h, C.byref(nn), C.byref(nt), C.byref(md))
@@ -463,6 +487,24 @@ class Renderer:
     def refit_chunk_device(self, scene_index, verts9_dev, normals9_dev, ntris):
         """dprt_refit_chunk_device on device buffers of ntris * 9 floats (normals9_dev may be None)."""
         self._ck(self.lib.dprt_refit_chunk_device(self.h, scene_index, verts9_dev, normals9_dev, ntris), "dprt_refit_chunk_device")
+
+    def build_chunk(self, scene_index, desc, verts9, normals9, uv6, mat_ids):
+        """dprt_build_chunk: upload_chunk_uv with the BVH8 built on the GPU (DESIGN.md 3.10), same arguments; normals9, uv6 and
+        mat_ids may be None."""
+        v = np.ascontiguousarray(verts9, np.float32).reshape(-1, 9)
+        n = None if normals9 is None else np.ascontiguousarray(normals9, np.float32).reshape(-1, 9)
+        u = None if uv6 is None else np.ascontiguousarray(uv6, np.float32).reshape(-1, 6)
+        m = None if mat_ids is None else np.ascontiguousarray(mat_ids, np.int32)
+        for name, a in (("normals9", n), ("uv6", u), ("mat_ids", m)):
+            if a is not None and a.shape[0] != v.shape[0]:
+                raise DprtError(f"build_chunk: {a.shape[0]} rows of {name} for {v.shape[0]} triangles")
+        self._ck(self.lib.dprt_build_chunk(self.h, scene_index, C.byref(desc), _ptr(v), _ptr(n), _ptr(u), _ptr(m), v.shape[0]),
+                 "dprt_build_chunk")
+
+    def build_chunk_device(self, scene_index, desc, verts9_dev, normals9_dev, uv6_dev, mat_ids_dev, ntris):
+        """dprt_build_chunk_device on device buffers (ntris * 9 / 9 / 6 floats, ntris ints; all but verts9_dev may be None)."""
+        self._ck(self.lib.dprt_build_chunk_device(self.h, scene_index, C.byref(desc), verts9_dev, normals9_dev, uv6_dev, mat_ids_dev, ntris),
+                 "dprt_build_chunk_device")
 
     def chunk_bvh8(self, scene_index):
         """dprt_chunk_bvh8_copy: the device BVH8 of local chunk scene_index -> (nodes[NODE_DTYPE], tris[TRI_DTYPE])."""
