@@ -117,6 +117,24 @@ int  dprt_upload_chunk_uv(dprt_ctx* ctx, int scene_index, const dprt_object_desc
 /* flatten + dprt_upload_chunk_uv: one scene object from its meshes and instances (GAS build + SBT records of the reference) */
 int  dprt_upload_instanced_chunk(dprt_ctx* ctx, int scene_index, const dprt_object_desc* desc, const dprt_mesh_desc* meshes,
                                  int n_meshes, const dprt_instance_desc* instances, int64_t n_instances);
+/* ---- instanced objects built and moved on the GPU (the counterparts of an OptiX IAS build and IAS update; DESIGN.md 3.11) ----
+ * dprt_build_instanced_chunk: dprt_upload_instanced_chunk's object, made on the device. The indexed arrays and the instance
+ * table (not the flattened triangles) are copied through the context; the device flattens them, bit for bit as
+ * dprt_flatten_instances does, straight into dprt_build_chunk's GPU build. The chunk keeps its own copy of the indexed meshes
+ * (shared with the contexts that adopt the scene, freed with the geometry) for dprt_update_instances. Returns after the
+ * context's stream is synchronised. The checks are dprt_upload_instanced_chunk's (mesh and instance descriptions, the flattened
+ * triangle count against 2^27 before any array is copied: DPRT_ERR_CAPACITY) and dprt_build_chunk's; DPRT_ERR_INVALID, with
+ * the object at the index unchanged, also for a position, normal or texture-coordinate index outside its mesh's array and for a
+ * singular or non-finite instance transform (checked on the device, read back with the other checks).
+ * dprt_update_instances: new transforms for the instance list of the build (same count, same mesh per instance): flattened on
+ * the device and refitted exactly as dprt_refit_chunk does it with the flattened moved instances. DPRT_ERR_INVALID, with
+ * nothing changed: an index that holds no chunk made by dprt_build_instanced_chunk (a proxy, an uploaded chunk), another
+ * instance count, an instance naming another mesh, a singular or non-finite transform, a vertex outside the object's
+ * aabbMin / aabbMax. Preconditions as for dprt_refit_chunk: no context that shares the scene (dprt_adopt_scene) may have work
+ * in flight, and proxies of this chunk on other ranks are not retrained. */
+int  dprt_build_instanced_chunk(dprt_ctx* ctx, int scene_index, const dprt_object_desc* desc, const dprt_mesh_desc* meshes,
+                                int n_meshes, const dprt_instance_desc* instances, int64_t n_instances);
+int  dprt_update_instances(dprt_ctx* ctx, int scene_index, const dprt_instance_desc* instances, int64_t n_instances);
 /* params.albedoTextures[texture_index] (renderer.cpp:1621-1721): width*height RGBA float texels, row 0 first (v = 0), filtered
  * bilinearly with wrap addressing on normalised coordinates like the reference's texture descriptor -- in software, in exact
  * binary32 (DESIGN.md 4), not by the texture unit's 9-bit fixed-point weights. rgba = NULL removes the texture. */

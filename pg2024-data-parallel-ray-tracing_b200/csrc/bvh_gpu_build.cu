@@ -378,7 +378,7 @@ size_t gpu_build_scratch_bytes(int64_t ntris) {
 }
 
 cudaError_t gpu_build_check(const float* verts9, const int32_t* mats, int64_t ntris, void* scratch, cudaStream_t stream, RefitStats* st,
-                            uint32_t* badMat) {
+                            uint32_t* badMat, const uint32_t* flags, uint32_t* flagsOut) {
     GbDevice d = carve(scratch, ntris, 0);
     cudaError_t e;
     if ((e = cudaMemsetAsync(d.badMat, 0, sizeof(uint32_t), stream)) != cudaSuccess) return e;
@@ -387,6 +387,7 @@ cudaError_t gpu_build_check(const float* verts9, const int32_t* mats, int64_t nt
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(st, d.vstats, sizeof(RefitStats), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(badMat, d.badMat, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
+    if (flags && (e = cudaMemcpyAsync(flagsOut, flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
     return cudaStreamSynchronize(stream);
 }
 

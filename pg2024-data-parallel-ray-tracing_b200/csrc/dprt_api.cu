@@ -94,8 +94,13 @@ struct ObjMem {
     void* d_nodes = nullptr; void* d_tris = nullptr; void* d_normals = nullptr;
     MlpModel* vis = nullptr; MlpModel* depth = nullptr;
     std::vector<int64_t> levels;     // chunk BVH8: node-index boundaries of the depth levels (dprt_refit_chunk), levels.size() - 1 levels
+    // instanced chunk (dprt_build_instanced_chunk): d_meshes holds the mesh table, its triangle scan and the indexed arrays;
+    // instMesh is the mesh of every instance, which dprt_update_instances holds the new instance list to
+    void* d_meshes = nullptr; const DevMesh* meshTable = nullptr;
+    std::vector<int32_t> instMesh;
     ~ObjMem() {
         cudaSetDevice(device);
+        if (d_meshes) cudaFree(d_meshes);
         if (d_nodes) cudaFree(d_nodes);
         if (d_tris) cudaFree(d_tris);
         if (d_normals) cudaFree(d_normals);
@@ -2151,12 +2156,17 @@ int refit_target(dprt_ctx* ctx, int si, bool has_normals, int64_t ntris, const c
 }
 }  // namespace
 
-int dprt_refit_chunk_device(dprt_ctx* ctx, int si, const void* verts9_dev, const void* normals9_dev, int64_t ntris) {
-    if (!ctx) return DPRT_ERR_INVALID;
-    if (!verts9_dev) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: null vertex array");
-    ObjectHost* o = nullptr;
-    int r = refit_target(ctx, si, normals9_dev != nullptr, ntris, "dprt_refit_chunk_device", &o);
-    if (r) return r;
+namespace {
+// the reason a nonzero word of the device flatten's kFlatten* bits rejects the call
+std::string flatten_failure(uint32_t flags) {
+    return (flags & kFlattenBadIndex) ? "a position, normal or texture-coordinate index lies outside its mesh's array"
+                                      : "a singular or non-finite instance transform";
+}
+
+// The refit of chunk o to the device arrays verts9 / normals9 (refit_target has passed). d_flags (may be null): a device word
+// that is read back with the vertex statistics and rejects the call when nonzero (the device flatten's kFlatten* bits).
+int refit_chunk_on_device(dprt_ctx* ctx, ObjectHost* o, const float* v, const void* normals9_dev, int64_t ntris, const char* fn,
+                          const uint32_t* d_flags) {
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = refit_scratch_bytes(o->nnodes);
     if (ctx->refit_bytes < bytes) {
@@ -2168,17 +2178,18 @@ int dprt_refit_chunk_device(dprt_ctx* ctx, int si, const void* verts9_dev, const
         ctx->refit_bytes = bytes;
     }
     // validate on the device: one reduction, one read-back; nothing is written before it has passed
-    const float* v = (const float*)verts9_dev;
     launch_refit_stats(v, ntris, ctx->d_refit, ctx->stream);
     CK(cudaGetLastError());
-    RefitStats st;
+    RefitStats st; uint32_t flags = 0;
     CK(cudaMemcpyAsync(&st, ctx->d_refit, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_flags) CK(cudaMemcpyAsync(&flags, d_flags, sizeof(flags), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: " + std::to_string(st.nonfinite) + " non-finite coordinates");
+    if (flags) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": " + flatten_failure(flags));
+    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": " + std::to_string(st.nonfinite) + " non-finite coordinates");
     float m = 0.f;
     for (int a = 0; a < 3; a++) {
         if (st.lo[a] < o->desc.aabbMin[a] || st.hi[a] > o->desc.aabbMax[a])
-            return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: a vertex lies outside the object's aabbMin / aabbMax");
+            return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": a vertex lies outside the object's aabbMin / aabbMax");
         m = std::max(m, std::max(std::fabs(st.lo[a]), std::fabs(st.hi[a])));
     }
     if (ctx->aux) CK(cudaStreamSynchronize(ctx->aux));     // the ShadowRay module dprt_render_sample may have left running
@@ -2190,6 +2201,16 @@ int dprt_refit_chunk_device(dprt_ctx* ctx, int si, const void* verts9_dev, const
         CK(cudaMemcpyAsync(o->d_normals, normals9_dev, (size_t)ntris * 9 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+}  // namespace
+
+int dprt_refit_chunk_device(dprt_ctx* ctx, int si, const void* verts9_dev, const void* normals9_dev, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    if (!verts9_dev) return fail(ctx, DPRT_ERR_INVALID, "dprt_refit_chunk_device: null vertex array");
+    ObjectHost* o = nullptr;
+    int r = refit_target(ctx, si, normals9_dev != nullptr, ntris, "dprt_refit_chunk_device", &o);
+    if (r) return r;
+    return refit_chunk_on_device(ctx, o, (const float*)verts9_dev, normals9_dev, ntris, "dprt_refit_chunk_device", nullptr);
 }
 
 int dprt_refit_chunk(dprt_ctx* ctx, int si, const float* verts9, const float* normals9, int64_t ntris) {
@@ -2225,11 +2246,12 @@ int build_target(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void
 }
 }  // namespace
 
-int dprt_build_chunk_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* verts9_dev, const void* normals9_dev,
-                            const void* uv6_dev, const void* mat_ids_dev, int64_t ntris) {
-    if (!ctx) return DPRT_ERR_INVALID;
-    int r = build_target(ctx, si, desc, verts9_dev, ntris, "dprt_build_chunk_device");
-    if (r) return r;
+namespace {
+// The GPU build of chunk si from the device arrays (build_target has passed) into `mem`, which then becomes the chunk's memory.
+// d_flags (may be null): a device word read back with the vertex statistics that rejects the call when nonzero (the device
+// flatten's kFlatten* bits). A rejected call leaves the object at si as it was.
+int build_chunk_on_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const float* v, const void* normals9_dev, const float* uv,
+                          const int32_t* mats, int64_t ntris, const char* fn, const uint32_t* d_flags, std::shared_ptr<ObjMem> mem) {
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = gpu_build_scratch_bytes(ntris);
     if (ctx->gbuild_bytes < bytes) {
@@ -2240,22 +2262,19 @@ int dprt_build_chunk_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc,
         CK(cudaMalloc(&ctx->d_gbuild, bytes));
         ctx->gbuild_bytes = bytes;
     }
-    const float* v = (const float*)verts9_dev;
-    const int32_t* mats = (const int32_t*)mat_ids_dev;
-    const float* uv = (const float*)uv6_dev;
     // validate on the device: one reduction (and the material range), one read-back; nothing is replaced before it has passed
-    RefitStats st; uint32_t badMat = 0;
-    CK(gpu_build_check(v, mats, ntris, ctx->d_gbuild, ctx->stream, &st, &badMat));
-    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, "dprt_build_chunk_device: " + std::to_string(st.nonfinite) + " non-finite coordinates");
+    RefitStats st; uint32_t badMat = 0, flags = 0;
+    CK(gpu_build_check(v, mats, ntris, ctx->d_gbuild, ctx->stream, &st, &badMat, d_flags, &flags));
+    if (flags) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": " + flatten_failure(flags));
+    if (st.nonfinite) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": " + std::to_string(st.nonfinite) + " non-finite coordinates");
     if (badMat) return fail(ctx, DPRT_ERR_INVALID, "material id out of range");
     float m = 0.f;
     for (int a = 0; a < 3; a++) m = std::max(m, std::max(std::fabs(st.lo[a]), std::fabs(st.hi[a])));
     std::vector<int64_t> levels, triBase;
     const char* why = nullptr;
     CK(gpu_build_tree(v, ntris, ctx->d_gbuild, ctx->stream, 36, levels, triBase, &why));
-    if (why) return fail(ctx, DPRT_ERR_STATE, std::string("dprt_build_chunk_device: ") + why);
+    if (why) return fail(ctx, DPRT_ERR_STATE, std::string(fn) + ": " + why);
     if ((int)levels.size() - 1 > 36) return fail(ctx, DPRT_ERR_CAPACITY, "BVH8 deeper than the traversal stack");
-    auto mem = std::make_shared<ObjMem>();
     mem->device = ctx->device;
     const int64_t nnodes = levels.back();
     // texture coordinates: 32 bytes per triangle in leaf order behind the triangle array (dprt_bvh8_tri.pad_ = triangle count)
@@ -2278,6 +2297,16 @@ int dprt_build_chunk_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc,
     o.nnodes = nnodes; o.ntris = ntris;
     return upload_objects(ctx);
 }
+}  // namespace
+
+int dprt_build_chunk_device(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* verts9_dev, const void* normals9_dev,
+                            const void* uv6_dev, const void* mat_ids_dev, int64_t ntris) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    int r = build_target(ctx, si, desc, verts9_dev, ntris, "dprt_build_chunk_device");
+    if (r) return r;
+    return build_chunk_on_device(ctx, si, desc, (const float*)verts9_dev, normals9_dev, (const float*)uv6_dev, (const int32_t*)mat_ids_dev,
+                                 ntris, "dprt_build_chunk_device", nullptr, std::make_shared<ObjMem>());
+}
 
 int dprt_build_chunk(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const float* verts9, const float* normals9, const float* uv6,
                      const int32_t* mat_ids, int64_t ntris) {
@@ -2295,6 +2324,123 @@ int dprt_build_chunk(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const 
     if (uv6) CK(cudaMemcpyAsync(d + ou, uv6, b6, cudaMemcpyHostToDevice, ctx->stream));
     if (mat_ids) CK(cudaMemcpyAsync(d + om, mat_ids, b1, cudaMemcpyHostToDevice, ctx->stream));
     return dprt_build_chunk_device(ctx, si, desc, d, normals9 ? d + on : nullptr, uv6 ? d + ou : nullptr, mat_ids ? d + om : nullptr, ntris);
+}
+
+// ---- instanced objects built and moved on the GPU (instance_flatten.cu, DESIGN.md 3.11) --------------------------------------
+namespace {
+size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// The device flatten of nt triangles of n instances, in the context's I/O buffer: the flattened streams (uv6 only when wanted,
+// mat_ids only for a build), the instance table, the flag word and the flatten scratch. Copies the instance table in, zeroes the
+// flags and enqueues the flatten; the caller reads the flags back with its own checks.
+struct FlattenIo { float* v; float* n; float* uv; int32_t* mats; uint32_t* flags; };
+int flatten_on_device(dprt_ctx* ctx, const DevMesh* meshTable, const dprt_instance_desc* instances, int64_t n, int64_t nt, bool uv,
+                      bool mats, FlattenIo& io) {
+    const size_t b9 = align256((size_t)nt * 9 * sizeof(float)), b6 = uv ? align256((size_t)nt * 6 * sizeof(float)) : 0;
+    const size_t b1 = mats ? align256((size_t)nt * sizeof(int32_t)) : 0, bi = align256((size_t)n * sizeof(dprt_instance_desc));
+    const size_t oi = 2 * b9 + b6 + b1, of = oi + bi, os = of + 256;
+    int r = ensure_io(ctx, os + instance_flatten_scratch_bytes(n));
+    if (r) return r;
+    char* d = (char*)ctx->d_io;
+    io.v = (float*)d; io.n = (float*)(d + b9);
+    io.uv = uv ? (float*)(d + 2 * b9) : nullptr;
+    io.mats = mats ? (int32_t*)(d + 2 * b9 + b6) : nullptr;
+    io.flags = (uint32_t*)(d + of);
+    const dprt_instance_desc* inst = (const dprt_instance_desc*)(d + oi);
+    CK(cudaMemcpyAsync(d + oi, instances, (size_t)n * sizeof(dprt_instance_desc), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(io.flags, 0, sizeof(uint32_t), ctx->stream));
+    CK(launch_instance_flatten(meshTable, inst, n, nt, d + os, io.v, io.n, io.uv, io.mats, io.flags, ctx->stream));
+    return 0;
+}
+}  // namespace
+
+int dprt_build_instanced_chunk(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const dprt_mesh_desc* meshes, int n_meshes,
+                               const dprt_instance_desc* instances, int64_t n_instances) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    const char* fn = "dprt_build_instanced_chunk";
+    if (!desc) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": null object description");
+    const int64_t nt = flatten_count(meshes, n_meshes, instances, n_instances);
+    if (nt <= 0) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": invalid mesh / instance description");
+    int r = build_target(ctx, si, desc, meshes, nt, fn);           // the triangle cap, before any array is copied
+    if (r) return r;
+    if (n_instances >= INT32_MAX) return fail(ctx, DPRT_ERR_CAPACITY, std::string(fn) + ": 2^31 - 1 or more instances");
+    CK(cudaSetDevice(ctx->device));
+    // the chunk's own copy of the indexed meshes: the mesh table, the scan of the meshes' triangle counts, then each mesh's arrays
+    auto mem = std::make_shared<ObjMem>();
+    mem->device = ctx->device;
+    std::vector<DevMesh> table((size_t)n_meshes);
+    std::vector<int64_t> triBase((size_t)n_meshes + 1, 0);
+    bool hasUv = false;
+    size_t bytes = align256(table.size() * sizeof(DevMesh)) + align256(triBase.size() * sizeof(int64_t));
+    for (int k = 0; k < n_meshes; k++) {
+        const dprt_mesh_desc& m = meshes[k];
+        const int64_t t = m.ntris;
+        triBase[k + 1] = triBase[k] + t;
+        if (t == 0) continue;
+        hasUv = hasUv || m.texCoords != nullptr;
+        bytes += align256((size_t)m.nPositions * 12) + align256((size_t)m.nNormals * 12) + 2 * align256((size_t)t * 12);
+        if (m.texCoords) bytes += align256((size_t)m.nTexCoords * 8) + align256((size_t)t * 12);
+    }
+    CK(cudaMalloc(&mem->d_meshes, bytes));
+    char* base = (char*)mem->d_meshes;
+    size_t off = align256(table.size() * sizeof(DevMesh)) + align256(triBase.size() * sizeof(int64_t));
+    cudaError_t copied = cudaSuccess;
+    auto put = [&](const void* src, size_t b) {
+        void* dst = base + off;
+        off += align256(b);
+        if (b && copied == cudaSuccess) copied = cudaMemcpyAsync(dst, src, b, cudaMemcpyHostToDevice, ctx->stream);
+        return dst;
+    };
+    for (int k = 0; k < n_meshes; k++) {
+        const dprt_mesh_desc& m = meshes[k];
+        DevMesh& e = table[k];
+        e = DevMesh{};
+        e.materialID = m.materialID;
+        if (m.ntris == 0) continue;
+        e.ntris = m.ntris; e.nPositions = m.nPositions; e.nNormals = m.nNormals;
+        e.positions = (const float*)put(m.positions, (size_t)m.nPositions * 12);
+        e.indices = (const int32_t*)put(m.indices, (size_t)m.ntris * 12);
+        e.normals = (const float*)put(m.normals, (size_t)m.nNormals * 12);
+        e.normalIndices = (const int32_t*)put(m.normalIndices, (size_t)m.ntris * 12);
+        if (m.texCoords) {
+            e.nTexCoords = m.nTexCoords;
+            e.texCoords = (const float*)put(m.texCoords, (size_t)m.nTexCoords * 8);
+            e.texCoordIndices = (const int32_t*)put(m.texCoordIndices, (size_t)m.ntris * 12);
+        }
+    }
+    CK(copied);
+    CK(cudaMemcpyAsync(base, table.data(), table.size() * sizeof(DevMesh), cudaMemcpyHostToDevice, ctx->stream));
+    const int64_t* d_triBase = (const int64_t*)(base + align256(table.size() * sizeof(DevMesh)));
+    CK(cudaMemcpyAsync((void*)d_triBase, triBase.data(), triBase.size() * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    mem->meshTable = (const DevMesh*)base;
+    mem->instMesh.resize((size_t)n_instances);
+    for (int64_t i = 0; i < n_instances; i++) mem->instMesh[i] = instances[i].mesh;
+    FlattenIo io;
+    if ((r = flatten_on_device(ctx, mem->meshTable, instances, n_instances, nt, hasUv, true, io))) return r;
+    CK(launch_mesh_index_check(mem->meshTable, d_triBase, n_meshes, triBase.back(), io.flags, ctx->stream));
+    return build_chunk_on_device(ctx, si, desc, io.v, io.n, io.uv, io.mats, nt, fn, io.flags, mem);
+}
+
+int dprt_update_instances(dprt_ctx* ctx, int si, const dprt_instance_desc* instances, int64_t n_instances) {
+    if (!ctx) return DPRT_ERR_INVALID;
+    const char* fn = "dprt_update_instances";
+    if (!instances) return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": null instance array");
+    if (si < 0 || si >= ctx->cfg.sceneSize || !ctx->objects[si].present)
+        return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": no scene object uploaded at this index");
+    ObjectHost& o = ctx->objects[si];
+    if (o.desc.isProxy || !o.mem || !o.mem->meshTable)
+        return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": the object was not made by dprt_build_instanced_chunk");
+    const std::vector<int32_t>& instMesh = o.mem->instMesh;
+    if (n_instances != (int64_t)instMesh.size())
+        return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": instance count differs from the build's");
+    for (int64_t i = 0; i < n_instances; i++)
+        if (instances[i].mesh != instMesh[i])
+            return fail(ctx, DPRT_ERR_INVALID, std::string(fn) + ": instance " + std::to_string(i) + " names another mesh than at the build");
+    CK(cudaSetDevice(ctx->device));
+    FlattenIo io;
+    int r = flatten_on_device(ctx, o.mem->meshTable, instances, n_instances, o.ntris, false, false, io);
+    if (r) return r;
+    return refit_chunk_on_device(ctx, &o, io.v, io.n, o.ntris, fn, io.flags);
 }
 
 int dprt_spec_bvh8_build_gpu(const float* verts9, const int32_t* mat_ids, int64_t ntris, dprt_bvh8** out) {

@@ -136,18 +136,38 @@ int spec_bvh8_refit(dprt_bvh8_node* nodes, int64_t nnodes, dprt_bvh8_tri* tris, 
 
 // GPU BVH8 build (bvh_gpu_build.cu, DESIGN.md 3.10); scratch: gpu_build_scratch_bytes(ntris), all calls on one stream.
 // gpu_build_check: the vertices' RefitStats and whether a material id lies outside [0, DPRT_MAX_MATERIALS) (mats may be null),
-// read back with one synchronisation. gpu_build_tree: Morton order, PLOC tree and emission pass 1 (one read-back per PLOC
+// and the caller's device word *flags into *flagsOut (flags may be null), read back with one synchronisation. gpu_build_tree: Morton order, PLOC tree and emission pass 1 (one read-back per PLOC
 // iteration and per level); levels gets the node-index boundaries of the BFS levels (depth = levels.size() - 1, which stops at
 // maxDepth + 1) and triBase the first triangle record of each level; *why is set only when the tree could not be built.
 // launch_gpu_build_write: emission pass 2 into nodes[levels.back()] and tris[ntris] (+ the texture-coordinate tail when uv6).
 size_t gpu_build_scratch_bytes(int64_t ntris);
 cudaError_t gpu_build_check(const float* verts9, const int32_t* mats, int64_t ntris, void* scratch, cudaStream_t stream, RefitStats* st,
-                            uint32_t* badMat);
+                            uint32_t* badMat, const uint32_t* flags, uint32_t* flagsOut);
 cudaError_t gpu_build_tree(const float* verts9, int64_t ntris, void* scratch, cudaStream_t stream, int maxDepth, std::vector<int64_t>& levels,
                            std::vector<int64_t>& triBase, const char** why);
 void launch_gpu_build_write(const float* verts9, const int32_t* mats, const float* uv6, int64_t ntris, float pad, void* scratch,
                             const std::vector<int64_t>& levels, const std::vector<int64_t>& triBase, dprt_bvh8_node* nodes,
                             dprt_bvh8_tri* tris, cudaStream_t stream);
+
+// Device flatten of instanced, indexed meshes (instance_flatten.cu, DESIGN.md 3.11). DevMesh: a dprt_mesh_desc whose arrays are
+// on the device. The launches or kFlatten* bits into *flags (one device word the caller zeroes and reads back).
+// launch_mesh_index_check: every index of the nMeshes meshes against their counts (meshTriBase: the exclusive scan of the
+// meshes' ntris, nMeshes + 1 entries, meshTris the total). launch_instance_flatten: verts9 / normals9 / uv6 / mats (the last two
+// may be null) of the ntris triangles of nInstances instances, in primID order, as flatten_instances writes them; the instance
+// table is on the device and its mesh indices are valid; scratch: instance_flatten_scratch_bytes(nInstances).
+struct DevMesh {
+    const float* positions; const int32_t* indices; const float* normals; const int32_t* normalIndices;
+    const float* texCoords; const int32_t* texCoordIndices;     // null: no texture coordinates
+    int64_t nPositions, nNormals, nTexCoords, ntris;
+    int32_t materialID, pad_;
+};
+enum : uint32_t { kFlattenBadIndex = 1u, kFlattenSingular = 2u };
+size_t instance_flatten_scratch_bytes(int64_t nInstances);
+cudaError_t launch_mesh_index_check(const DevMesh* meshes, const int64_t* meshTriBase, int nMeshes, int64_t meshTris, uint32_t* flags,
+                                    cudaStream_t stream);
+cudaError_t launch_instance_flatten(const DevMesh* meshes, const dprt_instance_desc* instances, int64_t nInstances, int64_t ntris,
+                                    void* scratch, float* verts9, float* normals9, float* uv6, int32_t* mats, uint32_t* flags,
+                                    cudaStream_t stream);
 
 // partition / bucketing (partition.cu)
 struct PartitionScratch {

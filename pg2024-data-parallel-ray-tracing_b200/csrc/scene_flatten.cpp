@@ -9,15 +9,13 @@
 // world-space triangle with three world-space normals and three texture coordinates, stored contiguously per primitive.
 // B200 has 180 GB of HBM; the per-hit cost drops to 36 + 24 contiguous bytes and the BVH is a single level.
 //
-// Arithmetic (the oracle restates it independently, bit for bit):
-//   corner   p_w = M p          per row  fma(m2, z, fma(m1, y, fma(m0, x, m3)))                      (binary32)
-//   normal   n_w = A^-T n       A = upper 3x3 of M; A^-T = cofactors / det evaluated in binary64 in the order written
-//                               below, each entry rounded to binary32; per row fma(g2, nz, fma(g1, ny, g0 * nx))
-// Built with -ffp-contract=off.
+// The instance arithmetic (corners M p, normals A^-T n) is instance_xform.cuh, shared with the device flatten of
+// instance_flatten.cu. Built with -ffp-contract=off.
 #include <cmath>
 #include <cstring>
 
 #include "scene_flatten.h"
+#include "instance_xform.cuh"
 
 namespace dprt {
 
@@ -66,29 +64,14 @@ int flatten_instances(const dprt_mesh_desc* meshes, int nMeshes, const dprt_inst
     for (int64_t i = 0; i < nInstances; i++) {
         const dprt_mesh_desc& me = meshes[instances[i].mesh];
         const float* M = instances[i].objectToWorld;
-        const double a00 = M[0], a01 = M[1], a02 = M[2], a10 = M[4], a11 = M[5], a12 = M[6], a20 = M[8], a21 = M[9], a22 = M[10];
-        const double c00 = a11 * a22 - a12 * a21, c01 = -(a10 * a22 - a12 * a20), c02 = a10 * a21 - a11 * a20;
-        const double c10 = -(a01 * a22 - a02 * a21), c11 = a00 * a22 - a02 * a20, c12 = -(a00 * a21 - a01 * a20);
-        const double c20 = a01 * a12 - a02 * a11, c21 = -(a00 * a12 - a02 * a10), c22 = a00 * a11 - a01 * a10;
-        const double det = a00 * c00 + a01 * c01 + a02 * c02;
-        if (!(det != 0.0) || !std::isfinite(det)) return -1;
-        const double inv = 1.0 / det;
-        const float g[9] = {(float)(c00 * inv), (float)(c01 * inv), (float)(c02 * inv), (float)(c10 * inv), (float)(c11 * inv),
-                            (float)(c12 * inv), (float)(c20 * inv), (float)(c21 * inv), (float)(c22 * inv)};
+        float g[9];
+        if (!instance_normal_matrix(M, g)) return -1;
 #pragma omp parallel for schedule(static) if (me.ntris > 4096)
         for (int64_t t = 0; t < me.ntris; t++) {
             const int64_t p = base + t;
             for (int c = 0; c < 3; c++) {
-                const float* v = me.positions + 3 * (int64_t)me.indices[3 * t + c];
-                float* o = verts9 + 9 * p + 3 * c;
-                o[0] = fmaf(M[2], v[2], fmaf(M[1], v[1], fmaf(M[0], v[0], M[3])));
-                o[1] = fmaf(M[6], v[2], fmaf(M[5], v[1], fmaf(M[4], v[0], M[7])));
-                o[2] = fmaf(M[10], v[2], fmaf(M[9], v[1], fmaf(M[8], v[0], M[11])));
-                const float* n = me.normals + 3 * (int64_t)me.normalIndices[3 * t + c];
-                float* q = normals9 + 9 * p + 3 * c;
-                q[0] = fmaf(g[2], n[2], fmaf(g[1], n[1], g[0] * n[0]));
-                q[1] = fmaf(g[5], n[2], fmaf(g[4], n[1], g[3] * n[0]));
-                q[2] = fmaf(g[8], n[2], fmaf(g[7], n[1], g[6] * n[0]));
+                instance_corner(M, me.positions + 3 * (int64_t)me.indices[3 * t + c], verts9 + 9 * p + 3 * c);
+                instance_normal(g, me.normals + 3 * (int64_t)me.normalIndices[3 * t + c], normals9 + 9 * p + 3 * c);
                 if (uv6) {
                     float* u = uv6 + 6 * p + 2 * c;
                     if (me.texCoords) {

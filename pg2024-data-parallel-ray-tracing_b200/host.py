@@ -46,6 +46,8 @@ _PROTOTYPES = {
                                         C.POINTER(C.c_int)]),
     "dprt_upload_chunk_uv": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
     "dprt_upload_instanced_chunk": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
+    "dprt_build_instanced_chunk": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(D.ObjectDesc), C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
+    "dprt_update_instances": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
     "dprt_set_texture": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]),
     "dprt_set_material_textures": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "dprt_set_env_map": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float]),
@@ -479,7 +481,7 @@ class Renderer:
 
     def refit_chunk(self, scene_index, verts9, normals9=None):
         """dprt_refit_chunk: moved corners (and normals, when the chunk has them) of local chunk scene_index, same triangles.
-        Instanced objects: flatten_instances with the moved instances, then this."""
+        Instanced objects made by build_instanced_chunk move with update_instances instead."""
         v = np.ascontiguousarray(verts9, np.float32).reshape(-1, 9)
         n = None if normals9 is None else np.ascontiguousarray(normals9, np.float32).reshape(-1, 9)
         self._ck(self.lib.dprt_refit_chunk(self.h, scene_index, _ptr(v), _ptr(n), v.shape[0]), "dprt_refit_chunk")
@@ -519,6 +521,19 @@ class Renderer:
         md, nm, ins, ni, keep = D.pack_meshes(meshes, instances)
         self._ck(self.lib.dprt_upload_instanced_chunk(self.h, scene_index, C.byref(desc), md, nm, ins, ni), "dprt_upload_instanced_chunk")
         del keep
+
+    def build_instanced_chunk(self, scene_index, desc, meshes, instances):
+        """dprt_build_instanced_chunk: upload_instanced_chunk's object flattened and built on the GPU (DESIGN.md 3.11), same
+        arguments; the chunk keeps the indexed meshes for update_instances."""
+        md, nm, ins, ni, keep = D.pack_meshes(meshes, instances)
+        self._ck(self.lib.dprt_build_instanced_chunk(self.h, scene_index, C.byref(desc), md, nm, ins, ni), "dprt_build_instanced_chunk")
+        del keep
+
+    def update_instances(self, scene_index, instances):
+        """dprt_update_instances: new (mesh, 3x4 matrix) instances of a build_instanced_chunk object, same count and meshes; the
+        device flattens them and refits the chunk."""
+        _, _, ins, ni, _ = D.pack_meshes([], instances)
+        self._ck(self.lib.dprt_update_instances(self.h, scene_index, ins, ni), "dprt_update_instances")
 
     def set_texture(self, texture_index, rgba):
         """params.albedoTextures[texture_index]: [h, w, 4] float RGBA (alpha = opacity), or None to remove it."""
