@@ -147,11 +147,26 @@ int  dprt_set_material_textures(dprt_ctx* ctx, const int32_t* texture_index, int
  * at (phi / 2pi, theta / pi) after phi += rotation_offset; wraps in u, clamps in v. rgba = NULL restores the analytic sky
  * of cfg.envColor. */
 int  dprt_set_env_map(dprt_ctx* ctx, const float* rgba, int width, int height, float rotation_offset);
+/* Rough conductor (bsdfType 2, DESIGN.md 3.12): a GGX microfacet metal with Schlick Fresnel, F0 = the material's albedo
+ * (baseColor, or the albedo-map texel of a textured material), Smith height-correlated masking, visible-normal sampling for
+ * the next path and f(wi, wo) in place of albedo / pi for the light samples. roughness[m] in [0, 1] is material m's GGX
+ * roughness (alpha = max(r^2, 1e-3)); 0 is a perfect mirror, a delta lobe that takes no light samples, like Water. The table
+ * holds DPRT_MAX_MATERIALS entries, all 0 at create, shared by dprt_adopt_scene, and read only for bsdfType 2 materials.
+ * DPRT_ERR_INVALID with the table unchanged: n outside [1, DPRT_MAX_MATERIALS], an entry not finite or outside [0, 1].
+ * Waits for the context's streams, then replaces entries [0, n). */
+int  dprt_set_material_roughness(dprt_ctx* ctx, const float* roughness, int n);
 /* The two texture look-ups above on host arrays, compiled from the very source the kernels use (dprt_math.cuh): lets a
  * machine without a GPU compare the arithmetic with the oracle. out4 = n RGBA results. */
 int  dprt_spec_texture_sample(const float* rgba, int width, int height, const float* u, const float* v, int64_t n, int clamp_v,
                               float* out4);
 int  dprt_spec_env_lookup(const float* rgba, int width, int height, float rotation_offset, const float* dirs3, int64_t n, float* out3);
+/* The conductor on host arrays, from the source the shading kernel compiles (conductor.cuh), per entry i: f0[3i..3i+2],
+ * roughness[i], the local outgoing direction wo[3i..3i+2] (+z = the face-forwarded shading normal). _sample takes the two
+ * uniforms xi[2i], xi[2i+1] and writes the next direction wi and the throughput factor weight (both 0 when the path ends);
+ * _eval writes f(wi, wo) per channel. */
+int  dprt_spec_conductor_sample(const float* f0, const float* roughness, const float* wo, const float* xi, int64_t n, float* wi,
+                                float* weight);
+int  dprt_spec_conductor_eval(const float* f0, const float* roughness, const float* wo, const float* wi, int64_t n, float* f);
 
 int  dprt_set_materials(dprt_ctx* ctx, const dprt_material* mats, int n);
 int  dprt_set_lights(dprt_ctx* ctx, const dprt_light_tri* lights, int n);   /* renderer.cpp:1798-1808 */

@@ -79,7 +79,8 @@ typedef struct dprt_object_desc {
 /* HitGroupData subset (pipeline_helper.cpp:182-193): per-mesh base colour and BSDF type. */
 typedef struct dprt_material {
     float   baseColor[3];
-    int32_t bsdfType;         /* 0 = Diffuse (Lambertian), 1 = Water */
+    int32_t bsdfType;         /* 0 = Diffuse (Lambertian), 1 = Water, 2 = rough conductor (baseColor is F0; roughness from
+                                 dprt_set_material_roughness, DESIGN.md 3.12); any other value shades as 0 */
 } dprt_material;
 
 /* ---- real-scene front end (SURVEY.md 8f row 3) ------------------------------------------------------------------------

@@ -142,6 +142,7 @@ struct dprt_ctx {
     // real-scene front end: texture table (DPRT_MAX_TEXTURES slots), texture index per material (-1 = none), environment map
     DevTexture* d_textures = nullptr;
     int32_t* d_matTex = nullptr;
+    float* d_roughness = nullptr;                  // DPRT_MAX_MATERIALS entries (dprt_set_material_roughness), read for bsdfType 2
     std::shared_ptr<TexMem> tex[DPRT_MAX_TEXTURES];
     std::shared_ptr<TexMem> envTex;
     size_t buf_bytes[DPRT_BUF_COUNT] = {0};
@@ -405,6 +406,8 @@ static int create_impl(const dprt_config* cfg, int rank, int world, int device, 
         CK(cudaMemsetAsync(ctx->d_textures, 0, sizeof(DevTexture) * DPRT_MAX_TEXTURES, ctx->stream));      // texels == null: empty slot
         CK(cudaMalloc(&ctx->d_matTex, sizeof(int32_t) * DPRT_MAX_MATERIALS));
         CK(cudaMemsetAsync(ctx->d_matTex, 0xff, sizeof(int32_t) * DPRT_MAX_MATERIALS, ctx->stream));        // -1: untextured
+        CK(cudaMalloc(&ctx->d_roughness, sizeof(float) * DPRT_MAX_MATERIALS));
+        CK(cudaMemsetAsync(ctx->d_roughness, 0, sizeof(float) * DPRT_MAX_MATERIALS, ctx->stream));          // 0: mirror
         int r;
         if ((r = alloc_buf(ctx, DPRT_BUF_PATHS, (1 + spc) * N * sizeof(dprt_path_record)))) return r;
         if ((r = alloc_buf(ctx, DPRT_BUF_TRANSFER, N * sizeof(dprt_path_record)))) return r;
@@ -531,6 +534,7 @@ void dprt_destroy(dprt_ctx* ctx) {
     if (ctx->d_lights) cudaFree(ctx->d_lights);
     if (ctx->d_textures) cudaFree(ctx->d_textures);
     if (ctx->d_matTex) cudaFree(ctx->d_matTex);
+    if (ctx->d_roughness) cudaFree(ctx->d_roughness);
     for (auto& t : ctx->tex) t.reset();
     ctx->envTex.reset();
     if (ctx->d_hist) cudaFree(ctx->d_hist);
@@ -779,6 +783,17 @@ int dprt_set_material_textures(dprt_ctx* ctx, const int32_t* texture_index, int 
     return 0;
 }
 
+int dprt_set_material_roughness(dprt_ctx* ctx, const float* roughness, int n) {
+    if (!ctx || !roughness || n < 1 || n > DPRT_MAX_MATERIALS) return DPRT_ERR_INVALID;
+    for (int i = 0; i < n; i++)      // !(r >= 0 && r <= 1) also rejects NaN; infinities are outside [0, 1]
+        if (!(roughness[i] >= 0.0f && roughness[i] <= 1.0f)) return fail(ctx, DPRT_ERR_INVALID, "roughness must be finite and in [0, 1]");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));            // nothing in flight shades with the old table
+    if (ctx->aux) CK(cudaStreamSynchronize(ctx->aux));
+    CK(cudaMemcpy(ctx->d_roughness, roughness, sizeof(float) * n, cudaMemcpyHostToDevice));
+    return 0;
+}
+
 int dprt_set_env_map(dprt_ctx* ctx, const float* rgba, int width, int height, float rotation_offset) {
     if (!ctx) return DPRT_ERR_INVALID;
     if (rgba && (width < 1 || height < 1 || (int64_t)width * height > ((int64_t)1 << 28))) return fail(ctx, DPRT_ERR_INVALID, "environment map size");
@@ -799,6 +814,12 @@ int dprt_spec_texture_sample(const float* rgba, int width, int height, const flo
 }
 int dprt_spec_env_lookup(const float* rgba, int width, int height, float rotation_offset, const float* dirs3, int64_t n, float* out3) {
     return spec_env_lookup(rgba, width, height, rotation_offset, dirs3, n, out3);
+}
+int dprt_spec_conductor_sample(const float* f0, const float* roughness, const float* wo, const float* xi, int64_t n, float* wi, float* weight) {
+    return spec_conductor_sample(f0, roughness, wo, xi, n, wi, weight);
+}
+int dprt_spec_conductor_eval(const float* f0, const float* roughness, const float* wo, const float* wi, int64_t n, float* f) {
+    return spec_conductor_eval(f0, roughness, wo, wi, n, f);
 }
 
 int dprt_upload_proxy(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* vis_blob, size_t vis_bytes,
@@ -835,6 +856,7 @@ int dprt_adopt_scene(dprt_ctx* ctx, dprt_ctx* from) {
     for (int i = 0; i < DPRT_MAX_TEXTURES; i++) ctx->tex[i] = from->tex[i];                 // shares the texels (TexMem)
     CK(cudaMemcpy(ctx->d_textures, from->d_textures, sizeof(DevTexture) * DPRT_MAX_TEXTURES, cudaMemcpyDeviceToDevice));
     CK(cudaMemcpy(ctx->d_matTex, from->d_matTex, sizeof(int32_t) * DPRT_MAX_MATERIALS, cudaMemcpyDeviceToDevice));
+    CK(cudaMemcpy(ctx->d_roughness, from->d_roughness, sizeof(float) * DPRT_MAX_MATERIALS, cudaMemcpyDeviceToDevice));
     ctx->envTex = from->envTex; ctx->hp.envMap = from->hp.envMap; ctx->hp.envRotation = from->hp.envRotation;
     ctx->hp.lightCount = from->hp.lightCount;
     if (from->hp.camera.width == ctx->cfg.width && from->hp.camera.height == ctx->cfg.height) ctx->hp.camera = from->hp.camera;
@@ -1084,8 +1106,8 @@ int dprt_shade(dprt_ctx* ctx) {
     ctx->recsInTransfer = false;
     float* aov = ctx->aovPending ? ctx->d_aov : nullptr;     // the sample's first shade: the camera paths' first hits
     ctx->aovPending = false;
-    if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, aov, ctx->stream);
-    else launch_shade(ctx->hp, ctx->pathSize, aov, ctx->stream);
+    if (cached) launch_shade_cached(ctx->hp, ctx->pathSize, aov, ctx->d_roughness, ctx->stream);
+    else launch_shade(ctx->hp, ctx->pathSize, aov, ctx->d_roughness, ctx->stream);
     ctx->stats.kernel_launches += (cached ? 1 : 2) * (ctx->pathSize > 0);   // [trace +] post
     ctx->stats.rays_shade += ctx->pathSize;
     ctx->epoch++;                       // the records now hold the next bounce's rays: cached hits are stale

@@ -90,9 +90,10 @@ struct DevParams {
 void launch_path_gen(const DevParams& p, int n, cudaStream_t stream);
 void launch_traverse(const DevParams& p, int n, cudaStream_t stream);
 // aov: first-hit guide buffers (6N floats) to add to, or null (AOVs off, or not the sample's first shade)
-void launch_shade(const DevParams& p, int n, float* aov, cudaStream_t stream);
+// roughness: the material roughness table (DPRT_MAX_MATERIALS floats), read for bsdfType 2 only
+void launch_shade(const DevParams& p, int n, float* aov, const float* roughness, cudaStream_t stream);
 // MainRay without its trace: shades the partition output p.transfer[0..n) with the hits of the hit cache (single rank only)
-void launch_shade_cached(const DevParams& p, int n, float* aov, cudaStream_t stream);
+void launch_shade_cached(const DevParams& p, int n, float* aov, const float* roughness, cudaStream_t stream);
 // proxies off: the any-hit trace also adds the unoccluded terms to directLightingBuffer and no post kernel follows
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t stream);
 void launch_secondary_trace(const DevParams& p, int n, cudaStream_t stream);
@@ -113,6 +114,9 @@ void launch_precom_labels(const DevObject* obj, const dprt_hit* hits, const floa
 // dprt_spec_*: the texture / environment look-ups of dprt_math.cuh on host arrays (kernels.cu: same source, host compile)
 int spec_texture_sample(const float* rgba, int width, int height, const float* u, const float* v, int64_t n, int clampV, float* out4);
 int spec_env_lookup(const float* rgba, int width, int height, float rotationOffset, const float* dirs3, int64_t n, float* out3);
+// the conductor BSDF of conductor.cuh on host arrays (f0, wo, wi, weight, f: 3 floats per entry; xi: 2; r: 1)
+int spec_conductor_sample(const float* f0, const float* r, const float* wo, const float* xi, int64_t n, float* wi, float* weight);
+int spec_conductor_eval(const float* f0, const float* r, const float* wo, const float* wi, int64_t n, float* f);
 
 // denoiser (denoise.cu, DESIGN.md 3.8). denoise_check resolves p (NULL: the defaults) into *out and checks the frame size and
 // parameters: DPRT_ERR_INVALID with the reason in *why. launch_denoise enqueues the pack launch and one launch per iteration on

@@ -15,30 +15,30 @@
 #include <float.h>
 
 #define DPRT_D __device__ __forceinline__
-// also compiled for the host: the texture / environment look-ups are exported as dprt_spec_* so that a machine without a GPU
-// can compare this very source with the oracle
+// also compiled for the host: the texture / environment look-ups and the conductor BSDF (conductor.cuh) are exported as
+// dprt_spec_* so that a machine without a GPU can compare this very source with the oracle
 #define DPRT_HD __host__ __device__ __forceinline__
 
 struct V3 { float x, y, z; };
 
 DPRT_HD V3 v3(float x, float y, float z) { V3 r; r.x = x; r.y = y; r.z = z; return r; }
-DPRT_D V3 v3sub(V3 a, V3 b) { return v3(a.x - b.x, a.y - b.y, a.z - b.z); }
-DPRT_D V3 v3add(V3 a, V3 b) { return v3(a.x + b.x, a.y + b.y, a.z + b.z); }
-DPRT_D V3 v3mul(V3 a, V3 b) { return v3(a.x * b.x, a.y * b.y, a.z * b.z); }
-DPRT_D V3 v3scale(V3 a, float s) { return v3(a.x * s, a.y * s, a.z * s); }
-DPRT_D V3 v3neg(V3 a) { return v3(-a.x, -a.y, -a.z); }
-DPRT_D float v3get(V3 a, int k) { return k == 0 ? a.x : (k == 1 ? a.y : a.z); }
+DPRT_HD V3 v3sub(V3 a, V3 b) { return v3(a.x - b.x, a.y - b.y, a.z - b.z); }
+DPRT_HD V3 v3add(V3 a, V3 b) { return v3(a.x + b.x, a.y + b.y, a.z + b.z); }
+DPRT_HD V3 v3mul(V3 a, V3 b) { return v3(a.x * b.x, a.y * b.y, a.z * b.z); }
+DPRT_HD V3 v3scale(V3 a, float s) { return v3(a.x * s, a.y * s, a.z * s); }
+DPRT_HD V3 v3neg(V3 a) { return v3(-a.x, -a.y, -a.z); }
+DPRT_HD float v3get(V3 a, int k) { return k == 0 ? a.x : (k == 1 ? a.y : a.z); }
 // dot = fma(z,z', fma(y,y', x*x'))
-DPRT_D float v3dot(V3 a, V3 b) { return fmaf(a.z, b.z, fmaf(a.y, b.y, a.x * b.x)); }
+DPRT_HD float v3dot(V3 a, V3 b) { return fmaf(a.z, b.z, fmaf(a.y, b.y, a.x * b.x)); }
 // cross component = fma(a1, b2, -(a2*b1))
-DPRT_D V3 v3cross(V3 a, V3 b) {
+DPRT_HD V3 v3cross(V3 a, V3 b) {
     return v3(fmaf(a.y, b.z, -(a.z * b.y)), fmaf(a.z, b.x, -(a.x * b.z)), fmaf(a.x, b.y, -(a.y * b.x)));
 }
-DPRT_D float v3length(V3 a) { return sqrtf(v3dot(a, a)); }
+DPRT_HD float v3length(V3 a) { return sqrtf(v3dot(a, a)); }
 // normalized = v * (1/length)
-DPRT_D V3 v3normalized(V3 a) { float inv = 1.0f / v3length(a); return v3scale(a, inv); }
+DPRT_HD V3 v3normalized(V3 a) { float inv = 1.0f / v3length(a); return v3scale(a, inv); }
 // point on ray = fma(t, d, o)
-DPRT_D V3 v3at(V3 o, V3 d, float t) { return v3(fmaf(t, d.x, o.x), fmaf(t, d.y, o.y), fmaf(t, d.z, o.z)); }
+DPRT_HD V3 v3at(V3 o, V3 d, float t) { return v3(fmaf(t, d.x, o.x), fmaf(t, d.y, o.y), fmaf(t, d.z, o.z)); }
 
 // ---- RNG: optix/random.hpp:31-67 (integer arithmetic, exact) ----
 DPRT_D uint32_t tea4(uint32_t val0, uint32_t val1) {
@@ -56,7 +56,7 @@ DPRT_D float rnd(uint32_t& prev) { return (float)lcg(prev) / (float)0x01000000; 
 
 // ---- deterministic transcendentals (spec; polynomial coefficients are the Cephes single-precision sets) ----
 // sin/cos of 2*pi*x for x in [0,1).
-DPRT_D void det_sincos2pi(float x, float* s, float* c) {
+DPRT_HD void det_sincos2pi(float x, float* s, float* c) {
     float r = x * 4.0f;                    // exact
     float qf = floorf(r + 0.5f);
     float f = r - qf;                      // in [-0.5, 0.5], exact
@@ -133,7 +133,7 @@ DPRT_D V3 uniform_hemisphere(float xi1, float xi2) {
 }
 
 // ---- Frame(normal).toWorld: branchless orthonormal basis (Duff et al. 2017) ----
-DPRT_D V3 frame_to_world(V3 n, V3 w) {
+DPRT_HD V3 frame_to_world(V3 n, V3 w) {
     float sign = copysignf(1.0f, n.z);
     float a = -1.0f / (sign + n.z);
     float b = n.x * n.y * a;
@@ -143,7 +143,7 @@ DPRT_D V3 frame_to_world(V3 n, V3 w) {
               fmaf(n.y, w.z, fmaf(t.y, w.y, s.y * w.x)),
               fmaf(n.z, w.z, fmaf(t.z, w.y, s.z * w.x)));
 }
-DPRT_D V3 frame_to_local(V3 n, V3 w) {
+DPRT_HD V3 frame_to_local(V3 n, V3 w) {
     float sign = copysignf(1.0f, n.z);
     float a = -1.0f / (sign + n.z);
     float b = n.x * n.y * a;

@@ -18,6 +18,8 @@
 //   | int32 envWidth envHeight (0 0 = analytic sky) | float rotationOffset | float rgba[4 w h]   (params.envLightTexture, :1851)
 //   per object: dprt_object_desc | int64 ntris | int32 hasUv | verts | normals | float uv[6 ntris] if hasUv | mats | vis blob | depth blob
 //   (instanced / indexed meshes arrive flattened: the file is written after dprt_flatten_instances)
+// Rough conductors (real_scene.py:save_scene_v2 when the scene has a roughness table; DESIGN.md 3.12):
+//   "DPRTSCN3" | the DPRTSCN2 layout after its magic | float roughness[nMaterials]   (dprt_set_material_roughness)
 //               [--frames F] [--camera-move dx,dy,dz] [--camera-target x,y,z] [--light-move dx,dy,dz] [--light-start dx,dy,dz]
 //                                      the frame loop of launch() (renderer.cpp:1938-2059): per frame the first two lights move by
 //                                      -light-move (after a one-off +light-start, LIGHT_MOVE :1941-1966) and the camera origin by
@@ -61,6 +63,7 @@ struct Scene {
     dprt_camera cam;
     std::vector<dprt_material> materials;
     std::vector<int32_t> matTex;                     // texture slot per material (-1 = none); empty for DPRTSCN1 files
+    std::vector<float> roughness;                    // per material (bsdfType 2); empty unless DPRTSCN3
     std::vector<dprt_light_tri> lights;
     std::vector<Texture> textures;
     Texture env; float envRotation = 0.f;            // env.w == 0: analytic sky
@@ -80,7 +83,8 @@ bool load_scene(const std::string& path, Scene& sc, std::string& err) {
     if (!f) { err = "cannot open " + path; return false; }
     char magic[8]; int32_t hdr[4] = {0, 0, 0, 0};
     bool ok = read_exact(f, magic, 8);
-    const bool v2 = ok && std::memcmp(magic, "DPRTSCN2", 8) == 0;
+    const bool v3 = ok && std::memcmp(magic, "DPRTSCN3", 8) == 0;
+    const bool v2 = ok && (v3 || std::memcmp(magic, "DPRTSCN2", 8) == 0);
     ok = ok && (v2 || std::memcmp(magic, "DPRTSCN1", 8) == 0) && read_exact(f, hdr, v2 ? 16 : 12);
     if (ok) ok = hdr[0] >= 1 && hdr[0] <= 32 && hdr[1] >= 1 && hdr[1] <= DPRT_MAX_MATERIALS && hdr[2] >= 1 && hdr[2] <= DPRT_MAX_LIGHTS &&
                  hdr[3] >= 0 && hdr[3] <= DPRT_MAX_TEXTURES;
@@ -118,6 +122,7 @@ bool load_scene(const std::string& path, Scene& sc, std::string& err) {
         if (ok) { o.vis.resize((size_t)vb); ok = read_exact(f, o.vis.data(), (size_t)vb) && read_exact(f, &db, 8) && db >= 0 && db < (int64_t(1) << 30); }
         if (ok) { o.depth.resize((size_t)db); ok = read_exact(f, o.depth.data(), (size_t)db); }
     }
+    if (ok && v3) { sc.roughness.resize(sc.materials.size()); ok = read_exact(f, sc.roughness.data(), 4 * sc.roughness.size()); }
     fclose(f);
     if (!ok) err = "malformed scene file " + path;
     return ok;
@@ -240,6 +245,7 @@ int upload_scene(dprt_ctx* ctx, const Scene& sc, int rank, bool gpuBuild) {
     // albedo / opacity maps, texture slot per material, environment map (renderer.cpp:1621-1721, :1851)
     for (const Texture& t : sc.textures) if ((r = dprt_set_texture(ctx, t.slot, t.rgba.data(), t.w, t.h))) return r;
     if (!sc.matTex.empty() && (r = dprt_set_material_textures(ctx, sc.matTex.data(), (int)sc.matTex.size()))) return r;
+    if (!sc.roughness.empty() && (r = dprt_set_material_roughness(ctx, sc.roughness.data(), (int)sc.roughness.size()))) return r;
     if (sc.env.w > 0 && (r = dprt_set_env_map(ctx, sc.env.rgba.data(), sc.env.w, sc.env.h, sc.envRotation))) return r;
     if ((r = dprt_set_lights(ctx, sc.lights.data(), (int)sc.lights.size()))) return r;
     return dprt_set_camera(ctx, &sc.cam);

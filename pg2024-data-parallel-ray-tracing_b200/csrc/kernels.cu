@@ -16,6 +16,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include "bvh_traverse.cuh"
+#include "conductor.cuh"
 
 namespace dprt {
 
@@ -497,8 +498,9 @@ DPRT_D BsdfSample sample_water(float xi1, V3 normal, V3 woWorld, bool isInside) 
 // aov: the first-hit guide buffers (albedo sums 3N, normal sums 3N) when this is the sample's first shade with AOVs on, else
 // null. A kernel argument rather than a DevParams field, so that no other kernel's parameters move. At most one record per
 // pixel reaches the first shade of a sample on a rank, and only the rank that owns the hit shades it: plain adds, no race.
+// roughness: DPRT_MAX_MATERIALS entries, read for bsdfType 2 only (conductor.cuh); a kernel argument for the same reason.
 __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, const dprt_path_record* src, bool fromCache,
-                                                            float* aov) {
+                                                            float* aov, const float* roughness) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) p.traceQueue[0] = 0;
     if (i >= n) return;
@@ -569,7 +571,17 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
     // createSamplingRecord (kernel.cu:50-64): the seed ignores the bounce, as in the reference
     uint32_t seed = tea4((uint32_t)path.pixelIndex, (uint32_t)p.sampleCount);
     const float xi1 = rnd(seed), xi2 = rnd(seed);
-    const BsdfSample bs = mat.bsdfType == 1 ? sample_water(xi1, normal, woWorld, isInside) : sample_lambertian(xi1, xi2);
+    // bsdfType 2, the conductor (DESIGN.md 3.12): albedo is its F0; the throughput factor replaces weight * cos * albedo
+    const bool isCond = mat.bsdfType == 2;
+    BsdfSample bs; CondSample cs; V3 woLocal; float rough = 0.0f;
+    if (isCond) {
+        woLocal = frame_to_local(normal, woWorld);
+        rough = roughness[matID];
+        cs = cond_sample(albedo, rough, woLocal, xi1, xi2);
+        bs.wiLocal = cs.wi; bs.weight = 0.0f; bs.isDelta = rough == 0.0f;
+    } else {
+        bs = mat.bsdfType == 1 ? sample_water(xi1, normal, woWorld, isInside) : sample_lambertian(xi1, xi2);
+    }
 
     // generateNextNewPath (kernel.cu:134-162)
     PathRegs next;
@@ -577,10 +589,11 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
     next.direction = v3normalized(frame_to_world(normal, bs.wiLocal));
     next.tMax = FLT_MAX;
     const float cosThetaWi = fabsf(bs.wiLocal.z);
-    next.throughput = v3mul(v3scale(v3scale(path.throughput, bs.weight), cosThetaWi), albedo);
+    next.throughput = isCond ? v3mul(path.throughput, cs.weight) : v3mul(v3scale(v3scale(path.throughput, bs.weight), cosThetaWi), albedo);
     next.pixelIndex = path.pixelIndex; next.shadowPathID = -1; next.visitedMask = 0u;
     next.currentNode = -1; next.targetNode = -1; next.flags = F_VALID;
-    store_path(p.paths + i, next);
+    if (isCond && !cs.valid) store_zero_path(p.paths + i);              // the rough lobe sampled below the surface: the path ends
+    else store_path(p.paths + i, next);
 
     // generateShadowPath x spc (kernel.cu:66-132, 442-465)
     for (int s = 0; s < p.spc; s++) {
@@ -606,11 +619,13 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
         const float stMax = v3length(ldir);
         const float f1 = fmaxf(0.0f, v3dot(ln, v3neg(wi)));
         const float f2 = fmaxf(0.0f, v3dot(wi, normal));
-        V3 c = v3mul(v3mul(v3(L.Le[0], L.Le[1], L.Le[2]), path.throughput), albedo);
+        // the conductor's f(wi, wo) takes the place of Lambert's albedo * 1/pi
+        const V3 fr = isCond ? cond_eval(albedo, rough, woLocal, frame_to_local(normal, wi)) : albedo;
+        V3 c = v3mul(v3mul(v3(L.Le[0], L.Le[1], L.Le[2]), path.throughput), fr);
         c = v3scale(v3scale(c, f1), f2);
         const float tt = stMax * stMax;
         c = v3(c.x / areaPDF / tt, c.y / areaPDF / tt, c.z / areaPDF / tt);
-        c = v3scale(c, 0.318309886183790671538f);
+        if (!isCond) c = v3scale(c, 0.318309886183790671538f);
         PathRegs sh;
         sh.origin = point; sh.direction = wi; sh.tMax = stMax; sh.throughput = c;
         sh.pixelIndex = path.pixelIndex; sh.shadowPathID = s; sh.visitedMask = 0u; sh.currentNode = -1; sh.targetNode = -1;
@@ -902,6 +917,27 @@ int spec_env_lookup(const float* rgba, int width, int height, float rotationOffs
     return 0;
 }
 
+// dprt_spec_conductor_sample / dprt_spec_conductor_eval: host loops over conductor.cuh
+int spec_conductor_sample(const float* f0, const float* r, const float* wo, const float* xi, int64_t n, float* wi, float* weight) {
+    if (!f0 || !r || !wo || !xi || !wi || !weight || n < 0) return DPRT_ERR_INVALID;
+    for (int64_t i = 0; i < n; i++) {
+        const CondSample s = cond_sample(v3(f0[3 * i], f0[3 * i + 1], f0[3 * i + 2]), r[i], v3(wo[3 * i], wo[3 * i + 1], wo[3 * i + 2]),
+                                         xi[2 * i], xi[2 * i + 1]);
+        wi[3 * i] = s.wi.x; wi[3 * i + 1] = s.wi.y; wi[3 * i + 2] = s.wi.z;
+        weight[3 * i] = s.weight.x; weight[3 * i + 1] = s.weight.y; weight[3 * i + 2] = s.weight.z;
+    }
+    return 0;
+}
+int spec_conductor_eval(const float* f0, const float* r, const float* wo, const float* wi, int64_t n, float* f) {
+    if (!f0 || !r || !wo || !wi || !f || n < 0) return DPRT_ERR_INVALID;
+    for (int64_t i = 0; i < n; i++) {
+        const V3 v = cond_eval(v3(f0[3 * i], f0[3 * i + 1], f0[3 * i + 2]), r[i], v3(wo[3 * i], wo[3 * i + 1], wo[3 * i + 2]),
+                               v3(wi[3 * i], wi[3 * i + 1], wi[3 * i + 2]));
+        f[3 * i] = v.x; f[3 * i + 1] = v.y; f[3 * i + 2] = v.z;
+    }
+    return 0;
+}
+
 size_t trace_scratch_bytes() {
     // 64 B for the ray-queue head + one cooperative-mode node pool per warp that can be resident
     return 64 + (size_t)num_sms() * std::max(tune_blocks(), 8) * (kTraceBlock / 32) * DPRT_POOLCAP * sizeof(uint32_t);
@@ -924,13 +960,13 @@ void launch_traverse(const DevParams& p, int n, cudaStream_t s) {
     launch_trace<TM_TRAVERSE>(trace_args(p, p.paths), n, s);
     traverse_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n);
 }
-void launch_shade(const DevParams& p, int n, float* aov, cudaStream_t s) {
+void launch_shade(const DevParams& p, int n, float* aov, const float* roughness, cudaStream_t s) {
     if (n <= 0) return;
     launch_trace<TM_SHADE>(trace_args(p, p.paths), n, s);
-    shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.paths, false, aov);
+    shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.paths, false, aov, roughness);
 }
-void launch_shade_cached(const DevParams& p, int n, float* aov, cudaStream_t s) {
-    if (n > 0) shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.transfer, true, aov);
+void launch_shade_cached(const DevParams& p, int n, float* aov, const float* roughness, cudaStream_t s) {
+    if (n > 0) shade_post_kernel<<<blocks_for(n), kBlock, 0, s>>>(p, n, p.transfer, true, aov, roughness);
 }
 void launch_shadow_trace(const DevParams& p, int nShadow, cudaStream_t s) {
     if (nShadow <= 0) return;

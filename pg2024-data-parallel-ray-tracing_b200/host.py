@@ -51,6 +51,9 @@ _PROTOTYPES = {
     "dprt_set_texture": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]),
     "dprt_set_material_textures": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "dprt_set_env_map": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float]),
+    "dprt_set_material_roughness": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
+    "dprt_spec_conductor_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "dprt_spec_conductor_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "dprt_spec_texture_sample": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "dprt_spec_env_lookup": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_int64, C.c_void_p]),
     "dprt_set_materials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
@@ -251,6 +254,38 @@ def spec_env_lookup(rgba, rotation, dirs):
     rc = load_library().dprt_spec_env_lookup(_ptr(t), t.shape[1], t.shape[0], float(rotation), _ptr(d), d.shape[0], _ptr(out))
     if rc:
         raise DprtError(f"dprt_spec_env_lookup failed ({rc})")
+    return out
+
+
+def _conductor_args(f0, roughness, wo):
+    wo = np.ascontiguousarray(wo, np.float32).reshape(-1, 3)
+    n = wo.shape[0]
+    f0 = np.ascontiguousarray(np.broadcast_to(np.asarray(f0, np.float32), (n, 3)))
+    r = np.ascontiguousarray(np.broadcast_to(np.asarray(roughness, np.float32), (n,)))
+    return f0, r, wo, n
+
+
+def spec_conductor_sample(f0, roughness, wo, xi):
+    """dprt_spec_conductor_sample (host only): the conductor's next direction wi [n, 3] and throughput factor [n, 3] for local
+    outgoing directions wo [n, 3] and uniforms xi [n, 2] (DESIGN.md 3.12); both 0 where the path ends. f0 [n, 3] or [3],
+    roughness [n] or scalar."""
+    f0, r, wo, n = _conductor_args(f0, roughness, wo)
+    x = np.ascontiguousarray(np.broadcast_to(np.asarray(xi, np.float32), (n, 2)))
+    wi, wt = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32)
+    rc = load_library().dprt_spec_conductor_sample(_ptr(f0), _ptr(r), _ptr(wo), _ptr(x), n, _ptr(wi), _ptr(wt))
+    if rc:
+        raise DprtError(f"dprt_spec_conductor_sample failed ({rc})")
+    return wi, wt
+
+
+def spec_conductor_eval(f0, roughness, wo, wi):
+    """dprt_spec_conductor_eval (host only): the conductor's f(wi, wo) [n, 3] for local directions wo, wi [n, 3]."""
+    f0, r, wo, n = _conductor_args(f0, roughness, wo)
+    w = np.ascontiguousarray(np.broadcast_to(np.asarray(wi, np.float32).reshape(-1, 3), (n, 3)))
+    out = np.zeros((n, 3), np.float32)
+    rc = load_library().dprt_spec_conductor_eval(_ptr(f0), _ptr(r), _ptr(wo), _ptr(w), n, _ptr(out))
+    if rc:
+        raise DprtError(f"dprt_spec_conductor_eval failed ({rc})")
     return out
 
 
@@ -547,6 +582,11 @@ class Renderer:
     def set_material_textures(self, texture_index):
         t = np.ascontiguousarray(texture_index, np.int32)
         self._ck(self.lib.dprt_set_material_textures(self.h, _ptr(t), t.size), "dprt_set_material_textures")
+
+    def set_material_roughness(self, roughness):
+        """GGX roughness in [0, 1] of materials 0 .. len - 1, read for bsdfType 2 (the conductor; 0 = mirror)."""
+        r = np.ascontiguousarray(roughness, np.float32)
+        self._ck(self.lib.dprt_set_material_roughness(self.h, _ptr(r), r.size), "dprt_set_material_roughness")
 
     def set_env_map(self, rgba, rotation_offset=0.0):
         """params.envLightTexture: [h, w, 4] float lat-long map, or None for the analytic sky."""

@@ -358,14 +358,21 @@ def save_scene_v2(path, garden, cam, flatten):
     """Scene file of the C++ host in its real-scene variant (csrc/dprt_render.cpp documents the layout): the dict of make_garden
     (or the same keys filled from load_obj / load_texture) with every object flattened by `flatten` = host.flatten_instances
     (dprt_flatten_instances: what dprt_upload_instanced_chunk would do); an object that already carries its flat streams
-    as `.flat = (verts9, normals9, uv6 or None, mat_ids)` is written as is (obj2scene.py cuts one flattened scene into chunks)."""
+    as `.flat = (verts9, normals9, uv6 or None, mat_ids)` is written as is (obj2scene.py cuts one flattened scene into chunks).
+    A scene with a "material_roughness" table (one float per material, dprt_set_material_roughness) is written as DPRTSCN3:
+    the same bytes after the magic, then the table."""
     import ctypes as C
     mats, mat_tex = np.ascontiguousarray(garden["materials"], D.MATERIAL_DTYPE), np.full(len(garden["materials"]), -1, np.int32)
     mt = np.asarray(garden.get("material_textures", []), np.int32)
     mat_tex[:mt.size] = mt
     textures = garden.get("textures") or {}
+    rough = garden.get("material_roughness")
+    if rough is not None:
+        rough = np.ascontiguousarray(rough, np.float32)
+        if rough.shape != (len(mats),):
+            raise ValueError(f"material_roughness has shape {rough.shape}, the scene has {len(mats)} materials")
     with open(path, "wb") as f:
-        f.write(b"DPRTSCN2")
+        f.write(b"DPRTSCN2" if rough is None else b"DPRTSCN3")
         f.write(np.array([len(garden["objects"]), len(mats), len(garden["lights"]), len(textures)], np.int32).tobytes())
         f.write(bytes(C.string_at(C.addressof(cam), C.sizeof(cam))))
         f.write(mats.tobytes()); f.write(mat_tex.tobytes())
@@ -391,3 +398,5 @@ def save_scene_v2(path, garden, cam, flatten):
                 f.write(np.ascontiguousarray(uv, np.float32).tobytes())
             f.write(np.ascontiguousarray(m, np.int32).tobytes())
             f.write(np.array([0], np.int64).tobytes()); f.write(np.array([0], np.int64).tobytes())      # no proxy networks
+        if rough is not None:
+            f.write(rough.tobytes())
