@@ -151,7 +151,9 @@ int  dprt_set_env_map(dprt_ctx* ctx, const float* rgba, int width, int height, f
  * (baseColor, or the albedo-map texel of a textured material), Smith height-correlated masking, visible-normal sampling for
  * the next path and f(wi, wo) in place of albedo / pi for the light samples. roughness[m] in [0, 1] is material m's GGX
  * roughness (alpha = max(r^2, 1e-3)); 0 is a perfect mirror, a delta lobe that takes no light samples, like Water. The table
- * holds DPRT_MAX_MATERIALS entries, all 0 at create, shared by dprt_adopt_scene, and read only for bsdfType 2 materials.
+ * holds DPRT_MAX_MATERIALS entries, all 0 at create, shared by dprt_adopt_scene, and read only for bsdfType 2 and 3 materials.
+ * For the glossy plastic (bsdfType 3, DESIGN.md 3.13) it is the roughness of the coat's specular lobe; 0 is a smooth coat whose
+ * specular lobe is a mirror, while its diffuse base still takes the light samples.
  * DPRT_ERR_INVALID with the table unchanged: n outside [1, DPRT_MAX_MATERIALS], an entry not finite or outside [0, 1].
  * Waits for the context's streams, then replaces entries [0, n). */
 int  dprt_set_material_roughness(dprt_ctx* ctx, const float* roughness, int n);
@@ -167,6 +169,12 @@ int  dprt_spec_env_lookup(const float* rgba, int width, int height, float rotati
 int  dprt_spec_conductor_sample(const float* f0, const float* roughness, const float* wo, const float* xi, int64_t n, float* wi,
                                 float* weight);
 int  dprt_spec_conductor_eval(const float* f0, const float* roughness, const float* wo, const float* wi, int64_t n, float* f);
+/* The glossy plastic on host arrays, from the source the shading kernel compiles (plastic.cuh), per entry i: the diffuse colour
+ * albedo[3i..3i+2], roughness[i], wo[3i..3i+2] as above. _sample takes three uniforms xi[3i..3i+2] (the third chooses the lobe)
+ * and writes wi and weight (both 0 when the path ends); _eval writes f(wi, wo) per channel. */
+int  dprt_spec_plastic_sample(const float* albedo, const float* roughness, const float* wo, const float* xi, int64_t n, float* wi,
+                              float* weight);
+int  dprt_spec_plastic_eval(const float* albedo, const float* roughness, const float* wo, const float* wi, int64_t n, float* f);
 
 int  dprt_set_materials(dprt_ctx* ctx, const dprt_material* mats, int n);
 int  dprt_set_lights(dprt_ctx* ctx, const dprt_light_tri* lights, int n);   /* renderer.cpp:1798-1808 */

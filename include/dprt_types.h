@@ -80,7 +80,9 @@ typedef struct dprt_object_desc {
 typedef struct dprt_material {
     float   baseColor[3];
     int32_t bsdfType;         /* 0 = Diffuse (Lambertian), 1 = Water, 2 = rough conductor (baseColor is F0; roughness from
-                                 dprt_set_material_roughness, DESIGN.md 3.12); any other value shades as 0 */
+                                 dprt_set_material_roughness, DESIGN.md 3.12), 3 = glossy plastic (baseColor is the diffuse
+                                 colour under a GGX coat of F0 0.04 and the same roughness, DESIGN.md 3.13); any other value
+                                 shades as 0 */
 } dprt_material;
 
 /* ---- real-scene front end (SURVEY.md 8f row 3) ------------------------------------------------------------------------

@@ -14,8 +14,8 @@ from . import ctypes_defs, host, proxy, proxy_train, real_scene, scene  # noqa: 
 from .ctypes_defs import make_camera, make_config, make_object_desc  # noqa: F401
 from .host import (DprtError, RankGroup, Renderer, SamplesInFlight, build_bvh8, flatten_instances, get_unique_id, load_library,  # noqa: F401
                    plan_exchange, plan_exchange_deque, spec_bvh8_build_gpu, spec_bvh8_refit, spec_conductor_eval, spec_conductor_sample, spec_denoise,
-                   spec_env_lookup, spec_texture_sample)
+                   spec_env_lookup, spec_plastic_eval, spec_plastic_sample, spec_texture_sample)
 
 __all__ = ["ctypes_defs", "host", "proxy", "proxy_train", "real_scene", "scene", "make_camera", "make_config", "make_object_desc", "DprtError",
            "RankGroup", "Renderer", "SamplesInFlight", "build_bvh8", "flatten_instances", "get_unique_id", "load_library", "spec_bvh8_build_gpu", "spec_bvh8_refit", "spec_conductor_eval", "spec_conductor_sample", "spec_denoise",
-           "spec_env_lookup", "spec_texture_sample"]
+           "spec_env_lookup", "spec_plastic_eval", "spec_plastic_sample", "spec_texture_sample"]

@@ -142,7 +142,7 @@ struct dprt_ctx {
     // real-scene front end: texture table (DPRT_MAX_TEXTURES slots), texture index per material (-1 = none), environment map
     DevTexture* d_textures = nullptr;
     int32_t* d_matTex = nullptr;
-    float* d_roughness = nullptr;                  // DPRT_MAX_MATERIALS entries (dprt_set_material_roughness), read for bsdfType 2
+    float* d_roughness = nullptr;                  // DPRT_MAX_MATERIALS entries (dprt_set_material_roughness), read for bsdfType 2 and 3
     std::shared_ptr<TexMem> tex[DPRT_MAX_TEXTURES];
     std::shared_ptr<TexMem> envTex;
     size_t buf_bytes[DPRT_BUF_COUNT] = {0};
@@ -820,6 +820,12 @@ int dprt_spec_conductor_sample(const float* f0, const float* roughness, const fl
 }
 int dprt_spec_conductor_eval(const float* f0, const float* roughness, const float* wo, const float* wi, int64_t n, float* f) {
     return spec_conductor_eval(f0, roughness, wo, wi, n, f);
+}
+int dprt_spec_plastic_sample(const float* albedo, const float* roughness, const float* wo, const float* xi, int64_t n, float* wi, float* weight) {
+    return spec_plastic_sample(albedo, roughness, wo, xi, n, wi, weight);
+}
+int dprt_spec_plastic_eval(const float* albedo, const float* roughness, const float* wo, const float* wi, int64_t n, float* f) {
+    return spec_plastic_eval(albedo, roughness, wo, wi, n, f);
 }
 
 int dprt_upload_proxy(dprt_ctx* ctx, int si, const dprt_object_desc* desc, const void* vis_blob, size_t vis_bytes,

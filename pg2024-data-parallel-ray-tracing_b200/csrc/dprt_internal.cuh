@@ -117,6 +117,9 @@ int spec_env_lookup(const float* rgba, int width, int height, float rotationOffs
 // the conductor BSDF of conductor.cuh on host arrays (f0, wo, wi, weight, f: 3 floats per entry; xi: 2; r: 1)
 int spec_conductor_sample(const float* f0, const float* r, const float* wo, const float* xi, int64_t n, float* wi, float* weight);
 int spec_conductor_eval(const float* f0, const float* r, const float* wo, const float* wi, int64_t n, float* f);
+// the plastic BSDF of plastic.cuh on host arrays (albedo, wo, wi, weight, f: 3 floats per entry; xi: 3; r: 1)
+int spec_plastic_sample(const float* albedo, const float* r, const float* wo, const float* xi, int64_t n, float* wi, float* weight);
+int spec_plastic_eval(const float* albedo, const float* r, const float* wo, const float* wi, int64_t n, float* f);
 
 // denoiser (denoise.cu, DESIGN.md 3.8). denoise_check resolves p (NULL: the defaults) into *out and checks the frame size and
 // parameters: DPRT_ERR_INVALID with the reason in *why. launch_denoise enqueues the pack launch and one launch per iteration on

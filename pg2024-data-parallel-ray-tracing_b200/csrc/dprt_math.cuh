@@ -15,8 +15,8 @@
 #include <float.h>
 
 #define DPRT_D __device__ __forceinline__
-// also compiled for the host: the texture / environment look-ups and the conductor BSDF (conductor.cuh) are exported as
-// dprt_spec_* so that a machine without a GPU can compare this very source with the oracle
+// also compiled for the host: the texture / environment look-ups and the conductor and plastic BSDFs (conductor.cuh,
+// plastic.cuh) are exported as dprt_spec_* so that a machine without a GPU can compare this very source with the oracle
 #define DPRT_HD __host__ __device__ __forceinline__
 
 struct V3 { float x, y, z; };
@@ -125,7 +125,7 @@ DPRT_HD void det_cartesian_to_spherical(V3 d, float* phi, float* theta) {
 }
 
 // ---- Sample::uniformHemisphere: optix/sample.hpp:7-17 ----
-DPRT_D V3 uniform_hemisphere(float xi1, float xi2) {
+DPRT_HD V3 uniform_hemisphere(float xi1, float xi2) {
     float z = xi1;
     float r = sqrtf(fmaxf(0.0f, fmaf(-z, z, 1.0f)));
     float s, c; det_sincos2pi(xi2, &s, &c);

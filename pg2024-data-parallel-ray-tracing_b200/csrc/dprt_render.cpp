@@ -18,7 +18,7 @@
 //   | int32 envWidth envHeight (0 0 = analytic sky) | float rotationOffset | float rgba[4 w h]   (params.envLightTexture, :1851)
 //   per object: dprt_object_desc | int64 ntris | int32 hasUv | verts | normals | float uv[6 ntris] if hasUv | mats | vis blob | depth blob
 //   (instanced / indexed meshes arrive flattened: the file is written after dprt_flatten_instances)
-// Rough conductors (real_scene.py:save_scene_v2 when the scene has a roughness table; DESIGN.md 3.12):
+// Rough conductors and glossy plastics (real_scene.py:save_scene_v2 when the scene has a roughness table; DESIGN.md 3.12, 3.13):
 //   "DPRTSCN3" | the DPRTSCN2 layout after its magic | float roughness[nMaterials]   (dprt_set_material_roughness)
 //               [--frames F] [--camera-move dx,dy,dz] [--camera-target x,y,z] [--light-move dx,dy,dz] [--light-start dx,dy,dz]
 //                                      the frame loop of launch() (renderer.cpp:1938-2059): per frame the first two lights move by
@@ -63,7 +63,7 @@ struct Scene {
     dprt_camera cam;
     std::vector<dprt_material> materials;
     std::vector<int32_t> matTex;                     // texture slot per material (-1 = none); empty for DPRTSCN1 files
-    std::vector<float> roughness;                    // per material (bsdfType 2); empty unless DPRTSCN3
+    std::vector<float> roughness;                    // per material (bsdfType 2 and 3); empty unless DPRTSCN3
     std::vector<dprt_light_tri> lights;
     std::vector<Texture> textures;
     Texture env; float envRotation = 0.f;            // env.w == 0: analytic sky

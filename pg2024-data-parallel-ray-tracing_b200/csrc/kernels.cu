@@ -16,7 +16,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include "bvh_traverse.cuh"
-#include "conductor.cuh"
+#include "plastic.cuh"
 
 namespace dprt {
 
@@ -498,7 +498,8 @@ DPRT_D BsdfSample sample_water(float xi1, V3 normal, V3 woWorld, bool isInside) 
 // aov: the first-hit guide buffers (albedo sums 3N, normal sums 3N) when this is the sample's first shade with AOVs on, else
 // null. A kernel argument rather than a DevParams field, so that no other kernel's parameters move. At most one record per
 // pixel reaches the first shade of a sample on a rank, and only the rank that owns the hit shades it: plain adds, no race.
-// roughness: DPRT_MAX_MATERIALS entries, read for bsdfType 2 only (conductor.cuh); a kernel argument for the same reason.
+// roughness: DPRT_MAX_MATERIALS entries, read for bsdfType 2 and 3 only (conductor.cuh, plastic.cuh); a kernel argument for
+// the same reason.
 __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, const dprt_path_record* src, bool fromCache,
                                                             float* aov, const float* roughness) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -571,14 +572,15 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
     // createSamplingRecord (kernel.cu:50-64): the seed ignores the bounce, as in the reference
     uint32_t seed = tea4((uint32_t)path.pixelIndex, (uint32_t)p.sampleCount);
     const float xi1 = rnd(seed), xi2 = rnd(seed);
-    // bsdfType 2, the conductor (DESIGN.md 3.12): albedo is its F0; the throughput factor replaces weight * cos * albedo
-    const bool isCond = mat.bsdfType == 2;
+    // bsdfType 2, the conductor (DESIGN.md 3.12; albedo is its F0), and 3, the plastic (DESIGN.md 3.13; albedo is its diffuse
+    // colour, and it draws a third uniform to choose its lobe): their throughput factor replaces weight * cos * albedo
+    const bool isCond = mat.bsdfType == 2, isGlossy = isCond || mat.bsdfType == 3;
     BsdfSample bs; CondSample cs; V3 woLocal; float rough = 0.0f;
-    if (isCond) {
+    if (isGlossy) {
         woLocal = frame_to_local(normal, woWorld);
         rough = roughness[matID];
-        cs = cond_sample(albedo, rough, woLocal, xi1, xi2);
-        bs.wiLocal = cs.wi; bs.weight = 0.0f; bs.isDelta = rough == 0.0f;
+        cs = isCond ? cond_sample(albedo, rough, woLocal, xi1, xi2) : plastic_sample(albedo, rough, woLocal, xi1, xi2, rnd(seed));
+        bs.wiLocal = cs.wi; bs.weight = 0.0f; bs.isDelta = isCond && rough == 0.0f;      // the plastic's diffuse lobe takes light
     } else {
         bs = mat.bsdfType == 1 ? sample_water(xi1, normal, woWorld, isInside) : sample_lambertian(xi1, xi2);
     }
@@ -589,10 +591,10 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
     next.direction = v3normalized(frame_to_world(normal, bs.wiLocal));
     next.tMax = FLT_MAX;
     const float cosThetaWi = fabsf(bs.wiLocal.z);
-    next.throughput = isCond ? v3mul(path.throughput, cs.weight) : v3mul(v3scale(v3scale(path.throughput, bs.weight), cosThetaWi), albedo);
+    next.throughput = isGlossy ? v3mul(path.throughput, cs.weight) : v3mul(v3scale(v3scale(path.throughput, bs.weight), cosThetaWi), albedo);
     next.pixelIndex = path.pixelIndex; next.shadowPathID = -1; next.visitedMask = 0u;
     next.currentNode = -1; next.targetNode = -1; next.flags = F_VALID;
-    if (isCond && !cs.valid) store_zero_path(p.paths + i);              // the rough lobe sampled below the surface: the path ends
+    if (isGlossy && !cs.valid) store_zero_path(p.paths + i);            // a lobe sampled below the surface: the path ends
     else store_path(p.paths + i, next);
 
     // generateShadowPath x spc (kernel.cu:66-132, 442-465)
@@ -619,13 +621,15 @@ __global__ void __launch_bounds__(kBlock) shade_post_kernel(DevParams p, int n, 
         const float stMax = v3length(ldir);
         const float f1 = fmaxf(0.0f, v3dot(ln, v3neg(wi)));
         const float f2 = fmaxf(0.0f, v3dot(wi, normal));
-        // the conductor's f(wi, wo) takes the place of Lambert's albedo * 1/pi
-        const V3 fr = isCond ? cond_eval(albedo, rough, woLocal, frame_to_local(normal, wi)) : albedo;
+        // the conductor's or the plastic's f(wi, wo) takes the place of Lambert's albedo * 1/pi
+        const V3 fr = isGlossy ? (isCond ? cond_eval(albedo, rough, woLocal, frame_to_local(normal, wi))
+                                         : plastic_eval(albedo, rough, woLocal, frame_to_local(normal, wi)))
+                               : albedo;
         V3 c = v3mul(v3mul(v3(L.Le[0], L.Le[1], L.Le[2]), path.throughput), fr);
         c = v3scale(v3scale(c, f1), f2);
         const float tt = stMax * stMax;
         c = v3(c.x / areaPDF / tt, c.y / areaPDF / tt, c.z / areaPDF / tt);
-        if (!isCond) c = v3scale(c, 0.318309886183790671538f);
+        if (!isGlossy) c = v3scale(c, 0.318309886183790671538f);
         PathRegs sh;
         sh.origin = point; sh.direction = wi; sh.tMax = stMax; sh.throughput = c;
         sh.pixelIndex = path.pixelIndex; sh.shadowPathID = s; sh.visitedMask = 0u; sh.currentNode = -1; sh.targetNode = -1;
@@ -933,6 +937,27 @@ int spec_conductor_eval(const float* f0, const float* r, const float* wo, const 
     for (int64_t i = 0; i < n; i++) {
         const V3 v = cond_eval(v3(f0[3 * i], f0[3 * i + 1], f0[3 * i + 2]), r[i], v3(wo[3 * i], wo[3 * i + 1], wo[3 * i + 2]),
                                v3(wi[3 * i], wi[3 * i + 1], wi[3 * i + 2]));
+        f[3 * i] = v.x; f[3 * i + 1] = v.y; f[3 * i + 2] = v.z;
+    }
+    return 0;
+}
+
+// dprt_spec_plastic_sample / dprt_spec_plastic_eval: host loops over plastic.cuh
+int spec_plastic_sample(const float* albedo, const float* r, const float* wo, const float* xi, int64_t n, float* wi, float* weight) {
+    if (!albedo || !r || !wo || !xi || !wi || !weight || n < 0) return DPRT_ERR_INVALID;
+    for (int64_t i = 0; i < n; i++) {
+        const CondSample s = plastic_sample(v3(albedo[3 * i], albedo[3 * i + 1], albedo[3 * i + 2]), r[i],
+                                            v3(wo[3 * i], wo[3 * i + 1], wo[3 * i + 2]), xi[3 * i], xi[3 * i + 1], xi[3 * i + 2]);
+        wi[3 * i] = s.wi.x; wi[3 * i + 1] = s.wi.y; wi[3 * i + 2] = s.wi.z;
+        weight[3 * i] = s.weight.x; weight[3 * i + 1] = s.weight.y; weight[3 * i + 2] = s.weight.z;
+    }
+    return 0;
+}
+int spec_plastic_eval(const float* albedo, const float* r, const float* wo, const float* wi, int64_t n, float* f) {
+    if (!albedo || !r || !wo || !wi || !f || n < 0) return DPRT_ERR_INVALID;
+    for (int64_t i = 0; i < n; i++) {
+        const V3 v = plastic_eval(v3(albedo[3 * i], albedo[3 * i + 1], albedo[3 * i + 2]), r[i], v3(wo[3 * i], wo[3 * i + 1], wo[3 * i + 2]),
+                                  v3(wi[3 * i], wi[3 * i + 1], wi[3 * i + 2]));
         f[3 * i] = v.x; f[3 * i + 1] = v.y; f[3 * i + 2] = v.z;
     }
     return 0;

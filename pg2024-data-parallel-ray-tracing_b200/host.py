@@ -54,6 +54,8 @@ _PROTOTYPES = {
     "dprt_set_material_roughness": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "dprt_spec_conductor_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "dprt_spec_conductor_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "dprt_spec_plastic_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "dprt_spec_plastic_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "dprt_spec_texture_sample": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "dprt_spec_env_lookup": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_int64, C.c_void_p]),
     "dprt_set_materials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
@@ -286,6 +288,30 @@ def spec_conductor_eval(f0, roughness, wo, wi):
     rc = load_library().dprt_spec_conductor_eval(_ptr(f0), _ptr(r), _ptr(wo), _ptr(w), n, _ptr(out))
     if rc:
         raise DprtError(f"dprt_spec_conductor_eval failed ({rc})")
+    return out
+
+
+def spec_plastic_sample(albedo, roughness, wo, xi):
+    """dprt_spec_plastic_sample (host only): the glossy plastic's next direction wi [n, 3] and throughput factor [n, 3] for
+    local outgoing directions wo [n, 3] and uniforms xi [n, 3], the third choosing the lobe (DESIGN.md 3.13); both 0 where the
+    path ends. albedo (the diffuse colour) [n, 3] or [3], roughness [n] or scalar."""
+    albedo, r, wo, n = _conductor_args(albedo, roughness, wo)
+    x = np.ascontiguousarray(np.broadcast_to(np.asarray(xi, np.float32), (n, 3)))
+    wi, wt = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32)
+    rc = load_library().dprt_spec_plastic_sample(_ptr(albedo), _ptr(r), _ptr(wo), _ptr(x), n, _ptr(wi), _ptr(wt))
+    if rc:
+        raise DprtError(f"dprt_spec_plastic_sample failed ({rc})")
+    return wi, wt
+
+
+def spec_plastic_eval(albedo, roughness, wo, wi):
+    """dprt_spec_plastic_eval (host only): the glossy plastic's f(wi, wo) [n, 3] for local directions wo, wi [n, 3]."""
+    albedo, r, wo, n = _conductor_args(albedo, roughness, wo)
+    w = np.ascontiguousarray(np.broadcast_to(np.asarray(wi, np.float32).reshape(-1, 3), (n, 3)))
+    out = np.zeros((n, 3), np.float32)
+    rc = load_library().dprt_spec_plastic_eval(_ptr(albedo), _ptr(r), _ptr(wo), _ptr(w), n, _ptr(out))
+    if rc:
+        raise DprtError(f"dprt_spec_plastic_eval failed ({rc})")
     return out
 
 
@@ -584,7 +610,8 @@ class Renderer:
         self._ck(self.lib.dprt_set_material_textures(self.h, _ptr(t), t.size), "dprt_set_material_textures")
 
     def set_material_roughness(self, roughness):
-        """GGX roughness in [0, 1] of materials 0 .. len - 1, read for bsdfType 2 (the conductor; 0 = mirror)."""
+        """GGX roughness in [0, 1] of materials 0 .. len - 1, read for bsdfType 2 (the conductor; 0 = mirror) and bsdfType 3 (the
+        glossy plastic's coat; 0 = a smooth coat whose specular lobe is a mirror over the still-lit diffuse base)."""
         r = np.ascontiguousarray(roughness, np.float32)
         self._ck(self.lib.dprt_set_material_roughness(self.h, _ptr(r), r.size), "dprt_set_material_roughness")
 

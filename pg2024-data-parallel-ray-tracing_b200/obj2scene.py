@@ -6,11 +6,13 @@ are not in its tree. This is the equivalent path here, host only (no GPU): the O
 own v / vt / vn index streams (HitGroupData, pipeline_helper.cpp:182-193), the MTL gives base colour (`Kd`), albedo / opacity
 map (`map_Kd`, loaded bottom row first like stbi_loadf after stbi_set_flip_vertically_on_load(1), renderer.cpp:1636-1647) and
 the BSDF (a dielectric `illum` 4 / 6 / 7 / 9 or `Ni` within 0.05 of 1.33 -> Water, everything else Lambertian: the two BSDFs the
-reference has), the geometry is flattened by dprt_flatten_instances and cut into W x-slabs by triangle centroid (one scene
+reference has; with --glossy, metallic and specular materials become the rough conductor and the glossy plastic, see
+glossy_material), the geometry is flattened by dprt_flatten_instances and cut into W x-slabs by triangle centroid (one scene
 object per chunk owner), and everything is written with real_scene.save_scene_v2.
 
     python pg2024-data-parallel-ray-tracing_b200/obj2scene.py scene.obj --out scene.dprt [--world 2] [--width 1920 --height 1080]
            [--eye x,y,z --look-at x,y,z --up 0,0,1 --vfov 40] [--env sky.pfm|sky.exr --env-rotation 2.0] [--lights default|bistro|...]
+           [--glossy]
     dprt_render --scene scene.dprt --out image.exr --spp 64 --world 2
 """
 import argparse
@@ -26,8 +28,14 @@ D = dprt.ctypes_defs
 RS = dprt.real_scene
 
 
+def _mtl_default():
+    return {"Kd": (0.8, 0.8, 0.8), "map_Kd": None, "water": False, "Ks": (0.0, 0.0, 0.0), "Ns": None, "illum": None, "Pr": None,
+            "Pm": None}
+
+
 def load_mtl(path):
-    """{name: {"Kd": (r, g, b), "map_Kd": file or None, "water": bool}} from a Wavefront MTL file."""
+    """{name: {"Kd": (r, g, b), "map_Kd": file or None, "water": bool, "Ks": (r, g, b), "Ns", "illum", "Pr", "Pm": number or
+    None when absent}} from a Wavefront MTL file (Pr / Pm: roughness and metallic of the PBR extension)."""
     mats, cur = {}, None
     with open(path) as f:
         for line in f:
@@ -35,18 +43,41 @@ def load_mtl(path):
             if not p:
                 continue
             if p[0] == "newmtl":
-                cur = mats.setdefault(p[1] if len(p) > 1 else "default", {"Kd": (0.8, 0.8, 0.8), "map_Kd": None, "water": False})
+                cur = mats.setdefault(p[1] if len(p) > 1 else "default", _mtl_default())
             elif cur is None:
                 continue
             elif p[0] == "Kd" and len(p) >= 4:
                 cur["Kd"] = tuple(float(x) for x in p[1:4])
             elif p[0] == "map_Kd" and len(p) >= 2:
                 cur["map_Kd"] = p[-1]
-            elif p[0] == "illum" and len(p) >= 2 and int(float(p[1])) in (4, 6, 7, 9):
-                cur["water"] = True
+            elif p[0] == "illum" and len(p) >= 2:
+                cur["illum"] = int(float(p[1]))
+                if cur["illum"] in (4, 6, 7, 9):
+                    cur["water"] = True
             elif p[0] == "Ni" and len(p) >= 2 and abs(float(p[1]) - 1.33) < 0.05:
                 cur["water"] = True
+            elif p[0] == "Ks" and len(p) >= 4:
+                cur["Ks"] = tuple(float(x) for x in p[1:4])
+            elif p[0] in ("Ns", "Pr", "Pm") and len(p) >= 2:
+                cur[p[0]] = float(p[1])
     return mats
+
+
+def glossy_material(m):
+    """(bsdfType, roughness) of an MTL material under --glossy, or None when it stays as without the flag:
+    - `Pm` >= 0.5 (metallic): the rough conductor (bsdfType 2), F0 = `Kd` (or the `map_Kd` texel);
+    - otherwise a non-water material with a non-zero `Ks` and `illum` >= 2: the glossy plastic (bsdfType 3), diffuse colour `Kd`
+      (or the `map_Kd` texel). `Ks`'s colour is not used: the plastic's coat has the fixed F0 0.04 (DESIGN.md 3.13).
+    Roughness: `Pr` when given, else (2 / (Ns + 2))^(1/4) (Walter et al. 2007's Phong-exponent match alpha = sqrt(2 / (Ns + 2))
+    with alpha = r^2; a missing `Ns` counts as 0), clipped to [0, 1]."""
+    if m["Pm"] is not None and m["Pm"] >= 0.5:
+        kind = 2
+    elif not m["water"] and any(k != 0.0 for k in m["Ks"]) and m["illum"] is not None and m["illum"] >= 2:
+        kind = 3
+    else:
+        return None
+    r = m["Pr"] if m["Pr"] is not None else (2.0 / (max(m["Ns"] or 0.0, 0.0) + 2.0)) ** 0.25
+    return kind, float(np.clip(r, 0.0, 1.0))
 
 
 def mtllibs_of(obj_path):
@@ -74,7 +105,9 @@ class FlatObject:
 
 
 def convert(obj_path, out_path, world=1, width=1920, height=1080, eye=None, look_at=None, up=(0, 0, 1), vfov=40.0, env=None,
-            env_rotation=0.0, lights="fit", light_scale=1.0):
+            env_rotation=0.0, lights="fit", light_scale=1.0, glossy=False):
+    """Writes the scene file; glossy: map metallic and specular MTL materials to bsdfType 2 / 3 (glossy_material) and write
+    their roughness table (DPRTSCN3) when any material was mapped. Without it the file does not depend on Ks / Ns / Pr / Pm."""
     base = os.path.dirname(os.path.abspath(obj_path))
     mtl = {}
     for lib in mtllibs_of(obj_path):
@@ -89,10 +122,15 @@ def convert(obj_path, out_path, world=1, width=1920, height=1080, eye=None, look
     mats = np.zeros(len(names), D.MATERIAL_DTYPE)
     mat_tex = np.full(len(names), -1, np.int32)
     textures, slot_of = {}, {}
+    rough, mapped = np.zeros(len(names), np.float32), False
     for i, nm in enumerate(names):
-        m = mtl.get(nm, {"Kd": (0.8, 0.8, 0.8), "map_Kd": None, "water": False})
+        m = mtl.get(nm, _mtl_default())
         mats["baseColor"][i] = (1.0, 1.0, 1.0) if m["water"] else m["Kd"]
         mats["bsdfType"][i] = 1 if m["water"] else 0
+        g = glossy_material(m) if glossy else None
+        if g is not None:
+            mats["baseColor"][i] = m["Kd"]
+            mats["bsdfType"][i], rough[i], mapped = g[0], g[1], True
         if m["map_Kd"]:
             f = os.path.join(base, m["map_Kd"].replace("\\", "/"))
             if f not in slot_of:
@@ -139,6 +177,8 @@ def convert(obj_path, out_path, world=1, width=1920, height=1080, eye=None, look
         L = dprt.scene.reference_lights(lights)
     garden = {"objects": objects, "materials": mats, "material_textures": mat_tex, "textures": textures, "lights": L,
               "env_map": None if env is None else RS.load_texture(env), "env_rotation": env_rotation}
+    if mapped:
+        garden["material_roughness"] = rough
     RS.save_scene_v2(out_path, garden, cam, dprt.flatten_instances)
     return {"triangles": int(v.shape[0]), "materials": names, "textures": {s: list(t.shape) for s, t in textures.items()},
             "chunks": [int(o.flat[0].shape[0]) for o in objects], "bounds": [lo.tolist(), hi.tolist()]}
@@ -160,9 +200,12 @@ def main():
     ap.add_argument("--env"); ap.add_argument("--env-rotation", type=float, default=0.0)
     ap.add_argument("--lights", default="fit", help='"fit" (two area lights over the scene) or a table of scene.reference_lights: default, san_miguel, air_drome, bistro')
     ap.add_argument("--light-scale", type=float, default=1.0)
+    ap.add_argument("--glossy", action="store_true", help="metallic (Pm >= 0.5) -> rough conductor, specular (Ks != 0, illum >= 2) -> "
+                    "glossy plastic, roughness from Pr or Ns; writes DPRTSCN3 when any material maps")
     a = ap.parse_args()
     import json
-    print(json.dumps(convert(a.obj, a.out, a.world, a.width, a.height, a.eye, a.look_at, a.up, a.vfov, a.env, a.env_rotation, a.lights, a.light_scale)))
+    print(json.dumps(convert(a.obj, a.out, a.world, a.width, a.height, a.eye, a.look_at, a.up, a.vfov, a.env, a.env_rotation, a.lights, a.light_scale,
+                             a.glossy)))
 
 
 if __name__ == "__main__":

@@ -9,7 +9,7 @@ of the same length the shade stage alone (dprt_stage_profile, DPRT_STAGE_SHADE: 
 where one is launched) and the records it shaded, since the materials change where paths go (a mirror sends more of them to
 the sky, where they end).
 The device name and power limit are read in the same process. Prints one JSON line per window and a summary line; --out
-also writes them to DIR/conductor_cost.jsonl.
+also writes them to DIR/conductor_cost.jsonl. profiles/plastic_cost.py runs the same windows for the glossy plastic.
 """
 import argparse
 import importlib
@@ -31,7 +31,8 @@ def device_info():
     return q.stdout.strip() if q.returncode == 0 else "nvidia-smi unavailable"
 
 
-def main():
+def main(bsdf=2, name="conductor"):
+    """The three material tables: all Lambertian, all `bsdf` (named `name`) at roughness 0.3, every other one `bsdf`."""
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=40)
     ap.add_argument("--warmup", type=int, default=4)
@@ -49,12 +50,12 @@ def main():
     R.set_lights(lights); R.set_camera(dprt.scene.default_camera(fw, fh))
     R.set_material_roughness(np.full(len(mats), 0.3, np.float32))
     tables = {}
-    for mode in ("lambert", "conductor", "mixed"):
+    for mode in ("lambert", name, "mixed"):
         m = np.array(mats, copy=True)
-        if mode == "conductor":
-            m["bsdfType"][:] = 2
+        if mode == name:
+            m["bsdfType"][:] = bsdf
         elif mode == "mixed":
-            m["bsdfType"][1::2] = 2
+            m["bsdfType"][1::2] = bsdf
         tables[mode] = m
     lines, first = [], 0
     info = device_info()
@@ -92,7 +93,7 @@ def main():
     print(json.dumps(summary), flush=True)
     if args.out:
         os.makedirs(args.out, exist_ok=True)
-        with open(os.path.join(args.out, "conductor_cost.jsonl"), "w") as f:
+        with open(os.path.join(args.out, f"{name}_cost.jsonl"), "w") as f:
             for ln in lines + [summary]:
                 f.write(json.dumps(ln) + "\n")
     R.close()
